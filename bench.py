@@ -5,6 +5,7 @@ one-class SVM -> per-strain accumulators), BASELINE.json's metric.
 
   python bench.py --gpus N --steps K --warmup W           # CUDA path (this repo)
   python bench.py --impl reference --gpus N --steps K ...  # reference CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                   # + the last timed step's outputs as DIR/*.npy
 
 A step is one pass over ``--fields`` synthetic 2048x2048 fields (config 2 of
 BASELINE.json: 1000 fields, ~500k cells) per GPU, visiting a resident pool of
@@ -385,6 +386,41 @@ def segmentation_extras(with_cpu: bool):
 
 
 # ---------------------------------------------------------------------------
+SCORE_KEYS = ("mse", "mae", "dec_cons", "dec_mod", "pred_cons", "pred_mod")
+# --dump-outputs: two row sets (device pass, end-to-end pass) of 16 columns x 8 bytes stay near 32 MB, within 64 MB
+MAX_DUMP_ROWS = 1 << 17
+
+
+def per_cell_rows(cells, scores, max_rows):
+    """Per-cell results as named columns, rows in (field, label) order so that two builds compare row by
+    row whatever order the device compacted them in; more than ``max_rows`` rows: a fixed seeded sample."""
+    order = np.lexsort((cells["label"], cells["field"]))
+    if len(order) > max_rows:
+        order = order[np.sort(np.random.default_rng(0).choice(len(order), max_rows, replace=False))]
+    cols = {f"cell_{k}": cells[k][order] for k in cells.dtype.names if k != "pad_"}
+    cols.update({k: scores[k][order] for k in SCORE_KEYS})
+    return cols
+
+
+def device_pass_outputs(bs, n_chunks):
+    """What a device-resident pass leaves its caller: the per-strain accumulators and the per-cell
+    results of its last chunk (``run_device`` writes chunk i into ``bs.out[i & 1]``)."""
+    from cell_image_analysis_b200 import _lib
+    o = bs.out[(n_chunks - 1) & 1]
+    n = min(int(o["counts"][0].item()), o["cap"])
+    cells = o["cells"][:n].cpu().numpy().view(_lib.CELL_DTYPE).reshape(-1)
+    rows = per_cell_rows(cells, {k: o[k][:n].cpu().numpy() for k in SCORE_KEYS}, MAX_DUMP_ROWS)
+    return dict(strain_acc=bs.acc.cpu().numpy(), field_counts=o["counts"][1:].cpu().numpy(), **rows)
+
+
+def write_outputs(path, arrays):
+    """``<path>/<name>.npy``: float32 arrays as they are, everything else as float64 (exact for the
+    integer columns)."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def run_native(args):
     import torch
     import torch.distributed as dist
@@ -478,6 +514,7 @@ def run_native(args):
             layer_ms = None
     stage_ms, nrec = bs.profile_end()
     eng.check_status()
+    dump = device_pass_outputs(bs, chunks_per_step) if args.dump_outputs and rank == 0 else None
     # cells per step on this rank: one extra untimed pass without the all-reduce
     cells_local = torch.tensor([0.0], dtype=torch.float64, device=dev)
     bs.sync(); bs.acc.zero_(); bs.run_device(g_dev, l_dev, NF, visit_strain); bs.sync()
@@ -511,6 +548,11 @@ def run_native(args):
     if world > 1:
         dist.all_reduce(ems, op=dist.ReduceOp.MAX)
     e2e_value = cells_per_step * args.steps / (float(ems.item()) * 1e-3)
+    if dump is not None:
+        last = bs.collect_host()
+        dump.update(e2e_field_counts=last["field_counts"],
+                    **{f"e2e_{k}": v for k, v in per_cell_rows(last["cells"], last, MAX_DUMP_ROWS).items()})
+        write_outputs(args.dump_outputs, dump)
     h2d, d2h = bs.host_bytes_per_pass(NF)
     eng.check_status()
     enc_s = getattr(bs, "encode_seconds", 0.0)          # host time inside the encoder during the LAST timed pass
@@ -655,7 +697,15 @@ def main():
     ap.add_argument("--image-transport", default="auto", choices=["auto", "patches", "dense"],
                     help="e2e pass: send whole images or only the bbox rectangles of the labelled regions "
                          "(auto = dense: measured faster on this host at 1 and 2 GPUs, DESIGN.md section 6)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last step computed as DIR/<name>.npy (float32 / float64): "
+                         "strain_acc and field_counts plus the per-cell rows of the device pass's last chunk, and "
+                         "e2e_* for the end-to-end pass (at most 2^17 rows each, a seeded sample beyond that)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native path")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,9 +1,12 @@
 """bench.py's output contract, checked on the committed bench lines (profiles/*.json are the driver-format
-lines of real B200 runs) and on the argument parser -- no GPU needed."""
+lines of real B200 runs) and on the argument parser -- no GPU needed -- and, on a GPU, on a tiny run of --dump-outputs."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -60,5 +63,46 @@ def test_multi_gpu_line_is_weak_scaling_with_config5_strains():
 def test_cli_defaults():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dump-outputs"):
         assert flag in out.stdout
+
+
+def test_dumped_rows_do_not_depend_on_the_device_order():
+    """per-cell rows come out in (field, label) order whatever order they went in, and a pass with more rows than
+    the cap is cut to the same seeded sample every time"""
+    import bench
+    from cell_image_analysis_b200 import _lib
+    rng = np.random.default_rng(5)
+    n = 1000
+    cells = np.zeros(n, _lib.CELL_DTYPE)
+    cells["field"], cells["label"] = rng.integers(0, 8, n), rng.permutation(n) + 1
+    scores = {k: rng.standard_normal(n) for k in bench.SCORE_KEYS}
+    a = bench.per_cell_rows(cells, scores, 300)
+    p = rng.permutation(n)
+    b = bench.per_cell_rows(cells[p], {k: v[p] for k, v in scores.items()}, 300)
+    assert all(np.array_equal(a[k], b[k]) for k in a) and len(a["mse"]) == 300
+    key = a["cell_field"].astype(np.int64) * n + a["cell_label"]
+    assert np.all(np.diff(key) > 0)
+
+
+@pytest.mark.gpu
+def test_steps_and_dumped_outputs(tmp_path):
+    """--steps sets the timed steps, and the last step's outputs do not depend on how many steps ran before it"""
+    dumps, launches = {}, {}
+    for steps in (1, 2):
+        d = tmp_path / f"steps{steps}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1",
+                              "--fields", "4", "--pool", "2", "--chunk", "2", "--no-cpu-baseline", "--no-svm-extras",
+                              "--no-seg-extras", "--dump-outputs", str(d)], capture_output=True, text=True)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == steps
+        launches[steps] = line["gpu_launches"]            # kernels launched inside the timed window
+        dumps[steps] = {f.stem: np.load(f) for f in d.glob("*.npy")}
+    assert launches[1] > 0 and launches[2] == 2 * launches[1], launches
+    a, b = dumps[1], dumps[2]
+    assert set(a) == set(b) and {"strain_acc", "field_counts", "mse", "e2e_mse", "e2e_field_counts"} <= set(a)
+    assert a["strain_acc"][:, 0].sum() > 0 and len(a["mse"]) == a["field_counts"].sum()
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        np.testing.assert_allclose(a[k], b[k], rtol=1e-6 if a[k].dtype == np.float32 else 1e-12, err_msg=k)

@@ -1,8 +1,9 @@
 """hdf5_min against files that were NOT produced by this repository's own writer.
 
-1. A file written by the real libhdf5: SciPy ships ``testhdf5_7.4_GLNX86.mat`` (a MATLAB 7.3
+1. A file written by the real libhdf5: ``tests/golden/testhdf5_7.4_GLNX86.mat``, a copy of the
+   4 KB file of SciPy's test data (scipy/io/matlab/tests/data, BSD-3-Clause) -- a MATLAB 7.3
    file = HDF5 1.6/1.8 behind a 512-byte user block: superblock v0, symbol-table root group, B-tree
-   v1 + SNOD + local heap, v1 object headers, contiguous IEEE dataset) in its test data.
+   v1 + SNOD + local heap, v1 object headers, contiguous IEEE dataset.
 2. Files assembled byte by byte in this test from the HDF5 File Format Specification 3.0 (section
    numbers in the comments) -- independent of ``oracle/h5write.py`` -- covering what h5py emits and
    the in-tree writer does not: a v1 object header whose symbol-table message sits in a
@@ -24,10 +25,7 @@ SIG = b"\x89HDF\r\n\x1a\n"
 
 
 def test_reads_a_file_written_by_the_real_libhdf5():
-    import scipy.io
-    p = os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat")
-    if not os.path.exists(p):
-        pytest.skip("SciPy's MATLAB-7.3 (HDF5) test file is not installed")
+    p = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "testhdf5_7.4_GLNX86.mat")
     f = hdf5_min.H5File(open(p, "rb").read())
     assert f.sb_version == 0 and f.base_addr == 512          # superblock found behind the user block
     ds = f.datasets()
