@@ -9,7 +9,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcia.so")
-SOURCES = ["api.cu", "scan.cu", "crop.cu", "cae_fp32.cu", "cae_tc.cu", "score.cu", "score_tc.cu", "segment.cu", "transport.cu", "host_rle.cpp", "host_tiff.cpp"]
+SOURCES = ["api.cu", "scan.cu", "crop.cu", "cae_fp32.cu", "cae_tc.cu", "score.cu", "score_tc.cu", "segment.cu", "fit.cu", "transport.cu", "host_rle.cpp", "host_tiff.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

@@ -100,6 +100,10 @@ SIGNATURES = {
     "cia_profile_layers": (_I, [_P, C.POINTER(C.c_double)]),
     "cia_debug_copy_workspace": (_I, [_P, _I, C.c_size_t, _P, C.c_size_t]),
     "cia_launch_count": (C.c_int64, [_P]),
+    # fits of create_anomaly_detector (csrc/fit.cu)
+    "cia_fit_robust_scaler": (_I, [_P, _P, _I, _I, _P, _P, _P, _P]),
+    "cia_fit_pca_gram": (_I, [_P, _P, _I, _I, _P, _P, _P]),
+    "cia_ocsvm_fit": (_I, [_P, _P, _I, _I, C.c_double, C.c_double, C.c_double, _I, _P, _P, _P]),
     # segmentation (csrc/segment.cu)
     "cia_seg_load": (_I, [_P, _P, _I, C.POINTER(_P), C.POINTER(_P), _P, _P, _P]),
     "cia_seg_normalize": (_I, [_P, _P, _I, _I, C.c_double, C.c_double, _P, _P, _P]),

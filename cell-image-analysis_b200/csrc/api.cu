@@ -125,7 +125,7 @@ int cia_destroy(cia_handle h) {
     for (int i = 0; i < 2; ++i) { cudaFree(h->svm[i].sv_t); cudaFree(h->svm[i].coef); cudaFree(h->svm[i].sv_pad); cudaFree(h->svm[i].gsn);
                                   cudaFree(h->svm[i].tc_hi); cudaFree(h->svm[i].tc_lo); cudaFree(h->svm[i].tc_gcol); }
     Workspace* ws[] = {&h->ws_flags, &h->ws_act, &h->ws_crop_scratch, &h->ws_pipe, &h->ws_feat,
-                       &h->ws_misc, &h->ws_stage, &h->ws_svm};
+                       &h->ws_misc, &h->ws_stage, &h->ws_svm, &h->ws_fit};
     for (Workspace* w : ws) cudaFree(w->p);
     cudaFree(h->status_dev);
     cudaFreeHost(h->status_host);
@@ -146,7 +146,7 @@ int64_t cia_launch_count(cia_handle h) { return h ? h->launches : 0; }
 int cia_debug_copy_workspace(cia_handle h, int ws_id, size_t offset, void* dst_host, size_t bytes) {
     if (!h) return bad_handle();
     Workspace* ws[] = {&h->ws_flags, &h->ws_act, &h->ws_crop_scratch, &h->ws_pipe, &h->ws_feat,
-                       &h->ws_misc, &h->ws_stage, &h->ws_svm};
+                       &h->ws_misc, &h->ws_stage, &h->ws_svm, &h->ws_fit};
     if (ws_id < 0 || ws_id >= (int)(sizeof(ws) / sizeof(ws[0])) || !dst_host || offset + bytes > ws[ws_id]->cap) {
         h->err = "cia_debug_copy_workspace: bad argument";
         return CIA_E_ARG;
@@ -166,6 +166,7 @@ int cia_check_status(cia_handle h, void* stream) {
     if (code == CIA_E_CAPACITY) h->err = "device: output capacity exceeded (cells_cap too small)";
     else if (code == CIA_E_LABEL) h->err = "device: label outside [0, max_label]";
     else if (code == CIA_E_UNSUPPORTED) h->err = "device: bbox side > 1024 not supported by the crop kernel";
+    else if (code == CIA_E_ARG) h->err = "device: NaN in the features given to cia_fit_robust_scaler";
     else if (code != 0) h->err = "device: unknown status";
     return code;
 }
@@ -394,6 +395,30 @@ int cia_strain_accumulate(cia_handle h, const cia_cell* cells, int n_cells,
     if (!cells || !scores || !acc || n_strains <= 0) { h->err = "cia_strain_accumulate: bad argument"; return CIA_E_ARG; }
     return k_strain_accumulate(h, cells, n_cells, n_cells_dev, scores, field_strain, acc, n_strains,
                                (cudaStream_t)stream);
+}
+
+// ---- fits of create_anomaly_detector (fit.cu; CAE_improved_modeltrain.py:404-423) ----
+int cia_fit_robust_scaler(cia_handle h, const float* features, int n, int n_features, float* center, double* scale,
+                          float* scaled, void* stream) {
+    if (!h) return bad_handle();
+    if (!features || !center || !scale || n < 1 || n_features < 1) { h->err = "cia_fit_robust_scaler: bad argument"; return CIA_E_ARG; }
+    return k_fit_robust_scaler(h, features, n, n_features, center, scale, scaled, (cudaStream_t)stream);
+}
+
+int cia_fit_pca_gram(cia_handle h, const float* x, int n, int n_features, double* mean, double* cov, void* stream) {
+    if (!h) return bad_handle();
+    if (!x || !mean || !cov || n < 2 || n_features < 1) { h->err = "cia_fit_pca_gram: bad argument"; return CIA_E_ARG; }
+    return k_fit_pca_gram(h, x, n, n_features, mean, cov, (cudaStream_t)stream);
+}
+
+int cia_ocsvm_fit(cia_handle h, const double* x, int l, int dim, double nu, double gamma, double tol, int max_iter,
+                  double* alpha, double* result, void* stream) {
+    if (!h) return bad_handle();
+    if (!x || !alpha || !result || l < 1 || dim < 1 || !(nu > 0 && nu <= 1) || !(gamma > 0) || !(tol > 0) || max_iter < -1) {
+        h->err = "cia_ocsvm_fit: bad argument";
+        return CIA_E_ARG;
+    }
+    return k_ocsvm_fit(h, x, l, dim, nu, gamma, tol, max_iter, alpha, result, (cudaStream_t)stream);
 }
 
 // ---- fused path ---------------------------------------------------------------

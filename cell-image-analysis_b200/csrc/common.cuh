@@ -91,6 +91,7 @@ struct cia_ctx {
     std::set<const void*> attr_done;       // kernels whose opt-in smem attribute is set on THIS device
     // grow-only workspaces
     Workspace ws_flags, ws_act, ws_crop_scratch, ws_pipe, ws_feat, ws_misc, ws_stage, ws_svm;
+    Workspace ws_fit;                      // fit.cu: sort buffers, covariance partials, SMO state
     cudaEvent_t ev = nullptr;
     // side stream: the exact-fp32 encoder pass (FMA pipe) overlaps the tensor-core autoencoder
     cudaStream_t side = nullptr;
@@ -222,6 +223,11 @@ int k_seg_details(cia_ctx* h, int cap, int32_t* points, float* prob, float* coor
 int k_seg_layer_info(cia_ctx* h, int layer, int* info);
 int k_seg_debug_layer(cia_ctx* h, int layer, const void* src0, const void* src1, const float* img, int Ho, int Wo,
                       void* out, float* prob, float* dist, cudaStream_t s);
+int k_fit_robust_scaler(cia_ctx* h, const float* x, int n, int F, float* center, double* scale, float* scaled,
+                        cudaStream_t s);
+int k_fit_pca_gram(cia_ctx* h, const float* x, int n, int F, double* mean, double* cov, cudaStream_t s);
+int k_ocsvm_fit(cia_ctx* h, const double* X, int l, int d, double nu, double gamma, double tol, int max_iter,
+                double* alpha, double* result, cudaStream_t s);
 int k_strain_accumulate(cia_ctx* h, const cia_cell* cells, int n, const int32_t* n_dev,
                         const cia_scores* sc, const int32_t* field_strain, double* acc,
                         int n_strains, cudaStream_t s);

@@ -8,6 +8,8 @@ extraction and CAE arithmetic as the screener, on the GPU:
 * ``evaluate_reconstruction_quality(autoencoder, cells)``   train:328-339 (the arithmetic; plots stay with the caller)
 * ``create_anomaly_detector(encoder, cells)``               train:394-446 (features on the GPU; the scikit-learn
                                                             fits are the reference's own library calls)
+* ``create_anomaly_detector_on_device(encoder, cells)``     train:394-446 with the four fits on the GPU too
+                                                            (fitting.py, csrc/fit.cu)
 
 Out of scope (SURVEY.md §2 C12-C14): the Keras model definition and ``fit`` loop
 (``create_improved_autoencoder`` / ``train_autoencoder``) -- they define the weight-file contract the
@@ -164,6 +166,7 @@ class ImprovedAnomalyDetectionTraining:
                       bns=list(ae["bns"]) + [tuple(np.ones(FILTERS[i], np.float32) for _ in range(4)) for i in range(3, 6)])
         arts = dict(autoencoder=ae, encoder_same=True, scaler_pca=A.scaler_pca_arrays(sc, pca),
                     svm_conservative=A.svm_arrays(det), svm_moderate=A.svm_arrays(det))
+        self._arts = arts
         self.engine.load_artifacts(arts)
 
     # train:328-339
@@ -213,6 +216,51 @@ class ImprovedAnomalyDetectionTraining:
         print("\nBaseline anomaly rates:")
         for name, detector in detectors.items():
             predictions = detector.predict(features_reduced)
+            print(f"{name}: {np.sum(predictions == -1) / len(predictions) * 100:.2f}%")
+        for fname, obj in (("scaler.pkl", scaler), ("pca.pkl", pca)):               # train:437-444
+            with open(os.path.join(self.output_dir, fname), "wb") as f:
+                pickle.dump(obj, f)
+        for name, detector in detectors.items():
+            with open(os.path.join(self.output_dir, f"detector_{name.lower()}.pkl"), "wb") as f:
+                pickle.dump(detector, f)
+        return detectors, scaler, pca
+
+    # train:394-446, every fit on the GPU: the features stay on the device from the encoder to the SVM fits
+    def create_anomaly_detector_on_device(self, encoder, cell_images):
+        import torch
+        from . import artifacts as A
+        from . import fitting
+        print("=== Creating Anomaly Detector ===")
+        self._load(encoder=self._weights(encoder, 3))
+        X = np.expand_dims(np.asarray(cell_images), axis=-1).astype("float32")
+        x = torch.from_numpy(np.ascontiguousarray(X[..., 0])).to(self.engine.tdev)
+        _mse, _mae, feat = self.engine.cae_forward(x, len(X))
+        self.engine.check_status()
+        n = len(X)
+        feat = feat[:n]
+        print(f"Encoded features shape: {(n, 8, 8, 32)}")
+        print(f"Flattened features shape: {tuple(feat.shape)}")
+        scaler, features_scaled = fitting.fit_robust_scaler_device(feat, self.engine)        # train:408
+        n_components = min(100, feat.shape[1], n - 1)                                      # train:412
+        pca = fitting.fit_pca(features_scaled, n_components, self.engine)
+        print(f"PCA reduced to {n_components} components")
+        print(f"Explained variance ratio (first 5): {pca.explained_variance_ratio_[:5]}")
+        # the PCA scores of the scoring path (scaler.transform -> pca.transform, the exact fp64 kernels) with the
+        # fitted arrays loaded; the detectors are placeholders here and their outputs unused
+        placeholder = dict(sv=np.zeros((1, n_components)), coef=np.ones(1), gamma=1.0, rho=0.0)
+        arts = dict(self._arts, scaler_pca=A.scaler_pca_arrays(scaler, pca), svm_conservative=placeholder,
+                    svm_moderate=placeholder)
+        self.engine.load_artifacts(arts)
+        features_reduced = self.engine.svm_decision(feat, n, want_pca=True, precision=0)[4][:n]
+        detectors = {"Conservative": fitting.fit_one_class_svm(features_reduced, 0.05, engine=self.engine),
+                     "Moderate": fitting.fit_one_class_svm(features_reduced, 0.10, engine=self.engine)}   # train:420-423
+        arts.update(svm_conservative=A.svm_arrays(detectors["Conservative"]),
+                    svm_moderate=A.svm_arrays(detectors["Moderate"]))
+        self.engine.load_artifacts(arts)
+        _dc, _dm, pred_c, pred_m, _ = self.engine.svm_decision(feat, n, precision=0)
+        print("\nBaseline anomaly rates:")
+        for name, pred in (("Conservative", pred_c), ("Moderate", pred_m)):
+            predictions = pred[:n].cpu().numpy()
             print(f"{name}: {np.sum(predictions == -1) / len(predictions) * 100:.2f}%")
         for fname, obj in (("scaler.pkl", scaler), ("pca.pkl", pca)):               # train:437-444
             with open(os.path.join(self.output_dir, fname), "wb") as f:

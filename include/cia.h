@@ -202,6 +202,25 @@ int cia_strain_accumulate(cia_handle h, const cia_cell* cells, int n_cells,
                           const int32_t* field_strain, double* acc, int n_strains,
                           void* stream);
 
+/* ---- fits of create_anomaly_detector (CAE_improved_modeltrain.py:404-423) ---- */
+/* RobustScaler().fit(features) (train:408): center_ = np.nanmedian(X, axis=0) (float32 [F]) and
+ * scale_ = q75 - q25 of np.nanpercentile(X, (25, 75)) (float64 [F]) with _handle_zeros_in_scale, from exact
+ * column sorts and numpy's "linear" interpolation.  features: float32 [n, F].  scaled (may be NULL): float32 [n, F],
+ * RobustScaler.transform of the same rows (train:408 fit_transform).  NaN is not supported: a NaN in features is
+ * reported as CIA_E_ARG by cia_check_status (np.nanmedian would skip it; the encoder never produces one). */
+int cia_fit_robust_scaler(cia_handle h, const float* features, int n, int n_features, float* center, double* scale,
+                          float* scaled, void* stream);
+/* The covariance PCA(n_components).fit diagonalises (train:412-414; sklearn's covariance_eigh, in fp64):
+ * mean float64 [F] of x float32 [n, F] and cov float64 [F, F] = X_c^T X_c / (n - 1), X_c = x - mean.  n >= 2. */
+int cia_fit_pca_gram(cia_handle h, const float* x, int n, int n_features, double* mean, double* cov, void* stream);
+/* OneClassSVM(kernel="rbf", nu, gamma, tol, max_iter).fit(x) (train:420-423): libsvm's solve_one_class and
+ * Solver::Solve (svm.cpp) iteration for iteration, without shrinking, in one cooperative kernel.  x: float64
+ * [l, dim], dim <= 512 (CIA_E_UNSUPPORTED above); gamma the numeric value (sklearn's _gamma); max_iter -1 = none.
+ * alpha: float64 [l] the dual solution (support vectors: alpha != 0); result: float64 [4] = rho, obj, n_iter,
+ * status (1 when max_iter stopped the solver).  No host synchronisation. */
+int cia_ocsvm_fit(cia_handle h, const double* x, int l, int dim, double nu, double gamma, double tol, int max_iter,
+                  double* alpha, double* result, void* stream);
+
 /* ---- fused path ----------------------------------------------------------- */
 /* The whole hot path for a batch of device-resident fields, with no host
  * synchronisation: scan -> gates -> crop/CLAHE/resize -> CAE -> scaler/PCA/SVM ->
