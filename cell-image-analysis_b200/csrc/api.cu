@@ -165,7 +165,8 @@ int cia_check_status(cia_handle h, void* stream) {
     const int code = *h->status_host;
     if (code == CIA_E_CAPACITY) h->err = "device: output capacity exceeded (cells_cap too small)";
     else if (code == CIA_E_LABEL) h->err = "device: label outside [0, max_label]";
-    else if (code == CIA_E_UNSUPPORTED) h->err = "device: bbox side > 1024 not supported by the crop kernel";
+    else if (code == CIA_E_UNSUPPORTED) h->err = "device: bbox side > 1024 not supported by the crop kernel, or a tensor-core "
+                                                 "autoencoder activation outside the fp16 range (use precision 0)";
     else if (code == CIA_E_ARG) h->err = "device: NaN in the features given to cia_fit_robust_scaler";
     else if (code != 0) h->err = "device: unknown status";
     return code;

@@ -92,13 +92,22 @@ __device__ __forceinline__ float pooled_act(float folded_max, float inv_scale, f
     return __fadd_rn(__fmul_rn(fmaxf(fmaf(m, inv_scale, fmaf(m, invd, b)), 0.f), s), t);
 }
 
-__device__ __forceinline__ void split_store8(const float (&o)[8], __half* hi_dst, __half* lo_dst) {
+// Every tensor-core activation is stored here, as fp16 (hi, and the fp16 remainder lo for the split
+// layers).  A value outside the fp16 range (|x| > 65504 after rounding, e.g. a BatchNorm with a large
+// gamma over a small moving variance) or a NaN would reach the next layer as inf / NaN and turn MSE / MAE
+// into inf or NaN -- or, masked by a later ReLU, into a wrong finite score -- without a word.  Such a
+// store raises CIA_E_UNSUPPORTED on the handle's status word (cia_check_status).
+__device__ __forceinline__ void split_store8(const float (&o)[8], __half* hi_dst, __half* lo_dst, bool& range_ok) {
     __align__(16) __half hh[8];
     __align__(16) __half ll[8];
+    // |x| < 65520 rounds to a finite fp16 (65504 is the largest; 65520 ties to even, to inf); NaN fails the
+    // comparison.  Tested on the fp32 values (one predicate-accumulating compare per element); the kernel
+    // raises the status once, at its end, if any of its stores failed
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
         hh[k] = __float2half_rn(o[k]);
         ll[k] = __float2half_rn(o[k] - __half2float(hh[k]));
+        range_ok = range_ok && fabsf(o[k]) < 65520.f;
     }
     *reinterpret_cast<uint4*>(hi_dst) = *reinterpret_cast<const uint4*>(hh);
     if (lo_dst) *reinterpret_cast<uint4*>(lo_dst) = *reinterpret_cast<const uint4*>(ll);
@@ -194,7 +203,9 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
                float* __restrict__ feat, const float* __restrict__ crops, float* __restrict__ mse,
                float* __restrict__ mae, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
-               int chunk_cells) {
+               int chunk_cells,
+               int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     using C = Cfg<CIN, COUT, R, EPI, NPASS>;
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ __align__(8) uint64_t bar[2];
@@ -398,7 +409,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                 }
                 if (Y < RO) {
                     const size_t off = ((((size_t)cell * (COUT / 8) + sl) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr);
+                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
                     if (feat) {
                         float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
                                                              (size_t)(Y * RO + X) * COUT + c0);
@@ -439,7 +450,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                             }
                             const size_t off = ((((size_t)cell * (CREAL / 8) + cs) * RO + 2 * y + (ph >> 1)) * RO +
                                                 2 * x + (ph & 1)) * 8;
-                            split_store8(o, out_hi + off, nullptr);
+                            split_store8(o, out_hi + off, nullptr, range_ok);
                         }
                     }
                 }
@@ -480,7 +491,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                     }
                     if (y < R) {
                         const size_t off = ((((size_t)cell * (COUT / 8) + sl) * R + y) * R + x) * 8;
-                        split_store8(o, out_hi + off, nullptr);
+                        split_store8(o, out_hi + off, nullptr, range_ok);
                     }
                 }
             }
@@ -507,6 +518,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, C::TMEM_COLS);
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -599,7 +611,9 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
                    const float* __restrict__ bias, const float* __restrict__ bn_s,
                    const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
                    float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
-                   int chunk_cells) {
+                   int chunk_cells,
+                   int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     using C = AccCfg<CIN, COUT, R>;
     // R = 16: the pooled output is only 8 x 8, so a 16-row-group tile takes BOTH row phases
     // (row group g = conv row g, stride one staged row) and there are two tiles (px = 0, 1) instead
@@ -864,7 +878,7 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
                     }
                     if (ROWPAIR && (r & 8)) continue;      // the even conv row's lane stores the pooled pixel
                     const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr);
+                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
                     if (feat) {
                         float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
                                                              (size_t)(Y * RO + X) * COUT + c0);
@@ -891,6 +905,7 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, TMEM_COLS);
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -952,7 +967,9 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                     const float* __restrict__ bias, const float* __restrict__ bn_s,
                     const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
                     float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
-                    int chunk_cells) {
+                    int chunk_cells,
+                    int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     using C = Acc2Cfg<CIN, COUT, R>;
     constexpr bool ROWPAIR = C::ROWPAIR;
     constexpr int NT = ROWPAIR ? 2 : 4;          // accumulator tiles per stage = issuing warps
@@ -1150,7 +1167,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                     }
                     if (ROWPAIR && (r & 8)) continue;      // the even conv row's lane stores the pooled pixel
                     const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr);
+                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
                     if (feat) {
                         float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
                                                              (size_t)(Y * RO + X) * COUT + c0);
@@ -1176,6 +1193,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, TMEM_COLS);
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1211,7 +1229,9 @@ conv_tc_l2_stack_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_
                         const float* __restrict__ bias, const float* __restrict__ bn_s,
                         const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
                         float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
-                        int chunk_cells) {
+                        int chunk_cells,
+                        int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     constexpr int CIN = 32, COUT = 64, R = 32;
     using C = Acc2Cfg<CIN, COUT, R>;
     constexpr int NGRP = (9 + G - 1) / G;        // main-group flushes per tile
@@ -1366,7 +1386,7 @@ conv_tc_l2_stack_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_
                         o[k] = pooled_act(m, inv_scale, invd, b, sc, sh);
                     }
                     const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr);
+                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
                     if (feat) {
                         float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
                                                              (size_t)(Y * RO + X) * COUT + c0);
@@ -1380,6 +1400,7 @@ conv_tc_l2_stack_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, 512);
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1394,7 +1415,9 @@ conv1_fp32_planar_kernel(const float* __restrict__ crops, const float* __restric
                          const float* __restrict__ bias, const float* __restrict__ bn_s,
                          const float* __restrict__ bn_t, __half* __restrict__ out_hi,
                          __half* __restrict__ out_lo, int n_cells, const int32_t* __restrict__ n_dev,
-                         int cell0, int chunk_cells) {
+                         int cell0, int chunk_cells,
+                         int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     __shared__ __align__(16) float xs[34][36];
     __shared__ __align__(16) float ws[9][32];
     int n = dev_count(n_cells, n_dev) - cell0;
@@ -1489,9 +1512,10 @@ conv1_fp32_planar_kernel(const float* __restrict__ crops, const float* __restric
                 }
             }
             const size_t off = ((((size_t)cell * 4 + cg) * 32 + (16 * qy + Y)) * 32 + (16 * qx + X)) * 8;
-            split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr);
+            split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
         }
     }
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1547,7 +1571,9 @@ __global__ void __launch_bounds__(l1tc::NT, 2)
 conv1_tc_split_kernel(const float* __restrict__ crops, const uint4* __restrict__ w_img, float inv_scale,
                       float debias, const float* __restrict__ bias, const float* __restrict__ bn_s,
                       const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
-                      int n_cells, const int32_t* __restrict__ n_dev, int cell0, int chunk_cells) {
+                      int n_cells, const int32_t* __restrict__ n_dev, int cell0, int chunk_cells,
+                      int32_t* __restrict__ status) {
+    bool range_ok = true;             // every fp16 activation store of this thread was finite
     using namespace l1tc;
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ __align__(8) uint64_t done_bar[2], afull_bar[2];
@@ -1712,13 +1738,14 @@ conv1_tc_split_kernel(const float* __restrict__ crops, const uint4* __restrict__
                                             fmaxf(__uint_as_float(v[2][k]), __uint_as_float(v[3][k]))),
                                       inv_scale, invd, b16[sl * 8 + k], s16[sl * 8 + k], t16[sl * 8 + k]);
                 const size_t off = ((((size_t)cell * 4 + (2 * hs + sl)) * 32 + Yp) * 32 + lane) * 8;
-                split_store8(o, out_hi + off, out_lo + off);
+                split_store8(o, out_hi + off, out_lo + off, range_ok);
             }
         }
     }
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, TMEM_COLS);
+    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1913,7 +1940,7 @@ int launch_tc(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_hi, c
     if (grid > cap) grid = cap;
     kern<<<grid, C::THREADS, C::SMEM_B, s>>>(in_hi, in_lo, (const uint4*)w.tc_w[layer][0], (const uint4*)w.tc_w[layer][1],
                                       w.tc_inv_scale[layer], w.bias[layer], w.bn_scale[layer], w.bn_shift[layer],
-                                      out_hi, out_lo, feat, crops, mse, mae, n, n_dev, cell0, chunk);
+                                      out_hi, out_lo, feat, crops, mse, mae, n, n_dev, cell0, chunk, h->status_dev);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
@@ -1954,7 +1981,7 @@ int launch_tc_acc(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_h
                                               (const uint4*)w.tc_w[layer][1], w.tc_inv_scale[layer],
                                               w.tc_inv_scale[layer] * acc_debias(h, layer), w.bias[layer],
                                               w.bn_scale[layer], w.bn_shift[layer], out_hi, out_lo, feat, n, n_dev,
-                                              cell0, chunk);
+                                              cell0, chunk, h->status_dev);
     CIA_LAUNCH_CHECK();
     acc_timing_dump("acc", CIN, COUT, R, G, s);
     return CIA_OK;
@@ -2007,7 +2034,7 @@ int launch_tc_acc2(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_
                                               (const uint4*)w.tc_w[layer][1], w.tc_inv_scale[layer],
                                               w.tc_inv_scale[layer] * acc_debias(h, layer), w.bias[layer],
                                               w.bn_scale[layer], w.bn_shift[layer], out_hi, out_lo, feat, n, n_dev,
-                                              cell0, chunk);
+                                              cell0, chunk, h->status_dev);
     CIA_LAUNCH_CHECK();
     acc_timing_dump("acc2", CIN, COUT, R, G, s);
     return CIA_OK;
@@ -2029,7 +2056,7 @@ int launch_l2_stack(cia_ctx* h, const CaeWeights& w, const __half* in_hi, const 
     if (grid > h->num_sms) grid = h->num_sms;
     kern<<<grid, ACC_THREADS, C::SMEM_B, s>>>(tm_hi, tm_lo, (const uint4*)w.tc_w[1][0], (const uint4*)w.tc_w[1][1],
                                               w.tc_inv_scale[1], w.tc_inv_scale[1] * acc_debias(h, 1), w.bias[1],
-                                              w.bn_scale[1], w.bn_shift[1], out_hi, out_lo, feat, n, n_dev, cell0, chunk);
+                                              w.bn_scale[1], w.bn_shift[1], out_hi, out_lo, feat, n, n_dev, cell0, chunk, h->status_dev);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
@@ -2258,10 +2285,10 @@ int k_cae_forward_tc(cia_ctx* h, const float* crops, int n, const int32_t* n_dev
                 if (gridt > h->num_sms * 2) gridt = h->num_sms * 2;
                 conv1_tc_split_kernel<<<gridt, l1tc::NT, l1tc::SMEM_B, s>>>(crops, (const uint4*)ae.tc_w[0][0], ae.tc_inv_scale[0],
                                                                             l1_debias, ae.bias[0], ae.bn_scale[0], ae.bn_shift[0],
-                                                                            a1h, a1l, n, n_dev, c0, chunk);
+                                                                            a1h, a1l, n, n_dev, c0, chunk, h->status_dev);
             } else {
                 conv1_fp32_planar_kernel<<<grid1, 256, 0, s>>>(crops, ae.kernel[0], ae.bias[0], ae.bn_scale[0],
-                                                               ae.bn_shift[0], a1h, a1l, n, n_dev, c0, chunk);
+                                                               ae.bn_shift[0], a1h, a1l, n, n_dev, c0, chunk, h->status_dev);
             }
             CIA_LAUNCH_CHECK();
             CIA_LMARK(1);
@@ -2302,7 +2329,7 @@ int k_cae_forward_tc(cia_ctx* h, const float* crops, int n, const int32_t* n_dev
             }
         } else {
             conv1_fp32_planar_kernel<<<grid1, 256, 0, s>>>(crops, ae.kernel[0], ae.bias[0], ae.bn_scale[0],
-                                                           ae.bn_shift[0], a1h, nullptr, n, n_dev, c0, chunk);
+                                                           ae.bn_shift[0], a1h, nullptr, n, n_dev, c0, chunk, h->status_dev);
             CIA_LAUNCH_CHECK();
             CIA_LMARK(1);
             if ((rc = launch_tc<32, 64, 32, EPI_POOL, 1>(h, ae, 1, a1h, nullptr, a2h, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;

@@ -98,7 +98,8 @@ int  cia_destroy(cia_handle h);
 const char* cia_last_error(cia_handle h);
 void cia_default_params(cia_params* p);
 /* Reads back the device status word (synchronises `stream`): 0 or a CIA_E_* code
- * raised by a kernel since the last check (capacity / label / unsupported). */
+ * raised by a kernel since the last check (capacity / label / unsupported: a crop kernel bbox too large,
+ * or a tensor-core autoencoder activation outside the fp16 range). */
 int  cia_check_status(cia_handle h, void* stream);
 /* Tuning knobs of the handle (no reference counterpart; defaults reproduce the documented
  * behaviour).  Unknown names / out-of-range values give CIA_E_ARG.
@@ -185,7 +186,13 @@ int cia_debug_clahe_levels(cia_handle h, const uint16_t* images, int H, int W,
                            const int64_t* level_offsets, void* stream);
 /* autoencoder.predict + MSE/MAE (det:125-127) and encoder.predict + flatten
  * (det:130-131).  features (may be NULL): float32 [n, 2048] HWC order.
- * precision: 0 = fp32 CUDA-core path, 1 = tcgen05 tensor-core path. */
+ * precision: 0 = fp32 CUDA-core path, 1 = tcgen05 tensor-core path (split-precision encoder, features
+ * from it), 2 = tensor-core autoencoder for MSE/MAE with the fp32 encoder for the features, 3 = as 1 with
+ * the third encoder layer in exact fp32 (an A/B mode).
+ * Precisions 1-3 store every activation as fp16.  An activation outside the fp16 range (|x| > 65504, e.g.
+ * a BatchNorm with a large gamma over a small moving variance) or a NaN raises CIA_E_UNSUPPORTED on the
+ * status word (cia_check_status); the scores of that call are then not valid.  Precision 0 has no such
+ * limit.  n_cells_dev (may be NULL): device int32 count <= n_cells; cells from it on get mse = mae = 0. */
 int cia_cae_forward(cia_handle h, const float* crops32, int n_cells,
                     const int32_t* n_cells_dev, float* mse, float* mae,
                     float* features, int precision, void* stream);

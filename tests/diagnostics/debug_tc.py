@@ -13,9 +13,11 @@ import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 from cell_image_analysis_b200.screening import ProductionMutantScreening  # noqa: E402
 from oracle import cae as ocae  # noqa: E402
+from test_gpu_cae_layers import PASS_CELLS, ws_layout  # noqa: E402
 
 
 def oracle_layers(X, w):
@@ -52,20 +54,16 @@ def main():
     x = torch.from_numpy(X).to(eng.tdev)
     mse, mae, feat = eng.cae_forward(x, n, precision=prec)
     torch.cuda.synchronize()
-    CH = min(16576, (n + 147) // 148 * 148)     # cells per pass in k_cae_forward_tc (buffer stride)
-    sizes = dict(a1=4 * 32 * 32 * 8, a2=8 * 16 * 16 * 8, a3=4 * 8 * 8 * 8, a4u=4 * 8 * 8 * 8,
-                 a5u=8 * 16 * 16 * 8, a6=4 * 32 * 32 * 8)
-    order = [("A1h", "a1"), ("A1l", "a1"), ("A2h", "a2"), ("A2l", "a2"), ("A3h", "a3"), ("A4u", "a4u"),
-             ("A5u", "a5u"), ("A6", "a6")]
-    off = 0
+    # buffer offsets of k_cae_forward_tc at the handle's default pass size (one pass for this field)
+    _, layout, c0, chunk = ws_layout(n, PASS_CELLS)
+    assert (c0, chunk) == (0, n)
     bufs = {}
-    for name, key in order:
-        nb = n * sizes[key] * 2
-        dst = np.empty(n * sizes[key], np.float16)
-        rc = eng.lib.cia_debug_copy_workspace(eng.h, 5, C.c_size_t(off * 2), C.c_void_p(dst.ctypes.data), C.c_size_t(nb))
+    for name, (off, per, _, _) in layout.items():
+        dst = np.empty(n * per, np.float16)
+        rc = eng.lib.cia_debug_copy_workspace(eng.h, 5, C.c_size_t(off * 2), C.c_void_p(dst.ctypes.data),
+                                              C.c_size_t(dst.nbytes))
         assert rc == 0, rc
         bufs[name] = dst.astype(np.float32)
-        off += CH * sizes[key]
 
     def rep(name, got, want):
         d = np.abs(got - want)

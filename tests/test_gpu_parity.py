@@ -323,7 +323,9 @@ def test_separate_encoder_weights(tmp_path, model_dir, golden_tiny, oracle_weigh
     from oracle import h5write
     from cell_image_analysis_b200.screening import ProductionMutantScreening
     d = tmp_path / "models"
-    shutil.copytree(model_dir, d)
+    # copy the bytes, not the permission bits: in a read-only checkout the copies would be read-only too
+    # and encoder.keras could not be overwritten below
+    shutil.copytree(model_dir, d, copy_function=shutil.copyfile)
     w2 = {"kernels": [k.copy() for k in oracle_weights["kernels"]],
           "biases": [b.copy() for b in oracle_weights["biases"]],
           "bns": [tuple(a.copy() for a in t) for t in oracle_weights["bns"]]}
