@@ -112,6 +112,11 @@ SIGNATURES = {
     "cia_seg_details": (_I, [_P, _I, _P, _P, _P, _P]),
     "cia_seg_layer_info": (_I, [_P, _I, _P]),
     "cia_seg_debug_layer": (_I, [_P, _I, _P, _P, _P, _I, _I, _P, _P, _P, _P]),
+    "cia_seg_normalize_fields": (_I, [_P, _P, _I, _I, _I, C.c_double, C.c_double, _P, _P]),
+    "cia_seg_predict_fields": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
+    "cia_seg_instances_fields": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _I, C.c_double, C.c_double, _P, _P, _P]),
+    "cia_screen_images": (_I, [_P, _P, _P, _I, _I, _I, C.c_double, C.c_double, _I, C.POINTER(Params), _I, _P, _I, _P, _P,
+                               C.POINTER(Scores), _P, _P, _P, _P, _I, _P, _P, _P]),
 }
 
 _lib = None

@@ -8,6 +8,8 @@ Two entry points:
   * ``run_host``: fields in pinned host memory; H2D copies run on a copy stream into
     double-buffered device chunks while the previous chunk is being scored, and the
     per-cell results are copied back D2H inside the pass.
+and their images-only forms ``run_images_device`` / ``run_images_host``, which segment every chunk on the
+device (``cia_screen_images``, a StarDist model loaded on the engine): no labels exist outside HBM.
 """
 from __future__ import annotations
 
@@ -97,6 +99,25 @@ class BatchScreen:
                 st = None if strain_of_visit is None else strain_of_visit[i * self.Fc:(i + 1) * self.Fc]
                 eng.screen_fields(images[p0:p0 + self.Fc], labels[p0:p0 + self.Fc], self.max_label, o,
                                   field_strain=st, acc=self.acc)
+
+    def run_images_device(self, seg: torch.Tensor, images: torch.Tensor, n_fields: int, prob_thresh: float,
+                          nms_thresh: float, strain_of_visit: torch.Tensor | None = None):
+        """``run_device`` with the labels made on the device: each chunk is segmented from ``seg`` (uint16 viewed
+        as int16 [P,H,W]; may be ``images``) and screened on ``images`` in one ``cia_screen_images`` call."""
+        P = images.shape[0]
+        assert P % self.Fc == 0 and seg.shape == images.shape
+        eng = self.eng
+        with torch.cuda.stream(self.compute):
+            if self._stage is not None:
+                for e in self._stage["out_free"]:
+                    self.compute.wait_event(e)
+            for i in range(-(-n_fields // self.Fc)):        # the last chunk may be short
+                p0 = (i * self.Fc) % P
+                nf = min(self.Fc, n_fields - i * self.Fc)
+                o = self.out[i & 1]
+                st = None if strain_of_visit is None else strain_of_visit[i * self.Fc:i * self.Fc + nf]
+                eng.screen_images(seg[p0:p0 + nf], images[p0:p0 + nf], self.max_label, o, prob_thresh,
+                                  nms_thresh, field_strain=st, acc=self.acc)
 
     # ---- host-resident pass (H2D + D2H inside) ----
     def _ensure_stage(self, n_chunks):
@@ -212,19 +233,64 @@ class BatchScreen:
                                   patches=S["d_patch"][b] if use_patches and patches_ok else None)
                 S["done"][b].record(self.compute)
                 S["out_ready"][b].record(self.compute)
-            with torch.cuda.stream(self.d2h):
-                self.d2h.wait_event(S["out_ready"][b])
-                self.h_counts[i].copy_(o["counts"], non_blocking=True)
-                self.h_cells[i].copy_(o["cells"], non_blocking=True)
-                self.h_mse[i].copy_(o["mse"], non_blocking=True)
-                self.h_mae[i].copy_(o["mae"], non_blocking=True)
-                self.h_dc[i].copy_(o["dec_cons"], non_blocking=True)
-                self.h_dm[i].copy_(o["dec_mod"], non_blocking=True)
-                self.h_pc[i].copy_(o["pred_cons"], non_blocking=True)
-                self.h_pm[i].copy_(o["pred_mod"], non_blocking=True)
-                S["out_free"][b].record(self.d2h)
+            self._read_back(i, b, o)
         self._last_chunks = n_chunks
+        self._last_fields = n_fields
         self.last_rle_share = n_rle / max(n_chunks, 1)        # share of the chunks that crossed PCIe as runs
+
+    def _read_back(self, i, b, o):
+        """D2H of chunk i's results (device buffer set b) on the read-back stream"""
+        S = self._stage
+        with torch.cuda.stream(self.d2h):
+            self.d2h.wait_event(S["out_ready"][b])
+            self.h_counts[i].copy_(o["counts"], non_blocking=True)
+            self.h_cells[i].copy_(o["cells"], non_blocking=True)
+            self.h_mse[i].copy_(o["mse"], non_blocking=True)
+            self.h_mae[i].copy_(o["mae"], non_blocking=True)
+            self.h_dc[i].copy_(o["dec_cons"], non_blocking=True)
+            self.h_dm[i].copy_(o["dec_mod"], non_blocking=True)
+            self.h_pc[i].copy_(o["pred_cons"], non_blocking=True)
+            self.h_pm[i].copy_(o["pred_mod"], non_blocking=True)
+            S["out_free"][b].record(self.d2h)
+
+    def run_images_host(self, seg_pinned: torch.Tensor, images_pinned: torch.Tensor, n_fields: int, prob_thresh: float,
+                        nms_thresh: float, strain_of_visit: torch.Tensor | None = None):
+        """``run_host`` with the labels made on the device: only images cross PCIe -- one buffer per chunk when
+        ``seg_pinned`` is ``images_pinned`` (single-channel fields), two when the segmentation channel differs.
+        Same chunking, double buffering, read-back and ``collect_host`` as ``run_host``."""
+        P = images_pinned.shape[0]
+        assert P % self.Fc == 0 and seg_pinned.shape == images_pinned.shape
+        n_chunks = -(-n_fields // self.Fc)          # the last chunk may be short
+        self._ensure_stage(n_chunks)
+        S, eng = self._stage, self.eng
+        same = seg_pinned is images_pinned
+        if not same and "seg" not in S:
+            S["seg"] = [torch.empty((self.Fc, self.H, self.W), dtype=torch.int16, device=eng.tdev) for _ in range(self.NB)]
+        self.h2d_bytes = 0
+        for i in range(n_chunks):
+            b = i % self.NB
+            p0 = (i * self.Fc) % P
+            nf = min(self.Fc, n_fields - i * self.Fc)
+            with torch.cuda.stream(self.copy):
+                self.copy.wait_event(S["done"][b])
+                S["img"][b][:nf].copy_(images_pinned[p0:p0 + nf], non_blocking=True)
+                if not same:
+                    S["seg"][b][:nf].copy_(seg_pinned[p0:p0 + nf], non_blocking=True)
+                self.h2d_bytes += (1 if same else 2) * 2 * nf * self.H * self.W
+                S["ready"][b].record(self.copy)
+            with torch.cuda.stream(self.compute):
+                self.compute.wait_event(S["ready"][b])
+                self.compute.wait_event(S["out_free"][b])
+                o = self.out[b]
+                o["counts"][1 + nf:].zero_()            # per-field counts of the fields a short chunk does not have
+                st = None if strain_of_visit is None else strain_of_visit[i * self.Fc:i * self.Fc + nf]
+                eng.screen_images((S["img"][b] if same else S["seg"][b])[:nf], S["img"][b][:nf], self.max_label, o,
+                                  prob_thresh, nms_thresh, field_strain=st, acc=self.acc)
+                S["done"][b].record(self.compute)
+                S["out_ready"][b].record(self.compute)
+            self._read_back(i, b, o)
+        self._last_chunks = n_chunks
+        self._last_fields = n_fields
 
     def collect_host(self):
         """Compact the per-chunk host buffers of the last ``run_host`` into flat arrays.  Raises if
@@ -243,7 +309,7 @@ class BatchScreen:
         chunk_of = np.repeat(np.arange(n_chunks), ks)
         cells = cells.copy()
         cells["field"] += chunk_of.astype(np.int32) * self.Fc      # visit index within the pass
-        return dict(n_cells=int(ks.sum()), field_counts=counts[:, 1:].reshape(-1), cells=cells,
+        return dict(n_cells=int(ks.sum()), field_counts=counts[:, 1:].reshape(-1)[:self._last_fields], cells=cells,
                     mse=cat(self.h_mse), mae=cat(self.h_mae), dec_cons=cat(self.h_dc),
                     dec_mod=cat(self.h_dm), pred_cons=cat(self.h_pc), pred_mod=cat(self.h_pm))
 

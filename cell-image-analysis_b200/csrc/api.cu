@@ -125,7 +125,7 @@ int cia_destroy(cia_handle h) {
     for (int i = 0; i < 2; ++i) { cudaFree(h->svm[i].sv_t); cudaFree(h->svm[i].coef); cudaFree(h->svm[i].sv_pad); cudaFree(h->svm[i].gsn);
                                   cudaFree(h->svm[i].tc_hi); cudaFree(h->svm[i].tc_lo); cudaFree(h->svm[i].tc_gcol); }
     Workspace* ws[] = {&h->ws_flags, &h->ws_act, &h->ws_crop_scratch, &h->ws_pipe, &h->ws_feat,
-                       &h->ws_misc, &h->ws_stage, &h->ws_svm, &h->ws_fit};
+                       &h->ws_misc, &h->ws_stage, &h->ws_svm, &h->ws_fit, &h->ws_seg_norm};
     for (Workspace* w : ws) cudaFree(w->p);
     cudaFree(h->status_dev);
     cudaFreeHost(h->status_host);
@@ -297,18 +297,54 @@ int cia_seg_normalize(cia_handle h, const uint16_t* image, int H, int W, double 
                       float* mi_ma, void* stream) {
     if (!h) return bad_handle();
     if (!image || !out || H <= 0 || W <= 0 || !(pmin >= 0 && pmin <= pmax && pmax <= 100)) { h->err = "cia_seg_normalize: bad argument"; return CIA_E_ARG; }
-    return k_seg_normalize(h, image, H, W, pmin, pmax, out, mi_ma, (cudaStream_t)stream);
+    return k_seg_normalize(h, image, 1, H, W, H, W, pmin, pmax, out, mi_ma, (cudaStream_t)stream);
 }
 int cia_seg_predict(cia_handle h, const float* image, int H, int W, float* prob, float* dist, void* stream) {
     if (!h) return bad_handle();
     if (!image) { h->err = "cia_seg_predict: null image"; return CIA_E_ARG; }
-    return k_seg_predict(h, image, H, W, prob, dist, (cudaStream_t)stream);
+    return k_seg_predict(h, image, 1, H, W, prob, dist, (cudaStream_t)stream);
 }
 int cia_seg_instances(cia_handle h, const float* prob, const float* dist, int Hg, int Wg, int grid, int H, int W,
                       double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_instances, void* stream) {
     if (!h) return bad_handle();
     if (!labels || Hg <= 0 || Wg <= 0 || grid <= 0 || H <= 0 || W <= 0) { h->err = "cia_seg_instances: bad argument"; return CIA_E_ARG; }
-    return k_seg_instances(h, prob, dist, Hg, Wg, grid, H, W, prob_thresh, nms_thresh, labels, n_instances, (cudaStream_t)stream);
+    return k_seg_instances(h, prob, dist, 1, Hg, Wg, Hg, Wg, grid, H, W, prob_thresh, nms_thresh, labels, n_instances,
+                           (cudaStream_t)stream);
+}
+
+// ---- segmentation of F equally sized fields per call -------------------------------
+static int seg_padded(cia_handle h, const char* who, int n_fields, int H, int W, int* Hp, int* Wp) {
+    const int div = k_seg_div(h);
+    if (!div) { h->err = std::string(who) + ": segmentation model not loaded (cia_seg_load)"; return CIA_E_STATE; }
+    if (n_fields < 1 || n_fields > 65535 || H <= 0 || W <= 0) { h->err = std::string(who) + ": bad argument"; return CIA_E_ARG; }
+    *Hp = (H + div - 1) / div * div;
+    *Wp = (W + div - 1) / div * div;
+    return CIA_OK;
+}
+int cia_seg_normalize_fields(cia_handle h, const uint16_t* images, int n_fields, int H, int W, double pmin, double pmax,
+                             float* out, void* stream) {
+    if (!h) return bad_handle();
+    int Hp, Wp, rc;
+    if ((rc = seg_padded(h, "cia_seg_normalize_fields", n_fields, H, W, &Hp, &Wp))) return rc;
+    if (!images || !out || !(pmin >= 0 && pmin <= pmax && pmax <= 100)) { h->err = "cia_seg_normalize_fields: bad argument"; return CIA_E_ARG; }
+    return k_seg_normalize(h, images, n_fields, H, W, Hp, Wp, pmin, pmax, out, nullptr, (cudaStream_t)stream);
+}
+int cia_seg_predict_fields(cia_handle h, const float* images, int n_fields, int Hp, int Wp, float* prob, float* dist,
+                           void* stream) {
+    if (!h) return bad_handle();
+    if (!images || n_fields < 1) { h->err = "cia_seg_predict_fields: bad argument"; return CIA_E_ARG; }
+    return k_seg_predict(h, images, n_fields, Hp, Wp, prob, dist, (cudaStream_t)stream);
+}
+int cia_seg_instances_fields(cia_handle h, const float* prob, const float* dist, int n_fields, int Hgp, int Wgp, int grid,
+                             int H, int W, double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_instances,
+                             void* stream) {
+    if (!h) return bad_handle();
+    if (!labels || n_fields < 1 || Hgp <= 0 || Wgp <= 0 || grid <= 0 || H <= 0 || W <= 0) {
+        h->err = "cia_seg_instances_fields: bad argument";
+        return CIA_E_ARG;
+    }
+    return k_seg_instances(h, prob, dist, n_fields, Hgp, Wgp, (H + grid - 1) / grid, (W + grid - 1) / grid, grid, H, W,
+                           prob_thresh, nms_thresh, labels, n_instances, (cudaStream_t)stream);
 }
 int cia_seg_details(cia_handle h, int cap, int32_t* points, float* prob, float* coord, void* stream) {
     if (!h) return bad_handle();
@@ -510,6 +546,31 @@ int cia_screen_fields(cia_handle h, const uint16_t* images, const int32_t* label
     return screen_fields_impl(h, images, labels, nullptr, 0, n_fields, H, W, max_label, params, precision,
                               cells, cells_cap, n_cells_dev, field_counts_dev, scores, crops32, features,
                               field_strain, acc, n_strains, stream);
+}
+
+int cia_screen_images(cia_handle h, const uint16_t* seg_images, const uint16_t* images, int n_fields, int H, int W,
+                      double prob_thresh, double nms_thresh, int max_label, const cia_params* params, int precision,
+                      cia_cell* cells, int cells_cap, int32_t* n_cells_dev, int32_t* field_counts_dev,
+                      const cia_scores* scores, float* crops32, float* features, const int32_t* field_strain,
+                      double* acc, int n_strains, int32_t* n_instances_dev, int32_t* labels_out, void* stream) {
+    if (!h) return bad_handle();
+    if (!seg_images) { h->err = "cia_screen_images: null pointer"; return CIA_E_ARG; }
+    int Hp, Wp, rc;
+    if ((rc = seg_padded(h, "cia_screen_images", n_fields, H, W, &Hp, &Wp))) return rc;
+    const int grid = k_seg_grid(h);
+    cudaStream_t s = (cudaStream_t)stream;
+    float* norm = nullptr;
+    int32_t* labels = nullptr;
+    const size_t label_bytes = labels_out ? 0 : (size_t)n_fields * H * W * sizeof(int32_t);
+    if ((rc = k_seg_screen_buffers(h, (size_t)n_fields * Hp * Wp * sizeof(float), label_bytes, &norm, &labels))) return rc;
+    if (labels_out) labels = labels_out;
+    // det:62 normalize(seg_channel) with csbdeep's defaults, det:63 predict_instances, then det:66-153
+    if ((rc = k_seg_normalize(h, seg_images, n_fields, H, W, Hp, Wp, 3.0, 99.8, norm, nullptr, s))) return rc;
+    if ((rc = k_seg_predict(h, norm, n_fields, Hp, Wp, nullptr, nullptr, s))) return rc;
+    if ((rc = k_seg_instances(h, nullptr, nullptr, n_fields, Hp / grid, Wp / grid, (H + grid - 1) / grid, (W + grid - 1) / grid,
+                              grid, H, W, prob_thresh, nms_thresh, labels, n_instances_dev, s))) return rc;
+    return screen_fields_impl(h, images, labels, nullptr, 0, n_fields, H, W, max_label, params, precision, cells, cells_cap,
+                              n_cells_dev, field_counts_dev, scores, crops32, features, field_strain, acc, n_strains, stream);
 }
 
 int cia_screen_fields_rle(cia_handle h, const uint16_t* images, const uint32_t* rle_slots,

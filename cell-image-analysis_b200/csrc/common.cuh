@@ -92,6 +92,7 @@ struct cia_ctx {
     // grow-only workspaces
     Workspace ws_flags, ws_act, ws_crop_scratch, ws_pipe, ws_feat, ws_misc, ws_stage, ws_svm;
     Workspace ws_fit;                      // fit.cu: sort buffers, covariance partials, SMO state
+    Workspace ws_seg_norm;                 // segment.cu: per-field histograms and percentiles of the normalisation
     cudaEvent_t ev = nullptr;
     // side stream: the exact-fp32 encoder pass (FMA pipe) overlaps the tensor-core autoencoder
     cudaStream_t side = nullptr;
@@ -214,11 +215,16 @@ int k_svm_tc(cia_ctx* h, const SvmModel& m, const double* z, int n, const int32_
 void k_seg_free(cia_ctx* h);
 int k_seg_load(cia_ctx* h, const cia_seg_config* cfg, int n_layers, const float* const* kernels,
                const float* const* biases, const int64_t* shapes, const double* ray_sin, const double* ray_cos);
-int k_seg_normalize(cia_ctx* h, const uint16_t* img, int H, int W, double pmin, double pmax, float* out,
-                    float* mi_ma_out, cudaStream_t s);
-int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, float* dist_out, cudaStream_t s);
-int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int Hg, int Wg, int grid, int H, int W,
-                    double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_inst_dev, cudaStream_t s);
+// segmentation of n_fields equally sized fields per call (the single-field entry points are n_fields = 1)
+int k_seg_normalize(cia_ctx* h, const uint16_t* img, int n_fields, int H, int W, int Hp, int Wp, double pmin, double pmax,
+                    float* out, float* mi_ma_out, cudaStream_t s);
+int k_seg_predict(cia_ctx* h, const float* img, int n_fields, int H, int W, float* prob_out, float* dist_out, cudaStream_t s);
+int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int n_fields, int Hgp, int Wgp, int hg, int wg,
+                    int grid, int H, int W, double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_inst_dev,
+                    cudaStream_t s);
+int k_seg_div(cia_ctx* h);
+int k_seg_grid(cia_ctx* h);
+int k_seg_screen_buffers(cia_ctx* h, size_t norm_bytes, size_t label_bytes, float** norm, int32_t** labels);
 int k_seg_details(cia_ctx* h, int cap, int32_t* points, float* prob, float* coord, cudaStream_t s);
 int k_seg_layer_info(cia_ctx* h, int layer, int* info);
 int k_seg_debug_layer(cia_ctx* h, int layer, const void* src0, const void* src1, const float* img, int Ho, int Wo,

@@ -78,6 +78,7 @@ struct SegModel {
     double* ray_sin = nullptr;   // [n_rays] np.sin(np.linspace(0, 2 pi, n_rays, endpoint=False)), from the host
     double* ray_cos = nullptr;
     Workspace act, post, cubtmp;
+    Workspace screen;            // cia_screen_images: normalized padded fields, labels when the caller keeps none
     // pointers into `post` of the last cia_seg_instances call (details of the kept polygons)
     int last_cap = 0;
     float *vy = nullptr, *vx = nullptr, *pprob = nullptr;
@@ -92,10 +93,14 @@ namespace {
 // ---------------------------------------------------------------------------------------
 // csbdeep.utils.normalize: np.percentile (linear interpolation) of a uint16 image from its exact histogram
 // ---------------------------------------------------------------------------------------
+// Every kernel of the normalisation takes the field from blockIdx.y (blockIdx.x for the one-CTA percentile): csbdeep
+// normalizes each image by its own percentiles, so each field has its own histogram copies, wsum and (mi, ma).
 constexpr int SEG_HIST_COPIES = 16;   // copies of the histogram (by CTA): the background's few grey levels are hot addresses
+constexpr size_t SEG_HIST_FIELD = (size_t)SEG_HIST_COPIES * 65536;   // histogram words per field
 
 __global__ void seg_hist_kernel(const uint16_t* __restrict__ img, size_t n, uint32_t* __restrict__ hist) {
-    hist += (size_t)(blockIdx.x % SEG_HIST_COPIES) * 65536;
+    img += (size_t)blockIdx.y * n;
+    hist += (size_t)blockIdx.y * SEG_HIST_FIELD + (size_t)(blockIdx.x % SEG_HIST_COPIES) * 65536;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     const int lane = threadIdx.x & 31;
     for (size_t i0 = (size_t)blockIdx.x * blockDim.x; i0 < n; i0 += stride) {     // warp-uniform trip count
@@ -109,6 +114,8 @@ __global__ void seg_hist_kernel(const uint16_t* __restrict__ img, size_t n, uint
 
 // copy 0 += copies 1..15; wsum[b / 32] = population of 32 consecutive bins (what the selection kernel scans)
 __global__ void seg_hist_reduce_kernel(uint32_t* __restrict__ hist, uint32_t* __restrict__ wsum) {
+    hist += (size_t)blockIdx.y * SEG_HIST_FIELD;
+    wsum += (size_t)blockIdx.y * 2048;
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t c = 0;
     for (int cp = 0; cp < SEG_HIST_COPIES; ++cp) c += hist[(size_t)cp * 65536 + b];
@@ -121,6 +128,9 @@ __global__ void seg_hist_reduce_kernel(uint32_t* __restrict__ hist, uint32_t* __
 // statistics a <= b and _lerp(a, b, t) = a + (b - a) t, or b - (b - a)(1 - t) where t >= 0.5 (numpy/lib/_function_base_impl.py)
 __global__ void __launch_bounds__(1024) seg_percentile_kernel(const uint32_t* __restrict__ hist, const uint32_t* __restrict__ wsum,
                                                               size_t n, double q_lo, double q_hi, float* __restrict__ mi_ma) {
+    hist += (size_t)blockIdx.x * SEG_HIST_FIELD;
+    wsum += (size_t)blockIdx.x * 2048;
+    mi_ma += 2 * blockIdx.x;
     typedef cub::BlockScan<unsigned long long, 1024> Scan;
     __shared__ typename Scan::TempStorage tmp;
     __shared__ unsigned s_val[4];
@@ -161,13 +171,34 @@ __global__ void __launch_bounds__(1024) seg_percentile_kernel(const uint32_t* __
     }
 }
 
-// normalize_mi_ma(x, mi, ma, clip=False, eps=1e-20, dtype=float32): (x - mi) / (ma - mi + eps) in float32
-__global__ void seg_normalize_kernel(const uint16_t* __restrict__ img, size_t n, const float* __restrict__ mi_ma,
-                                     float eps, float* __restrict__ out) {
+// np.pad(mode='reflect') source index of padded position i along a side of n pixels (the reflection is periodic
+// with period 2 (n - 1), as numpy's repeated reflection of pads wider than the image)
+__device__ __forceinline__ int seg_reflect(int i, int n) {
+    if (i < n) return i;
+    if (n == 1) return 0;
+    const int p = 2 * (n - 1), k = i % p;
+    return k < n ? k : p - k;
+}
+
+// normalize_mi_ma(x, mi, ma, clip=False, eps=1e-20, dtype=float32): (x - mi) / (ma - mi + eps) in float32, written
+// straight into the field's reflect-padded [Hp][Wp] frame (a pointwise map commutes with the padding)
+__global__ void seg_normalize_kernel(const uint16_t* __restrict__ img, int H, int W, int Hp, int Wp,
+                                     const float* __restrict__ mi_ma, float eps, float* __restrict__ out) {
+    img += (size_t)blockIdx.y * H * W;
+    out += (size_t)blockIdx.y * Hp * Wp;
+    mi_ma += 2 * blockIdx.y;
     const float mi = mi_ma[0], den = __fadd_rn(__fsub_rn(mi_ma[1], mi), eps);
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-        out[i] = __fdiv_rn(__fsub_rn((float)img[i], mi), den);
+    const size_t stride = (size_t)gridDim.x * blockDim.x, n = (size_t)Hp * Wp;
+    if (Hp == H && Wp == W) {
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+            out[i] = __fdiv_rn(__fsub_rn((float)img[i], mi), den);
+        return;
+    }
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int y = (int)(i / Wp), x = (int)(i - (size_t)y * Wp);
+        const size_t src = (size_t)seg_reflect(y, H) * W + seg_reflect(x, W);
+        out[i] = __fdiv_rn(__fsub_rn((float)img[src], mi), den);
+    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -179,13 +210,17 @@ __global__ void seg_normalize_kernel(const uint16_t* __restrict__ img, size_t n,
 // both pixels, fp16 chunk-planar output.
 __global__ void __launch_bounds__(256) seg_first_kernel(const float* __restrict__ img, const float* __restrict__ w,
                                                         const float* __restrict__ bias, __half* __restrict__ out, int H,
-                                                        int W, int cout) {
+                                                        int W, int cout, int F) {
     extern __shared__ __align__(16) float sw[];   // [9][cout] weights, [cout] bias
     for (int i = threadIdx.x; i < 10 * cout; i += blockDim.x) sw[i] = i < 9 * cout ? w[i] : bias[i - 9 * cout];
     __syncthreads();
     const int Wp = (W + 1) >> 1;
-    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= (size_t)H * Wp) return;
+    const size_t idx0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx0 >= (size_t)F * H * Wp) return;
+    const int f = (int)(idx0 / ((size_t)H * Wp));      // fields [F][H][W] in, [F][cout/8][H][W][8] out
+    const size_t idx = idx0 - (size_t)f * H * Wp;
+    img += (size_t)f * H * W;
+    out += (size_t)f * cout * H * W;
     const int y = (int)(idx / Wp), x = 2 * (int)(idx - (size_t)y * Wp);
     const bool two = x + 1 < W;
     float win[3][4];                               // rows y-1..y+1, columns x-1..x+2
@@ -241,6 +276,7 @@ struct SegConvArgs {
     float* prob;
     float* dist;
     int H, W;            // output resolution
+    int F;               // fields: every map is [F][...] with the field outermost, units are decomposed per field
     int c0, c1, mode, ntaps, groups, chunks;
     // mode 3 (seg_conv_ws_kernel only): the input IS the first layer, evaluated by the producer warps on the fly from
     // the normalized fp32 image: ReLU(conv3x3(img, w1) + b1) with c0 output channels (seg_first_kernel's arithmetic)
@@ -279,8 +315,8 @@ __device__ __forceinline__ uint4 hmax8(uint4 a, uint4 b) {
 
 // One 16-byte unit (8 channels of plane `pl` of the layer's input at output-resolution pixel (y, x)), with the
 // pooling / up-sampling / concatenation of the U-Net folded in.
-__device__ __forceinline__ uint4 seg_load(const SegConvArgs& a, int pl, int y, int x) {
-    const uint4* s0 = reinterpret_cast<const uint4*>(a.src0);
+// s0 / s1: the unit's field of src0 / src1 (seg_src).
+__device__ __forceinline__ uint4 seg_load(const SegConvArgs& a, const uint4* s0, const uint4* s1, int pl, int y, int x) {
     if (a.mode == 0) return __ldg(s0 + ((size_t)pl * a.H + y) * a.W + x);
     if (a.mode == 1) {                                   // MaxPooling2D((2, 2)) of the producer's 2H x 2W map
         const size_t Ws = 2 * (size_t)a.W;
@@ -289,7 +325,15 @@ __device__ __forceinline__ uint4 seg_load(const SegConvArgs& a, int pl, int y, i
     }
     const int p0 = a.c0 >> 3;                            // Concatenate([UpSampling2D((2, 2))(low), skip])
     if (pl < p0) return __ldg(s0 + ((size_t)pl * (a.H >> 1) + (y >> 1)) * (a.W >> 1) + (x >> 1));
-    return __ldg(reinterpret_cast<const uint4*>(a.src1) + ((size_t)(pl - p0) * a.H + y) * a.W + x);
+    return __ldg(s1 + ((size_t)(pl - p0) * a.H + y) * a.W + x);
+}
+
+// field f of the layer's inputs: src0 holds c0 channels at the resolution its mode implies, src1 c1 at the output's
+__device__ __forceinline__ void seg_src(const SegConvArgs& a, int f, const uint4*& s0, const uint4*& s1) {
+    const size_t px = (size_t)a.H * a.W;
+    const size_t px0 = a.mode == 1 ? 4 * px : a.mode == 2 ? (size_t)(a.H >> 1) * (a.W >> 1) : px;
+    s0 = reinterpret_cast<const uint4*>(a.src0) + (size_t)f * (a.c0 >> 3) * px0;
+    s1 = reinterpret_cast<const uint4*>(a.src1) + (size_t)f * (a.c1 >> 3) * px;
 }
 
 // EPI 0: bias + ReLU -> fp16 chunk-planar;  EPI 1: heads (columns 0..31 dist = max(1e-3, .), column 32 prob = sigmoid)
@@ -304,7 +348,8 @@ __global__ void __launch_bounds__(256, SegCfg<N, TILES>::CTAS_PER_SM) seg_conv_k
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
-    const int n_units = tiles_x * tiles_y * a.groups;
+    const int per_field = tiles_x * tiles_y;
+    const int n_units = per_field * a.F * a.groups;
     if ((int)blockIdx.x >= n_units) return;               // uniform: nothing allocated yet
 
     if (warp == 0) tmem_alloc(&tmem_base_s, C::TMEM_COLS);
@@ -320,10 +365,14 @@ __global__ void __launch_bounds__(256, SegCfg<N, TILES>::CTAS_PER_SM) seg_conv_k
     uint32_t phase = 0;
 
     for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
-        const int g = unit / (tiles_x * tiles_y);
-        const int t2 = unit - g * (tiles_x * tiles_y);
+        const int g = unit / (per_field * a.F);               // unit = (group, field, tile)
+        const int fu = unit - g * (per_field * a.F);
+        const int f = fu / per_field, t2 = fu - f * per_field;
         const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
         const int y0 = 16 * ty, x0 = 8 * TILES * tx;
+        const uint4 *s0, *s1;
+        seg_src(a, f, s0, s1);
+        const size_t fpx = (size_t)f * a.H * a.W;
 
         for (int kc = 0; kc < a.chunks; ++kc) {
             if (!(resident && w_loaded)) {
@@ -350,7 +399,7 @@ __global__ void __launch_bounds__(256, SegCfg<N, TILES>::CTAS_PER_SM) seg_conv_k
                         d[j] = (uint32_t)idx * 16u;
                         // a one-tap layer (the heads) never reads the halo ring
                         const bool halo = a.ntaps == 1 && (ry == 0 || ry == 17 || rc == 0 || rc == C::COLS - 1);
-                        if (!halo && y >= 0 && y < a.H && x >= 0 && x < a.W) v[j] = seg_load(a, kc * (SEG_KC / 8) + c, y, x);
+                        if (!halo && y >= 0 && y < a.H && x >= 0 && x < a.W) v[j] = seg_load(a, s0, s1, kc * (SEG_KC / 8) + c, y, x);
                     }
                 }
 #pragma unroll
@@ -403,7 +452,7 @@ __global__ void __launch_bounds__(256, SegCfg<N, TILES>::CTAS_PER_SM) seg_conv_k
                 for (int k = 0; k < 8; ++k)
                     o[k] = __float2half_rn(fmaxf(__fadd_rn(__uint_as_float(v[k]), __ldg(a.bias + c0 + k)), 0.f));
                 if (y < a.H && x < a.W)
-                    *reinterpret_cast<uint4*>(a.out + (((size_t)(c0 >> 3) * a.H + y) * a.W + x) * 8) =
+                    *reinterpret_cast<uint4*>(a.out + fpx * a.groups * N + (((size_t)(c0 >> 3) * a.H + y) * a.W + x) * 8) =
                         *reinterpret_cast<const uint4*>(o);
             }
         } else {
@@ -416,7 +465,7 @@ __global__ void __launch_bounds__(256, SegCfg<N, TILES>::CTAS_PER_SM) seg_conv_k
                 TMEM_LD8(lane_addr + (uint32_t)(t * N + sl * 8), v);
                 TMEM_WAIT8(v);
                 if (y < a.H && x < a.W) {
-                    const size_t px = (size_t)y * a.W + x;
+                    const size_t px = fpx + (size_t)y * a.W + x;
                     if (sl < SEG_RAYS / 8) {
                         float o[8];
 #pragma unroll
@@ -471,7 +520,7 @@ struct SegTmaCfg {
 template <int N, int TILES, int POOL>
 __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_constant__ CUtensorMap tm, const uint4* __restrict__ w,
                                                               const float* __restrict__ bias, __half* __restrict__ out,
-                                                              __half* __restrict__ out_pool, int H, int W) {
+                                                              __half* __restrict__ out_pool, int H, int W, int F) {
     using C = SegCfg<N, TILES>;
     using T = SegTmaCfg<N, TILES>;
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -479,8 +528,11 @@ __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_const
     __shared__ uint32_t tmem_base_s;
     unsigned char* sw = smem + T::STAGES * T::A_STRIDE;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    // unit = (field, tile); the tensor map's outermost dimension is field * 4 + plane, so a box at plane 4 f reads
+    // field f only and the y / x out-of-bounds zero fill is that field's own padding
     const int tiles_x = (W + 8 * TILES - 1) / (8 * TILES), tiles_y = (H + 15) / 16;
-    const int n_units = tiles_x * tiles_y;
+    const int per_field = tiles_x * tiles_y;
+    const int n_units = per_field * F;
     if ((int)blockIdx.x >= n_units) return;
 
     if (warp == 0) tmem_alloc(&tmem_base_s, T::TMEM_COLS);
@@ -504,9 +556,10 @@ __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_const
             for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++j) {
                 const int s = j % T::STAGES;
                 mbar_wait(&empty[s], (uint32_t)(((j / T::STAGES) & 1) ^ 1));
-                const int ty = unit / tiles_x, tx = unit - ty * tiles_x;
+                const int f = unit / per_field, t2 = unit - f * per_field;
+                const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
                 mbar_expect_tx(&full[s], C::A_B);
-                tma_load_4d(smem_u32(smem + s * T::A_STRIDE), &tm, 0, 8 * TILES * tx - 1, 16 * ty - 1, 0, &full[s]);
+                tma_load_4d(smem_u32(smem + s * T::A_STRIDE), &tm, 0, 8 * TILES * tx - 1, 16 * ty - 1, 4 * f, &full[s]);
             }
         }
     } else if (warp == 9) {
@@ -544,8 +597,11 @@ __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_const
         int j = 0;
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++j) {
             const int t = j & 1;
-            const int ty = unit / tiles_x, tx = unit - ty * tiles_x;
+            const int f = unit / per_field, t2 = unit - f * per_field;
+            const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
             const int y = 16 * ty + (r >> 3), x0 = 8 * TILES * tx;
+            __half* fout = out + (size_t)f * N * H * W;
+            __half* fpool = out_pool + (size_t)f * N * (H >> 1) * (W >> 1);
             mbar_wait(&tfull[t], (uint32_t)((j >> 1) & 1));
             tc_fence_after();
             const uint32_t lane_addr = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(t * TILES * N);
@@ -561,7 +617,7 @@ __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_const
                 for (int k = 0; k < 8; ++k)
                     o[k] = __float2half_rn(fmaxf(__fadd_rn(__uint_as_float(v[k]), __ldg(bias + sl * 8 + k)), 0.f));
                 if (POOL != 1 && y < H && x < W)
-                    *reinterpret_cast<uint4*>(out + (((size_t)sl * H + y) * W + x) * 8) = *reinterpret_cast<const uint4*>(o);
+                    *reinterpret_cast<uint4*>(fout + (((size_t)sl * H + y) * W + x) * 8) = *reinterpret_cast<const uint4*>(o);
                 if (POOL != 0) {
                     uint4 u = *reinterpret_cast<const uint4*>(o), p1;
                     p1.x = __shfl_xor_sync(0xffffffffu, u.x, 1); p1.y = __shfl_xor_sync(0xffffffffu, u.y, 1);
@@ -571,7 +627,7 @@ __global__ void __launch_bounds__(320, 1) seg_conv_tma_kernel(const __grid_const
                     p1.z = __shfl_xor_sync(0xffffffffu, u.z, 8); p1.w = __shfl_xor_sync(0xffffffffu, u.w, 8);
                     u = hmax8(u, p1);
                     if (((r & 1) | ((r >> 3) & 1)) == 0 && y < H && x < W)
-                        *reinterpret_cast<uint4*>(out_pool + (((size_t)sl * (H >> 1) + (y >> 1)) * (W >> 1) + (x >> 1)) * 8) = u;
+                        *reinterpret_cast<uint4*>(fpool + (((size_t)sl * (H >> 1) + (y >> 1)) * (W >> 1) + (x >> 1)) * 8) = u;
                 }
             }
             tc_fence_before();
@@ -606,7 +662,7 @@ struct SegHeadsCfg {
 template <int CIN>
 __global__ void __launch_bounds__(320, 1) seg_heads_tma_kernel(const __grid_constant__ CUtensorMap tm, const uint4* __restrict__ w,
                                                                const float* __restrict__ bias, float* __restrict__ prob,
-                                                               float* __restrict__ dist, int H, int W) {
+                                                               float* __restrict__ dist, int H, int W, int F) {
     using T = SegHeadsCfg<CIN>;
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ __align__(8) uint64_t full[T::STAGES], empty[T::STAGES], tfull[2], tempty[2];
@@ -614,7 +670,8 @@ __global__ void __launch_bounds__(320, 1) seg_heads_tma_kernel(const __grid_cons
     unsigned char* sw = smem + T::STAGES * T::A_B;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tiles_x = (W + 15) / 16, tiles_y = (H + 15) / 16;
-    const int n_units = tiles_x * tiles_y;
+    const int per_field = tiles_x * tiles_y;               // unit = (field, tile), as seg_conv_tma_kernel
+    const int n_units = per_field * F;
     if ((int)blockIdx.x >= n_units) return;
 
     if (warp == 0) tmem_alloc(&tmem_base_s, T::TMEM_COLS);
@@ -638,9 +695,10 @@ __global__ void __launch_bounds__(320, 1) seg_heads_tma_kernel(const __grid_cons
             for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++j) {
                 const int s = j % T::STAGES;
                 mbar_wait(&empty[s], (uint32_t)(((j / T::STAGES) & 1) ^ 1));
-                const int ty = unit / tiles_x, tx = unit - ty * tiles_x;
+                const int f = unit / per_field, t2 = unit - f * per_field;
+                const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
                 mbar_expect_tx(&full[s], T::A_B);
-                tma_load_4d(smem_u32(smem + s * T::A_B), &tm, 0, 16 * tx, 16 * ty, 0, &full[s]);
+                tma_load_4d(smem_u32(smem + s * T::A_B), &tm, 0, 16 * tx, 16 * ty, T::PLANES * f, &full[s]);
             }
         }
     } else if (warp == 9) {
@@ -674,7 +732,8 @@ __global__ void __launch_bounds__(320, 1) seg_heads_tma_kernel(const __grid_cons
         int j = 0;
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++j) {
             const int t = j & 1;
-            const int ty = unit / tiles_x, tx = unit - ty * tiles_x;
+            const int f = unit / per_field, t2 = unit - f * per_field;
+            const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
             const int y = 16 * ty + (r >> 3), x0 = 16 * tx;
             mbar_wait(&tfull[t], (uint32_t)((j >> 1) & 1));
             tc_fence_after();
@@ -687,7 +746,7 @@ __global__ void __launch_bounds__(320, 1) seg_heads_tma_kernel(const __grid_cons
                 TMEM_LD8(lane_addr + (uint32_t)(tile * T::N + sl * 8), v);
                 TMEM_WAIT8(v);
                 if (y < H && x < W) {
-                    const size_t px = (size_t)y * W + x;
+                    const size_t px = ((size_t)f * H + y) * W + x;
                     if (sl < SEG_RAYS / 8) {
                         float o[8];
 #pragma unroll
@@ -741,7 +800,7 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
     __shared__ __align__(16) float s_first[10 * 128];      // mode 3: first-layer weights [9][c0] and bias [c0]
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
-    const int per_group = tiles_x * tiles_y;
+    const int per_field = tiles_x * tiles_y, per_group = per_field * a.F;    // unit = (group, field, tile)
     const int n_units = per_group * a.groups;
     if ((int)blockIdx.x >= n_units) return;
 
@@ -766,9 +825,13 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
         const int pt = tid - 256;
         int step = 0;
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
-            const int g = unit / per_group, t2 = unit - g * per_group;
+            const int g = unit / per_group, fu = unit - g * per_group;
+            const int f = fu / per_field, t2 = fu - f * per_field;
             const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
             const int y0 = 16 * ty, x0 = 8 * TILES * tx;
+            const uint4 *s0, *s1;
+            seg_src(a, f, s0, s1);
+            const float* fimg = a.img + (size_t)f * a.H * a.W;
             for (int kc = 0; kc < a.chunks; ++kc, ++step) {
                 const int s = step % T::STAGES;
                 mbar_wait(&empty[s], (uint32_t)(((step / T::STAGES) & 1) ^ 1));
@@ -788,8 +851,8 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
 #pragma unroll
                         for (int t = 0; t < 9; ++t) {
                             const int yy = y + t / 3 - 1, xx = x + t % 3 - 1;
-                            const float f = (inside && yy >= 0 && yy < a.H && xx >= 0 && xx < a.W) ? __ldg(a.img + (size_t)yy * a.W + xx) : 0.f;
-                            v2[t] = pack2(f, f);
+                            const float v = (inside && yy >= 0 && yy < a.H && xx >= 0 && xx < a.W) ? __ldg(fimg + (size_t)yy * a.W + xx) : 0.f;
+                            v2[t] = pack2(v, v);
                         }
 #pragma unroll 1
                         for (int c = 0; c < SEG_KC / 8; ++c) {
@@ -836,7 +899,7 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
                             const int ry = rem / C::COLS, rc = rem - ry * C::COLS;
                             const int y = y0 + ry - 1, x = x0 + rc - 1;
                             d[j] = (uint32_t)idx * 16u;
-                            if (y >= 0 && y < a.H && x >= 0 && x < a.W) v[j] = seg_load(a, kc * (SEG_KC / 8) + c, y, x);
+                            if (y >= 0 && y < a.H && x >= 0 && x < a.W) v[j] = seg_load(a, s0, s1, kc * (SEG_KC / 8) + c, y, x);
                         }
                     }
 #pragma unroll
@@ -887,9 +950,11 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
         int j = 0;
         for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x, ++j) {
             const int t = j & 1;
-            const int g = unit / per_group, t2 = unit - g * per_group;
+            const int g = unit / per_group, fu = unit - g * per_group;
+            const int f = fu / per_field, t2 = fu - f * per_field;
             const int ty = t2 / tiles_x, tx = t2 - ty * tiles_x;
             const int y = 16 * ty + (r >> 3), x0 = 8 * TILES * tx;
+            __half* fout = a.out + (size_t)f * a.groups * N * a.H * a.W;
             mbar_wait(&tfull[t], (uint32_t)((j >> 1) & 1));
             tc_fence_after();
             const uint32_t lane_addr = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(t * TILES * N);
@@ -906,7 +971,7 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
                 for (int k = 0; k < 8; ++k)
                     o[k] = __float2half_rn(fmaxf(__fadd_rn(__uint_as_float(v[k]), __ldg(a.bias + c0 + k)), 0.f));
                 if (y < a.H && x < a.W)
-                    *reinterpret_cast<uint4*>(a.out + (((size_t)(c0 >> 3) * a.H + y) * a.W + x) * 8) = *reinterpret_cast<const uint4*>(o);
+                    *reinterpret_cast<uint4*>(fout + (((size_t)(c0 >> 3) * a.H + y) * a.W + x) * 8) = *reinterpret_cast<const uint4*>(o);
             }
             tc_fence_before();
             __syncwarp();
@@ -923,40 +988,53 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
 // ---------------------------------------------------------------------------------------
 // Candidates in descending probability, ties: the larger flat index first (np.argsort(prob, stable)[::-1]):
 // flags -> exclusive scan -> compaction in DESCENDING index order -> stable radix sort of the inverted probability
-// bits (32-bit keys, the index as the value: half the passes of a 64-bit key sort)
-__global__ void seg_cand_flags_kernel(const float* __restrict__ prob, int Hg, int Wg, float thr, int border,
-                                      int* __restrict__ flags) {
+// bits (32-bit keys, the index as the value: half the passes of a 64-bit key sort).
+// F fields [F][Hgp][Wgp] (maps padded to Hgp x Wgp, candidates only in the logical hg x wg part): the flat index runs
+// over all fields and the key carries the field above bit 32, so the sort over 32 + ceil(log2 F) bits orders by
+// field, then exactly as a one-field call; one field keeps 32-bit keys.
+__global__ void seg_cand_flags_kernel(const float* __restrict__ prob, int F, int Hgp, int Wgp, int hg, int wg, float thr,
+                                      int border, int* __restrict__ flags) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx >= Hg * Wg) return;
-    const int i = idx / Wg, j = idx - i * Wg;
-    flags[idx] = (prob[idx] > thr && i >= border && i < Hg - border && j >= border && j < Wg - border) ? 1 : 0;
+    if (idx >= F * Hgp * Wgp) return;
+    const int rem = idx % (Hgp * Wgp);
+    const int i = rem / Wgp, j = rem - i * Wgp;
+    flags[idx] = (prob[idx] > thr && i >= border && i < hg - border && j >= border && j < wg - border) ? 1 : 0;
 }
 
+template <typename K>
 __global__ void seg_cand_scatter_kernel(const float* __restrict__ prob, const int* __restrict__ flags, const int* __restrict__ excl,
-                                        int cap, unsigned* __restrict__ keys, unsigned* __restrict__ vals, int* __restrict__ count) {
+                                        int cap, int field_px, K* __restrict__ keys, unsigned* __restrict__ vals,
+                                        int* __restrict__ count) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= cap) return;
     const int total = excl[cap - 1] + flags[cap - 1];
     if (idx == 0) *count = total;
     if (flags[idx]) {
         const int pos = total - 1 - excl[idx];
-        keys[pos] = ~__float_as_uint(prob[idx]);
+        K key = (K)~__float_as_uint(prob[idx]);
+        if constexpr (sizeof(K) == 8) key |= (K)(idx / field_px) << 32;
+        keys[pos] = key;
         vals[pos] = (unsigned)idx;
     }
 }
 
 // dist_to_coord: coord = (dist * [sin, cos]).astype(float32); coord += points  (float32 += int: added in fp64, stored fp32)
+// rank r (sorted order over all fields) -> its field's polygon; rfield[r] = field.  Bins are per field: field f owns
+// bins [f nby nbx, (f + 1) nby nbx), so no reach ever crosses into another field.
 __global__ void seg_polygons_kernel(const unsigned* __restrict__ sorted_idx, const int* __restrict__ count, int cap,
-                                    const float* __restrict__ prob, const float* __restrict__ dist, int Wg, int grid,
+                                    const float* __restrict__ prob, const float* __restrict__ dist, int Hgp, int Wgp, int grid,
                                     const double* __restrict__ rsin, const double* __restrict__ rcos, int H, int W,
                                     float* __restrict__ vy, float* __restrict__ vx, int* __restrict__ pyx,
                                     float* __restrict__ pprob, float* __restrict__ rmax, double* __restrict__ area,
-                                    int* __restrict__ bin_of, int* __restrict__ bin_count, unsigned* __restrict__ rmax_all) {
+                                    int* __restrict__ bin_of, int* __restrict__ bin_count, unsigned* __restrict__ rmax_all,
+                                    int* __restrict__ rfield) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     const int n = min(*count, cap);
     if (r >= n) return;
     const unsigned idx = sorted_idx[r];
-    const int i = (int)(idx / (unsigned)Wg), j = (int)(idx - (unsigned)i * Wg);
+    const int f = (int)(idx / (unsigned)(Hgp * Wgp));
+    const unsigned rem = idx - (unsigned)f * (unsigned)(Hgp * Wgp);
+    const int i = (int)(rem / (unsigned)Wgp), j = (int)(rem - (unsigned)i * Wgp);
     const int py = i * grid, px = j * grid;
     const float* d = dist + (size_t)idx * SEG_RAYS;
     float ys[SEG_RAYS], xs[SEG_RAYS];
@@ -982,8 +1060,9 @@ __global__ void seg_polygons_kernel(const unsigned* __restrict__ sorted_idx, con
     pprob[r] = prob[idx];
     rmax[r] = rm;
     atomicMax(rmax_all, __float_as_uint(rm));            // rm >= 1e-3 > 0: the bit pattern orders like the value
-    const int nbx = (W + SEG_BIN - 1) / SEG_BIN;
-    const int bin = min(py / SEG_BIN, (H + SEG_BIN - 1) / SEG_BIN - 1) * nbx + min(px / SEG_BIN, nbx - 1);
+    const int nbx = (W + SEG_BIN - 1) / SEG_BIN, nby = (H + SEG_BIN - 1) / SEG_BIN;
+    const int bin = (f * nby + min(py / SEG_BIN, nby - 1)) * nbx + min(px / SEG_BIN, nbx - 1);
+    rfield[r] = f;
     bin_of[r] = bin;
     atomicAdd(bin_count + bin, 1);
 }
@@ -1115,13 +1194,13 @@ struct NmsArgs {
     const int* pyx;              // [rank][2]
     const double* area;          // [rank]
     const int* b_rank;           // candidates in BIN order (position k): rank,
-    const float4* b_yxr;         //   (y, x, rmax, -)
+    const float4* b_yxr;         //   (y, x, rmax, field as int bits)
     const int* bin_start;
     const int* count;
     const unsigned* rmax_all;
     int* state;          // by bin position: 0 undecided, 2 suppressed, 4 + round: kept (winner of that round)
     int* cnt;            // [3] undecided counters of rounds r, r + 1, r + 2 (mod 3)
-    int nbx, nby, cap;
+    int nbx, nby, cap;           // bins of ONE field; field f's bins start at f nby nbx
     double thr;
 };
 
@@ -1254,6 +1333,7 @@ __global__ void __launch_bounds__(256, SEG_NMS_CTAS) seg_nms_kernel(const NmsArg
                 if (ld_volatile(a.state + k) != 0) continue;                 // warp-uniform
                 const int rank = a.b_rank[k];
                 const float4 me = a.b_yxr[k];
+                const int* fbins = a.bin_start + __float_as_int(me.w) * a.nby * a.nbx;   // the candidate's field
                 const float reach = me.z + RM + 0.01f;
                 const int by0 = max(0, (int)floorf((me.x - reach) * inv_bin)), by1 = min(a.nby - 1, (int)floorf((me.x + reach) * inv_bin));
                 const int bx0 = max(0, (int)floorf((me.y - reach) * inv_bin)), bx1 = min(a.nbx - 1, (int)floorf((me.y + reach) * inv_bin));
@@ -1266,8 +1346,8 @@ __global__ void __launch_bounds__(256, SEG_NMS_CTAS) seg_nms_kernel(const NmsArg
                     int by;
                     if ((byc - up >= by0) && (up < dn || byc + dn > by1)) { by = byc - up; ++up; }
                     else { by = byc + dn; ++dn; }
-                    const int ke = a.bin_start[by * a.nbx + bx1 + 1];
-                    for (int k0 = a.bin_start[by * a.nbx + bx0]; k0 < ke && !done; k0 += 32) {
+                    const int ke = fbins[by * a.nbx + bx1 + 1];
+                    for (int k0 = fbins[by * a.nbx + bx0]; k0 < ke && !done; k0 += 32) {
                         const int kk = k0 + lane;
                         bool hit = false;
                         int rj = -1;
@@ -1307,12 +1387,13 @@ __global__ void __launch_bounds__(256, SEG_NMS_CTAS) seg_nms_kernel(const NmsArg
 // bin-order copies of what the suppression reads per neighbour
 __global__ void seg_binorder_kernel(const int* __restrict__ bin_of, int* __restrict__ bin_cursor, const int* __restrict__ count,
                                     int cap, const int* __restrict__ pyx, const float* __restrict__ rmax,
-                                    int* __restrict__ b_rank, float4* __restrict__ b_yxr, int* __restrict__ pos) {
+                                    const int* __restrict__ rfield, int* __restrict__ b_rank, float4* __restrict__ b_yxr,
+                                    int* __restrict__ pos) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= min(*count, cap)) return;
     const int k = atomicAdd(bin_cursor + bin_of[r], 1);
     b_rank[k] = r;
-    b_yxr[k] = make_float4((float)pyx[2 * r], (float)pyx[2 * r + 1], rmax[r], 0.f);
+    b_yxr[k] = make_float4((float)pyx[2 * r], (float)pyx[2 * r + 1], rmax[r], __int_as_float(rfield[r]));
     pos[r] = k;
 }
 
@@ -1323,12 +1404,24 @@ __global__ void seg_flags_kernel(const int* __restrict__ state, const int* __res
     flags[r] = (r < min(*count, cap) && state[pos[r]] >= 4) ? 1 : 0;
 }
 
+// kept polygons in rank order; ranks are grouped by field, so kstart[f] (kept polygons of the fields before f,
+// [F + 1]) is excl at the first rank of field f: written by that rank for f and the empty fields before it
 __global__ void seg_compact_kernel(const int* __restrict__ flags, const int* __restrict__ excl, int cap,
-                                   int* __restrict__ kept_rank, int* __restrict__ n_kept) {
+                                   const int* __restrict__ count, const int* __restrict__ rfield, int F,
+                                   int* __restrict__ kept_rank, int* __restrict__ n_kept, int* __restrict__ kstart) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= cap) return;
     if (flags[r]) kept_rank[excl[r]] = r;
     if (r == cap - 1) *n_kept = excl[r] + flags[r];
+    const int n = min(*count, cap);
+    if (r < n) {
+        const int fr = rfield[r], fp = r == 0 ? -1 : rfield[r - 1];
+        for (int f = fp + 1; f <= fr; ++f) kstart[f] = excl[r];
+        if (r == n - 1)
+            for (int f = fr + 1; f <= F; ++f) kstart[f] = excl[r] + flags[r];
+    } else if (r == 0) {
+        for (int f = 0; f <= F; ++f) kstart[f] = 0;
+    }
 }
 
 // skimage.draw.polygon's test (skimage/_shared/_geometry / _pnpoly.h point_in_polygon): crossings of the edges
@@ -1359,8 +1452,8 @@ constexpr int SEG_EMPTY = 0x7F7F7F7F;   // cudaMemset(0x7F) background of the at
 // the smallest index among the polygons that cover it
 __global__ void __launch_bounds__(256) seg_render_kernel(const float* __restrict__ vy, const float* __restrict__ vx,
                                                          const int* __restrict__ pyx, const int* __restrict__ kept_rank,
-                                                         const int* __restrict__ n_kept, int H, int W,
-                                                         int32_t* __restrict__ labels) {
+                                                         const int* __restrict__ n_kept, const int* __restrict__ rfield,
+                                                         int H, int W, int32_t* __restrict__ labels) {
     __shared__ float s_v[8][2][SEG_RAYS];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int gwarp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, gwarps = (gridDim.x * blockDim.x) >> 5;
@@ -1368,6 +1461,7 @@ __global__ void __launch_bounds__(256) seg_render_kernel(const float* __restrict
     for (int job = gwarp; job < nk * SEG_RENDER_SPLIT; job += gwarps) {
         const int k = job / SEG_RENDER_SPLIT, part = job - k * SEG_RENDER_SPLIT;    // rows part, part + 16, ... of polygon k
         const int r = kept_rank[k];
+        int32_t* flabels = labels + (size_t)rfield[r] * H * W;     // global kept index k + 1; seg_finalize_kernel rebases it
         __syncwarp();
         const float yv = vy[(size_t)r * SEG_RAYS + lane], xv = vx[(size_t)r * SEG_RAYS + lane];
         s_v[wib][0][lane] = yv; s_v[wib][1][lane] = xv;
@@ -1400,16 +1494,25 @@ __global__ void __launch_bounds__(256) seg_render_kernel(const float* __restrict
                 const float q2 = ((float)yy - cyf) * ((float)yy - cyf) + ((float)xx - cxf) * ((float)xx - cxf);
                 if (q2 > rout2) continue;
                 if (q2 < rin2 || seg_pnpoly(s_v[wib][1], s_v[wib][0], (double)xx, (double)yy))
-                    atomicMin(labels + (size_t)yy * W + xx, k + 1);
+                    atomicMin(flabels + (size_t)yy * W + xx, k + 1);
             }
         (void)bw;
     }
 }
 
-__global__ void seg_finalize_kernel(int32_t* __restrict__ labels, size_t n) {
+// field blockIdx.y: background -> 0, label k + 1 of the global kept order -> rank within the field + 1; n_inst [F]
+__global__ void seg_finalize_kernel(int32_t* __restrict__ labels, size_t n, const int* __restrict__ kstart,
+                                    int32_t* __restrict__ n_inst) {
+    const int f = blockIdx.y;
+    labels += (size_t)f * n;
+    const int base = kstart[f];
+    if (n_inst && blockIdx.x == 0 && threadIdx.x == 0) n_inst[f] = kstart[f + 1] - base;
     const size_t stride = (size_t)gridDim.x * blockDim.x;
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-        if (labels[i] == SEG_EMPTY) labels[i] = 0;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int32_t v = labels[i];
+        if (v == SEG_EMPTY) labels[i] = 0;
+        else if (base) labels[i] = v - base;
+    }
 }
 
 __global__ void seg_details_kernel(const float* __restrict__ vy, const float* __restrict__ vx, const int* __restrict__ pyx,
@@ -1434,7 +1537,7 @@ int launch_seg_conv(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
     if (first_use(h, (const void*)kern))
         CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_B));
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
-    int grid = tiles_x * tiles_y * a.groups;
+    int grid = tiles_x * tiles_y * a.F * a.groups;
     if (grid > C::CTAS_PER_SM * h->num_sms) grid = C::CTAS_PER_SM * h->num_sms;
     kern<<<grid, 256, C::SMEM_B, s>>>(a);
     CIA_LAUNCH_CHECK();
@@ -1456,9 +1559,9 @@ int launch_seg_conv_tma(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
         return (SegTensorMapEncodeFn)fn;
     }();
     if (!encode) { h->err = "cuTensorMapEncodeTiled is not available from this driver"; return CIA_E_UNSUPPORTED; }
-    // chunk-planar fp16 activations [4 planes][H][W][8]: dims (8, x, y, plane); out-of-bounds reads give zeros
+    // chunk-planar fp16 activations [F][4 planes][H][W][8]: dims (8, x, y, field * 4 + plane); out-of-bounds reads give zeros
     CUtensorMap tm;
-    const cuuint64_t dims[4] = {8, (cuuint64_t)a.W, (cuuint64_t)a.H, 4};
+    const cuuint64_t dims[4] = {8, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)4 * a.F};
     const cuuint64_t strides[3] = {16, (cuuint64_t)16 * a.W, (cuuint64_t)16 * a.W * a.H};
     const cuuint32_t box[4] = {8, (cuuint32_t)C::COLS, 18, 4};
     const cuuint32_t estr[4] = {1, 1, 1, 1};
@@ -1471,9 +1574,9 @@ int launch_seg_conv_tma(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
     if (first_use(h, (const void*)kern))
         CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM_B));
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
-    int grid = tiles_x * tiles_y;
+    int grid = tiles_x * tiles_y * a.F;
     if (grid > h->num_sms) grid = h->num_sms;
-    kern<<<grid, T::THREADS, T::SMEM_B, s>>>(tm, a.w, a.bias, a.out, a.out_pool, a.H, a.W);
+    kern<<<grid, T::THREADS, T::SMEM_B, s>>>(tm, a.w, a.bias, a.out, a.out_pool, a.H, a.W, a.F);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
@@ -1485,7 +1588,7 @@ int launch_seg_conv_ws(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
     if (first_use(h, (const void*)kern))
         CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM_B));
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
-    int grid = tiles_x * tiles_y * a.groups;
+    int grid = tiles_x * tiles_y * a.F * a.groups;
     if (grid > h->num_sms) grid = h->num_sms;
     kern<<<grid, T::THREADS, T::SMEM_B, s>>>(a);
     CIA_LAUNCH_CHECK();
@@ -1504,7 +1607,7 @@ int launch_seg_heads_tma(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
     }();
     if (!encode) { h->err = "cuTensorMapEncodeTiled is not available from this driver"; return CIA_E_UNSUPPORTED; }
     CUtensorMap tm;
-    const cuuint64_t dims[4] = {8, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)T::PLANES};
+    const cuuint64_t dims[4] = {8, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)T::PLANES * a.F};   // field * PLANES + plane
     const cuuint64_t strides[3] = {16, (cuuint64_t)16 * a.W, (cuuint64_t)16 * a.W * a.H};
     const cuuint32_t box[4] = {8, 16, 16, (cuuint32_t)T::PLANES};
     const cuuint32_t estr[4] = {1, 1, 1, 1};
@@ -1516,9 +1619,9 @@ int launch_seg_heads_tma(cia_ctx* h, const SegConvArgs& a, cudaStream_t s) {
     auto kern = seg_heads_tma_kernel<128>;
     if (first_use(h, (const void*)kern))
         CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM_B));
-    int grid = ((a.W + 15) / 16) * ((a.H + 15) / 16);
+    int grid = ((a.W + 15) / 16) * ((a.H + 15) / 16) * a.F;
     if (grid > h->num_sms) grid = h->num_sms;
-    kern<<<grid, T::THREADS, T::SMEM_B, s>>>(tm, a.w, a.bias, a.prob, a.dist, a.H, a.W);
+    kern<<<grid, T::THREADS, T::SMEM_B, s>>>(tm, a.w, a.bias, a.prob, a.dist, a.H, a.W, a.F);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
@@ -1564,7 +1667,7 @@ int free_model(SegModel* m) {
     if (!m) return 0;
     for (auto& c : m->conv) { cudaFree(c.w_img); cudaFree(c.bias); cudaFree(c.w32); }
     cudaFree(m->ray_sin); cudaFree(m->ray_cos);
-    cudaFree(m->act.p); cudaFree(m->post.p); cudaFree(m->cubtmp.p);
+    cudaFree(m->act.p); cudaFree(m->post.p); cudaFree(m->cubtmp.p); cudaFree(m->screen.p);
     delete m;
     return 0;
 }
@@ -1726,48 +1829,58 @@ int k_seg_load(cia_ctx* h, const cia_seg_config* cfg, int n_layers, const float*
     return CIA_OK;
 }
 
-int k_seg_normalize(cia_ctx* h, const uint16_t* img, int H, int W, double pmin, double pmax, float* out,
-                    float* mi_ma_out, cudaStream_t s) {
-    // scratch: 65536-bin histogram + the two percentiles
-    int rc = ws_reserve(h, h->ws_misc, (size_t)SEG_HIST_COPIES * 65536 * sizeof(uint32_t) + 2048 * sizeof(uint32_t) + 64);
+// n_fields uint16 fields [F][H][W] -> float32 [F][Hp][Wp] (Hp >= H, Wp >= W: reflect-padded); mi_ma_out [F][2] or null
+int k_seg_normalize(cia_ctx* h, const uint16_t* img, int n_fields, int H, int W, int Hp, int Wp, double pmin, double pmax,
+                    float* out, float* mi_ma_out, cudaStream_t s) {
+    if (n_fields > 65535) { h->err = "segmentation: at most 65535 fields per call"; return CIA_E_ARG; }
+    // scratch of the handle's own (not ws_misc, which the autoencoder uses): [F] histogram copies (4 MB per field),
+    // [F][2048] sums of 32 bins, [F][2] percentiles
+    const size_t words = (size_t)n_fields * (SEG_HIST_FIELD + 2048 + 2);
+    int rc = ws_reserve(h, h->ws_seg_norm, words * sizeof(uint32_t));
     if (rc) return rc;
-    uint32_t* hist = (uint32_t*)h->ws_misc.p;
-    uint32_t* wsum = hist + (size_t)SEG_HIST_COPIES * 65536;
-    float* mima = mi_ma_out ? mi_ma_out : (float*)(wsum + 2048);
+    uint32_t* hist = (uint32_t*)h->ws_seg_norm.p;
+    uint32_t* wsum = hist + (size_t)n_fields * SEG_HIST_FIELD;
+    float* mima = mi_ma_out ? mi_ma_out : (float*)(wsum + (size_t)n_fields * 2048);
     const size_t n = (size_t)H * W;
-    CIA_CUDA(cudaMemsetAsync(hist, 0, (size_t)SEG_HIST_COPIES * 65536 * sizeof(uint32_t), s));
-    seg_hist_kernel<<<h->num_sms * 8, 256, 0, s>>>(img, n, hist);
+    CIA_CUDA(cudaMemsetAsync(hist, 0, (size_t)n_fields * SEG_HIST_FIELD * sizeof(uint32_t), s));
+    const int gx = std::max(SEG_HIST_COPIES, h->num_sms * 8 / n_fields);
+    seg_hist_kernel<<<dim3(gx, n_fields), 256, 0, s>>>(img, n, hist);
     CIA_LAUNCH_CHECK();
-    seg_hist_reduce_kernel<<<65536 / 256, 256, 0, s>>>(hist, wsum);
+    seg_hist_reduce_kernel<<<dim3(65536 / 256, n_fields), 256, 0, s>>>(hist, wsum);
     CIA_LAUNCH_CHECK();
-    seg_percentile_kernel<<<1, 1024, 0, s>>>(hist, wsum, n, pmin / 100.0, pmax / 100.0, mima);   // np.true_divide(q, 100)
+    seg_percentile_kernel<<<n_fields, 1024, 0, s>>>(hist, wsum, n, pmin / 100.0, pmax / 100.0, mima);   // np.true_divide(q, 100)
     CIA_LAUNCH_CHECK();
-    seg_normalize_kernel<<<h->num_sms * 8, 256, 0, s>>>(img, n, mima, 1e-20f, out);
+    seg_normalize_kernel<<<dim3(gx, n_fields), 256, 0, s>>>(img, H, W, Hp, Wp, mima, 1e-20f, out);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
 
-// The network: normalized float32 field [H][W] (device) -> prob [H/grid][W/grid], dist [H/grid][W/grid][32]
-int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, float* dist_out, cudaStream_t s) {
+int k_seg_div(cia_ctx* h) { return h->seg ? h->seg->grid << h->seg->depth : 0; }
+int k_seg_grid(cia_ctx* h) { return h->seg ? h->seg->grid : 0; }
+
+// The network: F normalized float32 fields [F][H][W] (device) -> prob [F][H/grid][W/grid], dist [F][H/grid][W/grid][32].
+// Every layer is one launch for all F fields; per field the arithmetic is that of a one-field call.
+int k_seg_predict(cia_ctx* h, const float* img, int F, int H, int W, float* prob_out, float* dist_out, cudaStream_t s) {
     SegModel* m = h->seg;
     if (!m) { h->err = "segmentation model not loaded (cia_seg_load)"; return CIA_E_STATE; }
+    if (F < 1) { h->err = "segmentation: n_fields must be >= 1"; return CIA_E_ARG; }
     const int div = m->grid << m->depth;
     if (H % div || W % div || H <= 0 || W <= 0) {
         h->err = "segmentation: field sides must be multiples of " + std::to_string(div) +
                  " (StarDist pads with np.pad(mode='reflect') otherwise: pad on the host)";
         return CIA_E_UNSUPPORTED;
     }
-    // activation buffers (bump allocation; no reuse: 1.4 GB for a 2048 x 2048 field)
+    // activation buffers [F][C/8][y][x][8] (bump allocation; no reuse: 1.4 GB per 2048 x 2048 field)
     std::vector<size_t> off(m->buf_ch.size());
     size_t total = 0;
     for (size_t b = 0; b < off.size(); ++b) {
         off[b] = total;
-        total += align_up((size_t)m->buf_ch[b] * (H >> m->buf_shift[b]) * (W >> m->buf_shift[b]) * sizeof(__half), 256);
+        total += align_up((size_t)F * m->buf_ch[b] * (H >> m->buf_shift[b]) * (W >> m->buf_shift[b]) * sizeof(__half), 256);
     }
     const int gs = m->grid == 1 ? 0 : (m->grid == 2 ? 1 : 2);
     const int Hg = H >> gs, Wg = W >> gs;
-    const size_t prob_off = total; total += align_up((size_t)Hg * Wg * sizeof(float), 256);
-    const size_t dist_off = total; total += align_up((size_t)Hg * Wg * SEG_RAYS * sizeof(float), 256);
+    const size_t prob_off = total; total += align_up((size_t)F * Hg * Wg * sizeof(float), 256);
+    const size_t dist_off = total; total += align_up((size_t)F * Hg * Wg * SEG_RAYS * sizeof(float), 256);
     int rc = ws_reserve(h, m->act, total);
     if (rc) return rc;
     unsigned char* base = (unsigned char*)m->act.p;
@@ -1788,7 +1901,7 @@ int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, f
         if (fuse_first && l == 1) {
             SegConvArgs a{};
             a.w = (const uint4*)c.w_img; a.bias = c.bias; a.out = out;
-            a.H = Ho; a.W = Wo; a.c0 = op.c0; a.c1 = 0; a.mode = 3; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
+            a.H = Ho; a.W = Wo; a.F = F; a.c0 = op.c0; a.c1 = 0; a.mode = 3; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
             a.img = img; a.w1 = m->conv[0].w32; a.b1 = m->conv[0].bias;
             if (c.n_tile == 128) rc = launch_seg_conv_ws<128, 2>(h, a, s);
             else if (c.n_tile == 64) rc = launch_seg_conv_ws<64, 4>(h, a, s);
@@ -1797,8 +1910,8 @@ int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, f
             continue;
         }
         if (op.mode == -1) {
-            const size_t n = (size_t)Ho * ((Wo + 1) / 2);
-            seg_first_kernel<<<(unsigned)((n + 255) / 256), 256, 10 * c.cout * sizeof(float), s>>>(img, c.w32, c.bias, out, Ho, Wo, c.cout);
+            const size_t n = (size_t)F * Ho * ((Wo + 1) / 2);
+            seg_first_kernel<<<(unsigned)((n + 255) / 256), 256, 10 * c.cout * sizeof(float), s>>>(img, c.w32, c.bias, out, Ho, Wo, c.cout, F);
             CIA_LAUNCH_CHECK();
             continue;
         }
@@ -1806,7 +1919,7 @@ int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, f
         a.src0 = (const __half*)(base + off[op.src0]);
         a.src1 = op.src1 >= 0 ? (const __half*)(base + off[op.src1]) : nullptr;
         a.w = (const uint4*)c.w_img; a.bias = c.bias; a.out = out;
-        a.H = Ho; a.W = Wo; a.c0 = op.c0; a.c1 = op.c1; a.mode = op.mode; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
+        a.H = Ho; a.W = Wo; a.F = F; a.c0 = op.c0; a.c1 = op.c1; a.mode = op.mode; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
         // pooled input already written by the producer's epilogue: read it directly (a Cin = 32 layer then runs TMA-fed too)
         if (op.mode == 1 && l > 0 && pooled_by_producer[l - 1]) {
             a.mode = 0;
@@ -1828,12 +1941,12 @@ int k_seg_predict(cia_ctx* h, const float* img, int H, int W, float* prob_out, f
         a.src0 = (const __half*)(base + off[last.dst]);
         a.w = (const uint4*)c.w_img; a.bias = c.bias;
         a.prob = m->prob_map; a.dist = m->dist_map;
-        a.H = Hg; a.W = Wg; a.c0 = c.cin; a.c1 = 0; a.mode = 0; a.ntaps = 1; a.groups = 1; a.chunks = c.chunks;
+        a.H = Hg; a.W = Wg; a.F = F; a.c0 = c.cin; a.c1 = 0; a.mode = 0; a.ntaps = 1; a.groups = 1; a.chunks = c.chunks;
         rc = launch_seg_heads(h, c, a, s);
         if (rc) return rc;
     }
-    if (prob_out) CIA_CUDA(cudaMemcpyAsync(prob_out, m->prob_map, (size_t)Hg * Wg * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    if (dist_out) CIA_CUDA(cudaMemcpyAsync(dist_out, m->dist_map, (size_t)Hg * Wg * SEG_RAYS * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (prob_out) CIA_CUDA(cudaMemcpyAsync(prob_out, m->prob_map, (size_t)F * Hg * Wg * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    if (dist_out) CIA_CUDA(cudaMemcpyAsync(dist_out, m->dist_map, (size_t)F * Hg * Wg * SEG_RAYS * sizeof(float), cudaMemcpyDeviceToDevice, s));
     return CIA_OK;
 }
 
@@ -1847,7 +1960,7 @@ int k_seg_debug_layer(cia_ctx* h, int layer, const void* src0, const void* src1,
         const SegConv& c = m->conv.back();
         SegConvArgs a{};
         a.src0 = (const __half*)src0; a.w = (const uint4*)c.w_img; a.bias = c.bias; a.prob = prob; a.dist = dist;
-        a.H = Ho; a.W = Wo; a.c0 = c.cin; a.mode = 0; a.ntaps = 1; a.groups = 1; a.chunks = c.chunks;
+        a.H = Ho; a.W = Wo; a.F = 1; a.c0 = c.cin; a.mode = 0; a.ntaps = 1; a.groups = 1; a.chunks = c.chunks;
         return launch_seg_heads(h, c, a, s);
     }
     if (layer < 0 || layer >= (int)m->ops.size()) { h->err = "segmentation: no such layer"; return CIA_E_ARG; }
@@ -1855,13 +1968,13 @@ int k_seg_debug_layer(cia_ctx* h, int layer, const void* src0, const void* src1,
     const SegConv& c = m->conv[layer];
     if (op.mode == -1) {
         const size_t n = (size_t)Ho * ((Wo + 1) / 2);
-        seg_first_kernel<<<(unsigned)((n + 255) / 256), 256, 10 * c.cout * sizeof(float), s>>>(img, c.w32, c.bias, (__half*)out, Ho, Wo, c.cout);
+        seg_first_kernel<<<(unsigned)((n + 255) / 256), 256, 10 * c.cout * sizeof(float), s>>>(img, c.w32, c.bias, (__half*)out, Ho, Wo, c.cout, 1);
         CIA_LAUNCH_CHECK();
         return CIA_OK;
     }
     SegConvArgs a{};
     a.src0 = (const __half*)src0; a.src1 = (const __half*)src1; a.w = (const uint4*)c.w_img; a.bias = c.bias; a.out = (__half*)out;
-    a.H = Ho; a.W = Wo; a.c0 = op.c0; a.c1 = op.c1; a.mode = op.mode; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
+    a.H = Ho; a.W = Wo; a.F = 1; a.c0 = op.c0; a.c1 = op.c1; a.mode = op.mode; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
     return launch_seg_layer(h, c, a, s);
 }
 
@@ -1875,23 +1988,29 @@ int k_seg_layer_info(cia_ctx* h, int layer, int* info /* [6]: mode, c0, c1, cout
     return CIA_OK;
 }
 
-// _instances_from_prediction: prob [Hg][Wg], dist [Hg][Wg][32] (device; null = the last cia_seg_predict's) ->
-// labels int32 [H][W], n_instances
-int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int Hg, int Wg, int grid, int H, int W,
-                    double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_inst_dev, cudaStream_t s) {
+// _instances_from_prediction for F fields: prob [F][Hgp][Wgp], dist [F][Hgp][Wgp][32] (device; null = the last
+// cia_seg_predict's), candidates inside the logical hg x wg part of each map -> labels int32 [F][H][W] (rank within the
+// field + 1), n_inst_dev [F].  One launch sequence for all fields: the suppression runs every field's rounds together.
+int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int F, int Hgp, int Wgp, int hg, int wg, int grid,
+                    int H, int W, double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_inst_dev, cudaStream_t s) {
     SegModel* m = h->seg;
     if (!m) { h->err = "segmentation model not loaded (cia_seg_load)"; return CIA_E_STATE; }
     if (!prob) prob = m->prob_map;
     if (!dist) dist = m->dist_map;
     if (!prob || !dist) { h->err = "segmentation: no prob / dist maps"; return CIA_E_ARG; }
-    if ((size_t)Hg * Wg >= 0x7fffffffull) { h->err = "segmentation: grid too large"; return CIA_E_UNSUPPORTED; }
-    const int cap = Hg * Wg;
-    const int nbx = (W + SEG_BIN - 1) / SEG_BIN, nby = (H + SEG_BIN - 1) / SEG_BIN, nbins = nbx * nby;
+    if (F < 1 || F > 65535 || hg > Hgp || wg > Wgp) { h->err = "segmentation: bad field count or map size"; return CIA_E_ARG; }
+    if ((size_t)F * Hgp * Wgp >= 0x7fffffffull) { h->err = "segmentation: grid too large"; return CIA_E_UNSUPPORTED; }
+    const int cap = F * Hgp * Wgp;
+    const int nbx = (W + SEG_BIN - 1) / SEG_BIN, nby = (H + SEG_BIN - 1) / SEG_BIN, nbins = F * nbx * nby;
+    const bool wide = F > 1;                        // 64-bit keys with the field above bit 32
+    int key_bits = 32;
+    while ((1 << (key_bits - 32)) < F) ++key_bits;   // 32 + ceil(log2 F)
+    const size_t kb = wide ? 8 : 4;
 
     // workspace carve-up
     size_t o = 0;
     auto take = [&](size_t bytes) { const size_t at = o; o += align_up(bytes, 256); return at; };
-    const size_t o_keys0 = take((size_t)cap * 4), o_keys1 = take((size_t)cap * 4), o_vals0 = take((size_t)cap * 4), o_vals1 = take((size_t)cap * 4);
+    const size_t o_keys0 = take((size_t)cap * kb), o_keys1 = take((size_t)cap * kb), o_vals0 = take((size_t)cap * 4), o_vals1 = take((size_t)cap * 4);
     const size_t o_binof = take((size_t)cap * 4), o_bcnt = take((size_t)(nbins + 1) * 4), o_bcur = take((size_t)(nbins + 1) * 4);
     const size_t o_vy = take((size_t)cap * SEG_RAYS * 4), o_vx = take((size_t)cap * SEG_RAYS * 4);
     const size_t o_pyx = take((size_t)cap * 8), o_pp = take((size_t)cap * 4), o_rm = take((size_t)cap * 4);
@@ -1899,10 +2018,11 @@ int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int Hg, in
     const size_t o_excl = take((size_t)cap * 4), o_kept = take((size_t)cap * 4);
     const size_t o_bins = take((size_t)(nbins + 1) * 4), o_small = take(64);
     const size_t o_brank = take((size_t)cap * 4), o_byxr = take((size_t)cap * 16), o_pos = take((size_t)cap * 4);
+    const size_t o_rfield = take((size_t)cap * 4), o_kstart = take((size_t)(F + 1) * 4);
     int rc = ws_reserve(h, m->post, o);
     if (rc) return rc;
     unsigned char* b = (unsigned char*)m->post.p;
-    unsigned* keys0 = (unsigned*)(b + o_keys0); unsigned* keys1 = (unsigned*)(b + o_keys1);
+    void* keys0 = b + o_keys0; void* keys1 = b + o_keys1;
     unsigned* vals0 = (unsigned*)(b + o_vals0); unsigned* vals1 = (unsigned*)(b + o_vals1);
     int* bin_of = (int*)(b + o_binof); int* bin_count = (int*)(b + o_bcnt); int* bin_cursor = (int*)(b + o_bcur);
     float* vy = (float*)(b + o_vy); float* vx = (float*)(b + o_vx);
@@ -1911,37 +2031,46 @@ int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int Hg, in
     int* state = (int*)(b + o_state); int* flags = (int*)(b + o_flags); int* excl = (int*)(b + o_excl);
     int* kept = (int*)(b + o_kept); int* bins = (int*)(b + o_bins);
     int* b_rank = (int*)(b + o_brank); float4* b_yxr = (float4*)(b + o_byxr); int* pos = (int*)(b + o_pos);
+    int* rfield = (int*)(b + o_rfield); int* kstart = (int*)(b + o_kstart);
     int* small = (int*)(b + o_small);         // [0] count, [1] rmax bits, [2..4] nms counters, [5] n_kept
     m->last_cap = cap; m->vy = vy; m->vx = vx; m->pprob = pp; m->pyx = pyx; m->kept_rank = kept; m->n_kept = small + 5;
 
+    typedef unsigned long long K64;
     size_t tmp_sort = 0, tmp_scan = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, tmp_sort, keys0, keys1, vals0, vals1, cap, 0, 32, s);
+    if (wide) cub::DeviceRadixSort::SortPairs(nullptr, tmp_sort, (K64*)keys0, (K64*)keys1, vals0, vals1, cap, 0, key_bits, s);
+    else cub::DeviceRadixSort::SortPairs(nullptr, tmp_sort, (unsigned*)keys0, (unsigned*)keys1, vals0, vals1, cap, 0, 32, s);
     cub::DeviceScan::ExclusiveSum(nullptr, tmp_scan, flags, excl, cap, s);
     rc = ws_reserve(h, m->cubtmp, std::max(tmp_sort, tmp_scan));
     if (rc) return rc;
     size_t tmp_bytes = m->cubtmp.cap;
 
-    CIA_CUDA(cudaMemsetAsync(keys0, 0xFF, (size_t)cap * 4, s));
+    CIA_CUDA(cudaMemsetAsync(keys0, 0xFF, (size_t)cap * kb, s));
     CIA_CUDA(cudaMemsetAsync(bin_count, 0, (size_t)(nbins + 1) * 4, s));
     CIA_CUDA(cudaMemsetAsync(state, 0, (size_t)cap * 4, s));
     CIA_CUDA(cudaMemsetAsync(small, 0, 64, s));
-    CIA_CUDA(cudaMemsetAsync(labels, 0x7F, (size_t)H * W * sizeof(int32_t), s));
-    seg_cand_flags_kernel<<<(cap + 255) / 256, 256, 0, s>>>(prob, Hg, Wg, (float)prob_thresh, 2, flags);
+    CIA_CUDA(cudaMemsetAsync(labels, 0x7F, (size_t)F * H * W * sizeof(int32_t), s));
+    seg_cand_flags_kernel<<<(cap + 255) / 256, 256, 0, s>>>(prob, F, Hgp, Wgp, hg, wg, (float)prob_thresh, 2, flags);
     CIA_LAUNCH_CHECK();
     tmp_bytes = m->cubtmp.cap;
     CIA_CUDA(cub::DeviceScan::ExclusiveSum(m->cubtmp.p, tmp_bytes, flags, excl, cap, s));
     h->launches++;
-    seg_cand_scatter_kernel<<<(cap + 255) / 256, 256, 0, s>>>(prob, flags, excl, cap, keys0, vals0, small);
-    CIA_LAUNCH_CHECK();
     tmp_bytes = m->cubtmp.cap;
-    CIA_CUDA(cub::DeviceRadixSort::SortPairs(m->cubtmp.p, tmp_bytes, keys0, keys1, vals0, vals1, cap, 0, 32, s));
+    if (wide) {
+        seg_cand_scatter_kernel<K64><<<(cap + 255) / 256, 256, 0, s>>>(prob, flags, excl, cap, Hgp * Wgp, (K64*)keys0, vals0, small);
+        CIA_LAUNCH_CHECK();
+        CIA_CUDA(cub::DeviceRadixSort::SortPairs(m->cubtmp.p, tmp_bytes, (K64*)keys0, (K64*)keys1, vals0, vals1, cap, 0, key_bits, s));
+    } else {
+        seg_cand_scatter_kernel<unsigned><<<(cap + 255) / 256, 256, 0, s>>>(prob, flags, excl, cap, Hgp * Wgp, (unsigned*)keys0, vals0, small);
+        CIA_LAUNCH_CHECK();
+        CIA_CUDA(cub::DeviceRadixSort::SortPairs(m->cubtmp.p, tmp_bytes, (unsigned*)keys0, (unsigned*)keys1, vals0, vals1, cap, 0, 32, s));
+    }
     h->launches++;
-    seg_polygons_kernel<<<(cap + 127) / 128, 128, 0, s>>>(vals1, small, cap, prob, dist, Wg, grid, m->ray_sin, m->ray_cos, H, W, vy, vx,
-                                                         pyx, pp, rm, area, bin_of, bin_count, (unsigned*)(small + 1));
+    seg_polygons_kernel<<<(cap + 127) / 128, 128, 0, s>>>(vals1, small, cap, prob, dist, Hgp, Wgp, grid, m->ray_sin, m->ray_cos, H, W,
+                                                         vy, vx, pyx, pp, rm, area, bin_of, bin_count, (unsigned*)(small + 1), rfield);
     CIA_LAUNCH_CHECK();
     seg_bins_kernel<<<1, 1024, 0, s>>>(bin_count, nbins, bins, bin_cursor);
     CIA_LAUNCH_CHECK();
-    seg_binorder_kernel<<<(cap + 255) / 256, 256, 0, s>>>(bin_of, bin_cursor, small, cap, pyx, rm, b_rank, b_yxr, pos);
+    seg_binorder_kernel<<<(cap + 255) / 256, 256, 0, s>>>(bin_of, bin_cursor, small, cap, pyx, rm, rfield, b_rank, b_yxr, pos);
     CIA_LAUNCH_CHECK();
     {
         NmsArgs a{};
@@ -1961,13 +2090,23 @@ int k_seg_instances(cia_ctx* h, const float* prob, const float* dist, int Hg, in
     tmp_bytes = m->cubtmp.cap;
     CIA_CUDA(cub::DeviceScan::ExclusiveSum(m->cubtmp.p, tmp_bytes, flags, excl, cap, s));
     h->launches++;
-    seg_compact_kernel<<<(cap + 255) / 256, 256, 0, s>>>(flags, excl, cap, kept, small + 5);
+    seg_compact_kernel<<<(cap + 255) / 256, 256, 0, s>>>(flags, excl, cap, small, rfield, F, kept, small + 5, kstart);
     CIA_LAUNCH_CHECK();
-    seg_render_kernel<<<h->num_sms * 8, 256, 0, s>>>(vy, vx, pyx, kept, small + 5, H, W, labels);
+    seg_render_kernel<<<h->num_sms * 8, 256, 0, s>>>(vy, vx, pyx, kept, small + 5, rfield, H, W, labels);
     CIA_LAUNCH_CHECK();
-    seg_finalize_kernel<<<h->num_sms * 8, 256, 0, s>>>(labels, (size_t)H * W);
+    seg_finalize_kernel<<<dim3(std::max(1, h->num_sms * 8 / F), F), 256, 0, s>>>(labels, (size_t)H * W, kstart, n_inst_dev);
     CIA_LAUNCH_CHECK();
-    if (n_inst_dev) CIA_CUDA(cudaMemcpyAsync(n_inst_dev, small + 5, sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+    return CIA_OK;
+}
+
+int k_seg_screen_buffers(cia_ctx* h, size_t norm_bytes, size_t label_bytes, float** norm, int32_t** labels) {
+    SegModel* m = h->seg;
+    if (!m) { h->err = "segmentation model not loaded (cia_seg_load)"; return CIA_E_STATE; }
+    const size_t lo = align_up(norm_bytes, 256);
+    const int rc = ws_reserve(h, m->screen, lo + label_bytes);
+    if (rc) return rc;
+    *norm = (float*)m->screen.p;
+    *labels = (int32_t*)((unsigned char*)m->screen.p + lo);
     return CIA_OK;
 }
 

@@ -158,12 +158,73 @@ class GpuFieldScorer:
         return total, out
 
 
+    def score_images(self, fields, strains, n_strains, prob_thresh: float, nms_thresh: float, max_label: int = 4096):
+        """``score`` for fields given as (seg channel, green channel) uint16 [H,W] pairs (or zero-argument callables
+        returning one; None = the loader gave up on the file): each chunk is segmented AND screened on the device
+        through ``BatchScreen.run_images_host`` (StarDist model loaded on the engine), so only the images cross PCIe
+        and the loader threads make no GPU calls.  ``max_label`` bounds the instances of one field (CIA_E_LABEL
+        beyond).  Returns what ``score`` returns."""
+        from concurrent.futures import ThreadPoolExecutor
+        from .batch import BatchScreen
+        dev = self.eng.tdev
+        total = torch.zeros((n_strains, ACC_COLS), dtype=torch.float64, device=dev)
+        if not fields:
+            return total, []
+        empty = lambda: {**{k: np.zeros(0) for k in ROW_KEYS}, "label": np.zeros(0, np.int32)}
+        out = []
+        chunks = [list(range(c0, min(c0 + self.Fc, len(fields)))) for c0 in range(0, len(fields), self.Fc)]
+        resolve = lambda f: f() if callable(f) else f
+        with ThreadPoolExecutor(max_workers=min(8, self.Fc)) as pool:
+            pending = [pool.submit(resolve, fields[i]) for i in chunks[0]]
+            for ci, idx in enumerate(chunks):
+                chunk = [p.result() for p in pending]
+                pending = [pool.submit(resolve, fields[i]) for i in chunks[ci + 1]] if ci + 1 < len(chunks) else []
+                ok = [j for j, f in enumerate(chunk) if f is not None]
+                if not ok:
+                    out.extend(empty() for _ in chunk)
+                    continue
+                H, W = chunk[ok[0]][1].shape
+                bs = self._bs
+                if bs is None or (bs.H, bs.W, bs.n_strains, bs.max_label) != (H, W, n_strains, max_label):
+                    if bs is not None:
+                        bs.sync()
+                    bs = BatchScreen(self.eng, H, W, max_label, chunk_fields=self.Fc, n_strains=n_strains)
+                    self._g = torch.zeros((self.Fc, H, W), dtype=torch.int16).pin_memory()
+                    self._s = torch.zeros((self.Fc, H, W), dtype=torch.int16).pin_memory()
+                    self._bs = bs
+                bs.acc.zero_()
+                same = all(chunk[j][0] is chunk[j][1] for j in ok)     # single-channel fields: one upload
+                for k, j in enumerate(ok):
+                    seg, g = chunk[j]
+                    if seg.shape != (H, W) or g.shape != (H, W):
+                        raise ValueError("a chunk needs equally sized fields (pad or group by size)")
+                    if g.dtype != np.uint16 or seg.dtype not in (np.uint16, np.uint8):
+                        raise TypeError("fields must be uint16 (widen 8-bit fields before screening)")
+                    self._g[k].copy_(torch.from_numpy(np.ascontiguousarray(g).view(np.int16)))
+                    if not same:
+                        self._s[k].copy_(torch.from_numpy(np.ascontiguousarray(seg, np.uint16).view(np.int16)))
+                st = torch.tensor([strains[idx[j]] for j in ok], dtype=torch.int32)
+                bs.run_images_host(self._g if same else self._s, self._g, len(ok), prob_thresh, nms_thresh, st.to(dev))
+                r = bs.collect_host()                          # synchronises, raises on a device-side status
+                total += bs.acc
+                starts = np.concatenate([[0], np.cumsum(r["field_counts"])])
+                rows = {}
+                for k, j in enumerate(ok):
+                    s0, s1 = int(starts[k]), int(starts[k + 1])
+                    rows[j] = {kk: r[kk][s0:s1].copy() for kk in ROW_KEYS}
+                    rows[j]["label"] = r["cells"]["label"][s0:s1].copy()
+                out.extend(rows.get(j) or empty() for j in range(len(chunk)))
+        return total, out
+
+
 class ShardedScreen:
     """Shards a list of fields over the ranks of the current process group, scores each rank's share
     and assembles the global result.  ``scorer.score(fields, strains, n_strains) -> (acc, rows)``."""
 
-    def __init__(self, scorer):
+    def __init__(self, scorer, score=None):
+        """``score``: the scorer's method to call (default ``scorer.score``; e.g. a bound ``score_images``)."""
         self.scorer = scorer
+        self.score = score or scorer.score
         self.rank, self.world = _world()
 
     def screen(self, load_field, n_fields: int, field_strain, n_strains: int):
@@ -174,7 +235,7 @@ class ShardedScreen:
         (``None`` on the other ranks)."""
         mine = shard_fields(n_fields, self.rank, self.world)
         fields = [(lambda i=i: load_field(i)) for i in mine]       # resolved chunk by chunk by the scorer
-        acc, rows = self.scorer.score(fields, [int(field_strain[i]) for i in mine], n_strains)
+        acc, rows = self.score(fields, [int(field_strain[i]) for i in mine], n_strains)
         acc = allreduce_strain_acc(acc)                       # the path's only collective
         local = [(i, r) for i, r in zip(mine, rows)]
         if self.world > 1:
@@ -203,7 +264,10 @@ def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, 
     from every rank of an initialised process group (one process per GPU; ``screener`` built on that
     rank's device).  Files are enumerated like the reference (strains in dict order, ``sorted(glob)``),
     sharded round robin, read and segmented on their rank, scored through the fused path; the
-    per-strain numbers come from the all-reduced accumulator.  Returns ``(results, detailed_results)``
+    per-strain numbers come from the all-reduced accumulator.  With a GPU StarDist model (``stardist_dir=``)
+    the loader threads only read files and split channels; segmentation and screening run per chunk in
+    ``cia_screen_images`` on the rank's stream (no labels through the host).  A caller's own ``segmenter``
+    keeps the (green, labels) route.  Returns ``(results, detailed_results)``
     on rank 0 -- same keys as det:202-212 / 225-234 -- and ``({}, [])`` elsewhere."""
     rank, world = _world()
     names, files, strain_of = [], [], []
@@ -218,6 +282,18 @@ def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, 
         strain_of.extend([len(names) - 1] * len(tif))
     if not files:
         return {}, []
+
+    sd_model = screener.stardist_model
+
+    def load_images(i):
+        try:
+            image = screener.imread(files[i])
+            if image.ndim == 3 and image.shape[-1] >= 3:                  # det:54-59
+                return np.ascontiguousarray(image[..., 2]), np.ascontiguousarray(image[..., 1])
+            return image, image
+        except Exception as e:                                            # det:113-115: the file contributes no cells
+            print(f"Error processing {files[i]}: {e}")
+            return None
 
     def load(i):
         try:
@@ -234,8 +310,14 @@ def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, 
             print(f"Error processing {files[i]}: {e}")
             return None
 
-    sh = ShardedScreen(GpuFieldScorer(screener.engine, chunk_fields=chunk_fields))
-    acc, rows = sh.screen(load, len(files), strain_of, len(names))
+    scorer = GpuFieldScorer(screener.engine, chunk_fields=chunk_fields)
+    if sd_model is not None:
+        th = sd_model.thresholds
+        sh = ShardedScreen(scorer, lambda f, st, ns: scorer.score_images(f, st, ns, th["prob"], th["nms"]))
+        acc, rows = sh.screen(load_images, len(files), strain_of, len(names))
+    else:
+        sh = ShardedScreen(scorer)
+        acc, rows = sh.screen(load, len(files), strain_of, len(names))
     if rank != 0:
         return {}, []
     results, detailed = {}, []

@@ -313,6 +313,25 @@ class Engine:
             C.byref(sc), _ptr(out["crops"]), _ptr(out["features"]), _ptr(field_strain), _ptr(acc), ns,
             self._stream()))
 
+    def screen_images(self, seg_images: torch.Tensor, images: torch.Tensor, max_label: int, out: dict,
+                      prob_thresh: float, nms_thresh: float, n_instances: torch.Tensor = None,
+                      labels_out: torch.Tensor = None, field_strain: torch.Tensor = None, acc: torch.Tensor = None,
+                      precision=None):
+        """``screen_fields`` with the labels made on the device from ``seg_images`` (uint16 [F, H, W], may be
+        ``images`` itself): batched StarDist segmentation (needs ``cia_seg_load``) then the fused path, no host
+        sync.  ``n_instances`` int32 [F] and ``labels_out`` int32 [F, H, W] are optional device outputs."""
+        F, H, W = images.shape
+        if tuple(seg_images.shape) != (F, H, W):
+            raise ValueError(f"seg_images {tuple(seg_images.shape)} and images {(F, H, W)} differ in shape")
+        sc = self._scores(out)
+        prec = self.precision if precision is None else precision
+        ns = 0 if acc is None else acc.shape[0]
+        self._check(self.lib.cia_screen_images(
+            self.h, _ptr(seg_images), _ptr(images), F, H, W, float(prob_thresh), float(nms_thresh), max_label,
+            C.byref(self.params), prec, _ptr(out["cells"]), out["cap"], _ptr(out["counts"]),
+            C.c_void_p(out["counts"].data_ptr() + 4), C.byref(sc), _ptr(out["crops"]), _ptr(out["features"]),
+            _ptr(field_strain), _ptr(acc), ns, _ptr(n_instances), _ptr(labels_out), self._stream()))
+
     def screen_fields_host(self, images: np.ndarray, labels: np.ndarray, max_label: int,
                            cells_cap: int, precision=None):
         """Host buffers in, host results out (H2D + D2H inside the call; synchronises)."""
@@ -564,13 +583,16 @@ class ProductionMutantScreening:
         from .distributed import screen_mutant_samples_sharded
         return screen_mutant_samples_sharded(self, test_folders_dict, output_dir, chunk_fields)
 
-    def screen_images(self, images, cells_cap_per_field: int = 4096, prob_thresh=None, nms_thresh=None):
-        """det:51-153 for a batch of single-channel uint16 fields with NOTHING but the images given: per field
-        normalize -> U-Net -> instances (csrc/segment.cu) -> region scan -> gates -> crops -> autoencoder -> SVMs, all
-        enqueued on one stream (the labels never leave the device, no host synchronisation inside the loop; one at
-        the end).  Needs ``stardist_dir=`` (or ``self.stardist_model``).  Returns per-cell arrays in (field, ascending
-        label) order: ``field``, ``label``, ``reconstruction_mse`` / ``_mae``, ``conservative_scores`` /
-        ``moderate_scores`` (negated decisions, det:149-150), ``*_predictions``, and ``n_instances`` per field."""
+    def screen_images(self, images, cells_cap_per_field: int = 4096, prob_thresh=None, nms_thresh=None,
+                      seg_images=None, chunk_fields: int = 16):
+        """det:51-153 for a batch of uint16 fields with NOTHING but the images given: normalize -> U-Net -> instances
+        (csrc/segment.cu) -> region scan -> gates -> crops -> autoencoder -> SVMs through ``cia_screen_images``, up to
+        ``chunk_fields`` fields per call, all enqueued on one stream (the labels never leave the device; one host
+        synchronisation at the end).  ``seg_images`` (same shape) is the segmentation channel when it differs from the
+        analysis channel (det:54-59); default: ``images`` itself.  Needs ``stardist_dir=`` (or ``self.stardist_model``).
+        At most ``cells_cap_per_field`` instances per field.  Returns per-cell arrays in (field, ascending label) order:
+        ``field``, ``label``, ``reconstruction_mse`` / ``_mae``, ``conservative_scores`` / ``moderate_scores`` (negated
+        decisions, det:149-150), ``*_predictions``, and ``n_instances`` per field."""
         m = self.stardist_model
         if m is None:
             raise RuntimeError("screen_images needs the GPU segmentation: construct with stardist_dir=<model folder>")
@@ -578,35 +600,28 @@ class ProductionMutantScreening:
         imgs = np.ascontiguousarray(images)
         if imgs.dtype != np.uint16 or imgs.ndim != 3:
             raise UnsupportedImageError(f"screen_images takes uint16 [F, H, W] fields, got {imgs.dtype} {imgs.shape}")
+        segs = imgs if seg_images is None else np.ascontiguousarray(seg_images)
+        if segs.dtype != np.uint16 or segs.shape != imgs.shape:
+            raise UnsupportedImageError(f"seg_images must be uint16 {imgs.shape}, got {segs.dtype} {segs.shape}")
         F, H, W = imgs.shape
         cap = int(cells_cap_per_field)
-        dev = torch.from_numpy(imgs.view(np.int16)).to(eng.tdev)
-        outs = [eng.alloc_outputs(cap, 1) for _ in range(F)]
-        n_inst = torch.zeros(F, dtype=torch.int32, device=eng.tdev)
-        x = torch.empty((H, W), dtype=torch.float32, device=eng.tdev)
         pt = m.thresholds["prob"] if prob_thresh is None else prob_thresh
         nt = m.thresholds["nms"] if nms_thresh is None else nms_thresh
-        labels = torch.empty((H, W), dtype=torch.int32, device=eng.tdev)
-        padded = (-H % m.div_by, -W % m.div_by) != (0, 0)
-        for f in range(F):
-            eng._check(eng.lib.cia_seg_normalize(eng.h, _ptr(dev[f]), H, W, 3.0, 99.8, _ptr(x), C.c_void_p(0), eng._stream()))
-            if padded:                       # StarDist's reflect padding (host-side mirror of the device tensor ops)
-                prob, dist = m.predict(x)
-                lab, cnt = m.instances_from_prediction((H, W), prob, dist, pt, nt, sync=False)
-                labels.copy_(lab)
-                n_inst[f:f + 1].copy_(cnt)
-            else:
-                eng._check(eng.lib.cia_seg_predict(eng.h, _ptr(x), H, W, C.c_void_p(0), C.c_void_p(0), eng._stream()))
-                eng._check(eng.lib.cia_seg_instances(eng.h, C.c_void_p(0), C.c_void_p(0), H // m.grid, W // m.grid, m.grid,
-                                                     H, W, float(pt), float(nt), _ptr(labels), _ptr(n_inst[f:f + 1]),
-                                                     eng._stream()))
-            eng.screen_fields(dev[f:f + 1], labels.view(1, H, W), cap, outs[f])
+        dev = torch.from_numpy(imgs.view(np.int16)).to(eng.tdev)
+        sdev = dev if segs is imgs else torch.from_numpy(segs.view(np.int16)).to(eng.tdev)
+        n_inst = torch.zeros(F, dtype=torch.int32, device=eng.tdev)
+        outs = []
+        for f0 in range(0, F, chunk_fields):
+            nf = min(chunk_fields, F - f0)
+            o = eng.alloc_outputs(cap * nf, nf)
+            eng.screen_images(sdev[f0:f0 + nf], dev[f0:f0 + nf], cap, o, pt, nt, n_instances=n_inst[f0:f0 + nf])
+            outs.append((f0, o))
         eng.check_status()                   # synchronises; raises on capacity / label overflow
         cols = {k: [] for k in ("field", "label", "mse", "mae", "dec_cons", "dec_mod", "pred_cons", "pred_mod")}
-        for f, o in enumerate(outs):
+        for f0, o in outs:
             n = int(o["counts"][0].item())
             rec = o["cells"][:n].cpu().numpy().view(_lib.CELL_DTYPE).reshape(-1)
-            cols["field"].append(np.full(n, f, np.int64))
+            cols["field"].append(f0 + rec["field"].astype(np.int64))
             cols["label"].append(rec["label"].astype(np.int64))
             for k in ("mse", "mae", "dec_cons", "dec_mod", "pred_cons", "pred_mod"):
                 cols[k].append(o[k][:n].cpu().numpy())

@@ -308,6 +308,43 @@ class StarDist2D:
         details = self.details(n)
         return (labels if return_device else labels.cpu().numpy()), details
 
+    def segment_fields(self, seg_images, prob_thresh=None, nms_thresh=None):
+        """normalize + predict_instances of F equally sized fields in one launch sequence per stage: uint16 [F, H, W]
+        (NumPy or a cuda tensor; uint8 is widened) -> (labels int32 cuda [F, H, W], n_instances int32 cuda [F]), each
+        field equal bit for bit to ``segment_device`` of that field (reflect padding is done on the device)."""
+        eng = self.engine
+        if isinstance(seg_images, torch.Tensor):
+            t = seg_images
+            if t.dtype == torch.uint8:
+                t = t.to(torch.int16)
+            elif t.dtype == torch.uint16:
+                t = t.view(torch.int16)
+            elif t.dtype != torch.int16:       # int16: raw uint16 bits, as the rest of this package passes them
+                raise TypeError(f"segment_fields takes uint16 / uint8 fields, got {t.dtype}")
+            d = t.to(eng.tdev).contiguous()
+        else:
+            x = np.ascontiguousarray(seg_images)
+            if x.dtype == np.uint8:
+                x = x.astype(np.uint16)
+            if x.dtype != np.uint16:
+                raise TypeError(f"segment_fields takes uint16 / uint8 fields, got {x.dtype}")
+            d = torch.from_numpy(x.view(np.int16)).to(eng.tdev)
+        if d.ndim != 3:
+            raise ValueError(f"segment_fields takes [F, H, W] fields, got shape {tuple(d.shape)}")
+        F, H, W = d.shape
+        pt = self.thresholds["prob"] if prob_thresh is None else prob_thresh
+        nt = self.thresholds["nms"] if nms_thresh is None else nms_thresh
+        Hp, Wp = H + (-H % self.div_by), W + (-W % self.div_by)
+        x = torch.empty((F, Hp, Wp), dtype=torch.float32, device=eng.tdev)
+        labels = torch.empty((F, H, W), dtype=torch.int32, device=eng.tdev)
+        n = torch.zeros(F, dtype=torch.int32, device=eng.tdev)
+        s = eng._stream()
+        eng._check(eng.lib.cia_seg_normalize_fields(eng.h, _ptr(d), F, H, W, 3.0, 99.8, _ptr(x), s))
+        eng._check(eng.lib.cia_seg_predict_fields(eng.h, _ptr(x), F, Hp, Wp, None, None, s))
+        eng._check(eng.lib.cia_seg_instances_fields(eng.h, None, None, F, Hp // self.grid, Wp // self.grid, self.grid, H, W,
+                                                    float(pt), float(nt), _ptr(labels), _ptr(n), s))
+        return labels, n
+
     def segment_device(self, seg_channel):
         """normalize + predict_instances with everything resident: uint16 field -> int32 cuda labels, n."""
         x = self.normalize_device(seg_channel)

@@ -382,6 +382,44 @@ int cia_seg_instances(cia_handle h, const float* prob, const float* dist, int Hg
 /* `details` of the last cia_seg_instances for the first `cap` kept polygons, in label order:
  * points int32 [cap][2] (y, x), prob float32 [cap], coord float32 [cap][2][n_rays]. */
 int cia_seg_details(cia_handle h, int cap, int32_t* points, float* prob, float* coord, void* stream);
+/* ---- F equally sized fields per call (the calls above are the F = 1 case of the same kernels) ----
+ * Every stage runs all F fields in one launch sequence: the number of launches does not depend on F, and per
+ * field the arithmetic (and its order) is that of the one-field call, so the outputs equal it bit for bit.
+ * Fields of different sizes go to separate calls.  Device memory held by the handle per field (grow-only):
+ *   normalisation   4.2 MB (per-field histograms; its own workspace, not shared with the screen)
+ *   U-Net           sum over the plan's buffers of C * (Hp/2^s) * (Wp/2^s) * 2 bytes + prob / dist maps:
+ *                   1.4 GB for a 2048 x 2048 field with 2D_versatile_fluo
+ *   instances       352 bytes per map pixel of Hp/grid x Wp/grid (0.37 GB for a 2048 x 2048 field, grid 2)
+ *   cia_screen_images  additionally Hp * Wp * 4 (normalized field) and, when labels_out is NULL, H * W * 4
+ *
+ * cia_seg_normalize_fields  csbdeep normalize of each field by ITS OWN percentiles (images uint16 [F][H][W]),
+ *                    written reflect-padded to out float32 [F][Hp][Wp], Hp / Wp the next multiples of
+ *                    grid * 2^depth of the loaded model (np.pad(mode='reflect') of the normalized field, what
+ *                    StarDist pads with).  CIA_E_STATE without a loaded model.
+ * cia_seg_predict_fields   the network on images float32 [F][Hp][Wp] (Hp, Wp multiples of grid * 2^depth):
+ *                    prob float32 [F][Hp/g][Wp/g], dist float32 [F][Hp/g][Wp/g][n_rays]; either may be NULL (the
+ *                    maps stay in the handle for cia_seg_instances_fields).
+ * cia_seg_instances_fields _instances_from_prediction per field on maps [F][Hgp][Wgp] (padded: candidates only
+ *                    inside each field's ceil(H/grid) x ceil(W/grid) part, the 2-pixel border measured from
+ *                    that edge); prob / dist NULL = the maps of the last predict call.  labels int32 [F][H][W]
+ *                    numbered per field (1..n_instances[f]); n_instances device int32 [F] (may be NULL).
+ * cia_screen_images  det:51-153 for F fields given nothing but images: the three calls above (pmin 3, pmax 99.8)
+ *                    on seg_images, then the cia_screen_fields path on `images` with those labels, with no host
+ *                    synchronisation.  seg_images may equal images (single-channel fields, det:57-59).
+ *                    max_label bounds the instances of one field: a field with more is reported as CIA_E_LABEL by
+ *                    cia_check_status, nothing is written out of bounds.  labels_out (may be NULL): int32 [F][H][W]. */
+int cia_seg_normalize_fields(cia_handle h, const uint16_t* images, int n_fields, int H, int W, double pmin, double pmax,
+                             float* out, void* stream);
+int cia_seg_predict_fields(cia_handle h, const float* images, int n_fields, int Hp, int Wp, float* prob, float* dist,
+                           void* stream);
+int cia_seg_instances_fields(cia_handle h, const float* prob, const float* dist, int n_fields, int Hgp, int Wgp, int grid,
+                             int H, int W, double prob_thresh, double nms_thresh, int32_t* labels, int32_t* n_instances,
+                             void* stream);
+int cia_screen_images(cia_handle h, const uint16_t* seg_images, const uint16_t* images, int n_fields, int H, int W,
+                      double prob_thresh, double nms_thresh, int max_label, const cia_params* params, int precision,
+                      cia_cell* cells, int cells_cap, int32_t* n_cells_dev, int32_t* field_counts_dev,
+                      const cia_scores* scores, float* crops32, float* features, const int32_t* field_strain,
+                      double* acc, int n_strains, int32_t* n_instances_dev, int32_t* labels_out, void* stream);
 /* Test taps: the plan entry of a layer (info[6] = mode {-1 first, 0 direct, 1 pooled, 2 up ++ skip}, c0, c1, cout,
  * log2 of the resolution divisor, number of 3x3 layers) and one layer run on caller-provided fp16 chunk-planar
  * activations [C/8][H][W][8] (layer -2 = the heads). */
