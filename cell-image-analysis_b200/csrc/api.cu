@@ -55,13 +55,6 @@ int cia_create(int device, cia_handle* out) {
         delete h;
         return CIA_E_CUDA;
     }
-    // run-time defaults of the options (A/B scripts): see cia_set_option
-    if (const char* e = getenv("CIA_CAE_CHUNK")) { const int v = atoi(e); if (v > 0) h->cae_pass_cells = v; }
-    if (const char* e = getenv("CIA_L1_DEBIAS")) h->cae_debias[0] = (float)atof(e);
-    if (const char* e = getenv("CIA_L2_DEBIAS")) h->cae_debias[1] = (float)atof(e);
-    if (const char* e = getenv("CIA_L3_DEBIAS")) h->cae_debias[2] = (float)atof(e);
-    if (const char* e = getenv("CIA_SVM_KERNEL")) h->svm_kernel = atoi(e) ? 1 : 0;
-    if (const char* e = getenv("CIA_PCA_KERNEL")) h->pca_kernel = atoi(e) ? 1 : 0;
     *out = h;
     return CIA_OK;
 }
@@ -89,8 +82,6 @@ int cia_set_option(cia_handle h, const char* name, double value) {
         h->seg_conv_tma = value != 0;
     } else if (n == "seg_pool_out") {
         h->seg_pool_out = value != 0;
-    } else if (n == "seg_fuse_first") {
-        h->seg_fuse_first = value != 0;
     } else if (n == "seg_conv_ws") {
         // segmentation: the warp-specialised software-producer kernel: 1 = for the layers where it measured faster, 2 = every
         // layer the TMA kernel does not take, 0 = the staged kernel
@@ -121,7 +112,7 @@ int cia_destroy(cia_handle h) {
     cudaDeviceSynchronize();
     free_cae(h->cae[0]); free_cae(h->cae[1]);
     k_seg_free(h);
-    cudaFree(h->sp.center); cudaFree(h->sp.scale); cudaFree(h->sp.rscale); cudaFree(h->sp.comp_t); cudaFree(h->sp.comp_pad); cudaFree(h->sp.offset); cudaFree(h->sp.tc_img); cudaFree(h->sp.tc_par);
+    cudaFree(h->sp.center); cudaFree(h->sp.scale); cudaFree(h->sp.rscale); cudaFree(h->sp.comp_pad); cudaFree(h->sp.offset); cudaFree(h->sp.tc_img); cudaFree(h->sp.tc_par);
     for (int i = 0; i < 2; ++i) { cudaFree(h->svm[i].sv_t); cudaFree(h->svm[i].coef); cudaFree(h->svm[i].sv_pad); cudaFree(h->svm[i].gsn);
                                   cudaFree(h->svm[i].tc_hi); cudaFree(h->svm[i].tc_lo); cudaFree(h->svm[i].tc_gcol); }
     Workspace* ws[] = {&h->ws_flags, &h->ws_act, &h->ws_crop_scratch, &h->ws_pipe, &h->ws_feat,
@@ -234,7 +225,6 @@ int cia_load_scaler_pca(cia_handle h, int F, int C, const double* center, const 
     std::vector<double> t((size_t)F * C);
     for (int c = 0; c < C; ++c)
         for (int f = 0; f < F; ++f) t[(size_t)f * C + c] = components[(size_t)c * F + f];
-    if ((rc = upload(h, &sp.comp_t, t.data(), t.size()))) return rc;
     {
         const int FP = (F + 31) / 32 * 32, CP = (C + 103) / 104 * 104;
         std::vector<double> tp((size_t)FP * CP, 0.0);

@@ -17,16 +17,19 @@
 // fp32-grade encoder features: operands are split x = hi + lo (two fp16), weights scaled by
 // a power of two; three MMAs (hi*hi, hi*lo, lo*hi) accumulate into one fp32 TMEM tile.
 //
-// Default pass (precision 1), one launch per layer over up to cae_pass_cells (18944) cells:
+// One kernel per layer and path, one launch per layer over up to cae_pass_cells (18944) cells.
+// Split-precision encoder (precision 1 and 3 unless a separate encoder is loaded; precision 3 runs L3 as below):
 //   L1  1->32 @64  conv1_tc_split_kernel         K = 9 im2col rows built by byte permutes, 3 MMAs per phase, writes hi/lo fp16
-//                  (conv1_fp32_planar_kernel, exact fp32 on the CUDA cores: CIA_L1_KERNEL=0 and precision 2)
 //   L2 32->64 @32  conv_tc_acc2_kernel<..,32,3>  TMA-fed double-buffered half-cell blocks, 3 taps per flush
 //   L3 64->32 @16  conv_tc_acc_kernel<..,16,1>   row-pair tiles, N-stacked weights, register-staged, 1 tap per flush -> features
+// Single-pass encoder (precision 2, a separately loaded encoder; precision 3's L3, its features from an exact fp32 L3):
+//   L1  1->32 @64  conv1_fp32_planar_kernel      exact fp32 on the CUDA cores, writes hi fp16
+//   L2, L3         conv_tc_kernel<EPI_POOL>      four pooling-phase tiles
+// Decoder (every path):
 //   L4 32->32 @8   conv_tc_kernel<EPI_PLAIN>     single pass, TMEM double-buffered
 //   L5 32->64 @16  conv_tc_kernel<EPI_PLAIN,UPSIN> up-sampling folded into the staging
 //   L6 64->32 @32  conv_tc_kernel<EPI_PHASE>     phase form at 16x16, N = 128
 //   L7 32->1  @64  final_tapsum_kernel           one tap, (phase, neighbour) pairs on N, shifted tap sum + sigmoid + MSE/MAE
-//                  (conv_tc_kernel<EPI_FINAL>, the nine-tap phase form: CIA_L7_KERNEL=0)
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -40,43 +43,20 @@ namespace {
 constexpr int TCT = 256;   // 8 warps: warp&3 = TMEM lane quadrant, warp>>2 = column-slice parity
 // EPI_PHASE: the layer runs at its INPUT's (pre-upsampling) resolution R with the four output phases
 // (py,px) of the 2x nearest up-sampled grid as column groups: N = 4 * Cout, output is 2R x 2R
-enum { EPI_POOL = 0, EPI_PLAIN = 2, EPI_FINAL = 3, EPI_PHASE = 4 };
+enum { EPI_POOL = 0, EPI_PLAIN = 2, EPI_PHASE = 4 };
 
 using namespace tcptx;
 
 // MMA issue loops of the accumulating encoder kernels (L2, L3): the whole warp runs the loop and one elected lane
 // executes the tcgen05 instructions, so that descriptors stay in uniform registers (tc_ptx.cuh, elect_one):
 // ~3 instead of ~20 instructions per MMA.  Measured (bench.py cae_layers, 486k cells): L2 52.4 -> 45.6 ms,
-// L3 23.4 -> 22.1 ms.  The single-pass kernels (L1, L4-L7) measured 2-5 % SLOWER in that form and keep
-// `if (lane == 0) { loop }` (ISSUE1_*).  -DCIA_LANE0_ISSUE restores the round-1 form everywhere for A/B runs.
-#ifdef CIA_LANE0_ISSUE
-#define ISSUE_WARP(cond) (lane == 0 && (cond))
-#define ISSUE_BEGIN {
-#define ISSUE_END }
-#else
-#define ISSUE_WARP(cond) (cond)
+// L3 23.4 -> 22.1 ms (the form with lane 0 running the loop was removed).  The single-pass kernels (L1, L4-L7)
+// measured 2-5 % SLOWER in the elected form and keep `if (lane == 0) { loop }`.
 #define ISSUE_BEGIN if (elect_one()) {
 #define ISSUE_END } __syncwarp();
-#endif
-// waits of the accumulating kernels: with the suspend-time hint a waiting warp sleeps in hardware instead of
-// re-issuing try_wait + branch next to the issuing warp of its scheduler (-DCIA_SPIN_WAIT: the plain loop)
-#ifdef CIA_SPIN_WAIT
-#define MBAR_WAIT mbar_wait
-#else
-#define MBAR_WAIT mbar_wait_sleep
-#endif
-#ifdef CIA_SLEEP_WAIT_ALL          // A/B: the single-pass kernels' waits with the suspend-time hint as well
-#define mbar_wait mbar_wait_sleep
-#endif
-#ifdef CIA_UNIFORM_ISSUE_ALL
-#define ISSUE1_WARP(cond) (cond)
-#define ISSUE1_BEGIN if (elect_one()) {
-#define ISSUE1_END } __syncwarp();
-#else
-#define ISSUE1_WARP(cond) (lane == 0 && (cond))
-#define ISSUE1_BEGIN {
-#define ISSUE1_END }
-#endif
+// The accumulating kernels wait with the suspend-time hint (mbar_wait_sleep): a waiting warp sleeps in hardware
+// instead of re-issuing try_wait + branch next to the issuing warp of its scheduler.  The plain loop for these
+// kernels, and the hint for the single-pass kernels' waits, were measured and removed.
 
 // Pooling layers: value of a pooled pixel from the max over its 2x2 window of the SIGN-FOLDED conv
 // accumulators (weight columns carry sign(bn scale), see k_cae_tc_prepare).  bias -> ReLU -> BN is
@@ -140,7 +120,7 @@ struct Cfg {
     static constexpr int PARTS = NPASS > 1 ? 2 : 1;
     static constexpr int SMEM_B = PARTS * (REGION_B + W_B);
     // one CTA per SM, single pass, no pooling phases: a ninth warp issues the MMAs
-    static constexpr bool DED_ISSUER = NPASS == 1 && !POOL && EPI != EPI_FINAL && SMEM_B > 100 * 1024;
+    static constexpr bool DED_ISSUER = NPASS == 1 && !POOL && SMEM_B > 100 * 1024;
     static constexpr int THREADS = TCT + (DED_ISSUER ? 32 : 0);
 };
 
@@ -201,8 +181,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                const uint4* __restrict__ w_hi, const uint4* __restrict__ w_lo, float inv_scale,
                const float* __restrict__ bias, const float* __restrict__ bn_s,
                const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
-               float* __restrict__ feat, const float* __restrict__ crops, float* __restrict__ mse,
-               float* __restrict__ mae, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
+               float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
                int chunk_cells,
                int32_t* __restrict__ status) {
     bool range_ok = true;             // every fp16 activation store of this thread was finite
@@ -210,7 +189,6 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ __align__(8) uint64_t bar[2];
     __shared__ uint32_t tmem_base_s;
-    __shared__ float red_s[2][2][TCT / 32];    // [unit parity][mse | mae][warp]
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     unsigned char* a_part[2] = {smem, smem + C::REGION_B};
@@ -288,9 +266,8 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
             // one extra warp issues for all tiles (an N = 128 MMA takes longer than the ~60 cycles a single
             // thread needs per issue; two issuing warps measured slower): the eight worker warps go straight
             // to their epilogue instead of two of them first spending the whole MMA time inside the issue loop
-            if (ISSUE1_WARP(warp == TCT / 32)) {
+            if (lane == 0 && warp == TCT / 32) {
                 tc_fence_after();
-                ISSUE1_BEGIN
                 const uint64_t ad0 = make_smem_desc(smem_u32(a_part[0]), C::CHUNK_B, C::SBO_A);
                 const uint64_t bd0 = make_smem_desc(smem_u32(w_part[0]), COUT * 16, 128);
 #pragma unroll
@@ -307,13 +284,11 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                         }
                 }
                 umma_commit(&bar[tbuf]);
-                ISSUE1_END
             }
             return;
         }
-        if (ISSUE1_WARP(warp < NISS)) {
+        if (lane == 0 && warp < NISS) {
             tc_fence_after();
-            ISSUE1_BEGIN
             const int t = warp, py = t >> 1, px = t & 1;
             uint64_t dxo[3];          // tap-column offset in 16-byte units (pool: parity plane + half-column)
 #pragma unroll
@@ -339,7 +314,6 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                 }
             }
             umma_commit(&bar[tbuf]);
-            ISSUE1_END
         }
     };
 
@@ -387,7 +361,6 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
         const int q = warp & 3, half_sel = warp >> 2;
         const int r = 32 * q + lane;                   // MMA row = TMEM lane
         const uint32_t lane_addr = tmem_base + ((uint32_t)(32 * q) << 16) + tbuf * C::TBUF_COLS;
-        float se = 0.f, ae = 0.f;
         if (EPI == EPI_POOL) {
             constexpr int RO = R / 2;
             const int Y = r >> 3, X = 8 * sub + (r & 7);
@@ -458,7 +431,7 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
         } else {
             const int y = 16 * (sub / C::COL_BLOCKS) + (r >> 3);
             const int xblk = C::UNIT_COLS * (sub % C::COL_BLOCKS);
-            constexpr int SL = EPI == EPI_FINAL ? 1 : COUT / 8;
+            constexpr int SL = COUT / 8;
 #pragma unroll 1
             for (int p = half_sel; p < C::TILES * SL; p += 2) {
                 const int t = p / SL, sl = p - t * SL;
@@ -467,52 +440,23 @@ conv_tc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ in_l
                 uint32_t v[8];
                 TMEM_LD8(lane_addr + (uint32_t)(t * COUT + c0), v);
                 TMEM_WAIT8(v);
-                if (EPI == EPI_FINAL) {
-                    // columns 0..3 = output phases (py,px) of the up-sampled 64x64 reconstruction
-                    if (y < R) {
-                        const float b = __ldg(bias);
-                        const float* xr = crops + (size_t)cell * 4096;
+                float o[8];
 #pragma unroll
-                        for (int ph = 0; ph < 4; ++ph) {
-                            const float a = fmaf(__uint_as_float(v[ph]), inv_scale, b);
-                            const float rec = __fdividef(1.f, 1.f + __expf(-a));   // |err| ~1e-6, MSE gate is 1e-3
-                            const float d = __ldg(xr + (2 * y + (ph >> 1)) * 64 + 2 * x + (ph & 1)) - rec;
-                            se = fmaf(d, d, se);
-                            ae += fabsf(d);
-                        }
-                    }
-                } else {
-                    float o[8];
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        float a = fmaf(__uint_as_float(v[k]), inv_scale, __ldg(bias + c0 + k));
-                        a = fmaxf(a, 0.f);
-                        o[k] = __fadd_rn(__fmul_rn(a, __ldg(bn_s + c0 + k)), __ldg(bn_t + c0 + k));
-                    }
-                    if (y < R) {
-                        const size_t off = ((((size_t)cell * (COUT / 8) + sl) * R + y) * R + x) * 8;
-                        split_store8(o, out_hi + off, nullptr, range_ok);
-                    }
+                for (int k = 0; k < 8; ++k) {
+                    float a = fmaf(__uint_as_float(v[k]), inv_scale, __ldg(bias + c0 + k));
+                    a = fmaxf(a, 0.f);
+                    o[k] = __fadd_rn(__fmul_rn(a, __ldg(bn_s + c0 + k)), __ldg(bn_t + c0 + k));
+                }
+                if (y < R) {
+                    const size_t off = ((((size_t)cell * (COUT / 8) + sl) * R + y) * R + x) * 8;
+                    split_store8(o, out_hi + off, nullptr, range_ok);
                 }
             }
         }
-        if (EPI == EPI_FINAL) {
-            se = warp_sum(se); ae = warp_sum(ae);
-            if (lane == 0) { red_s[it & 1][0][warp] = se; red_s[it & 1][1][warp] = ae; }
-        }
-        // single-pass layers need no barrier here (the one before the next MMA issue orders the TMEM
-        // reads); the final layer's block reduction does, with red_s alternating between units
-        if (!PIPE || EPI == EPI_FINAL) {
+        // single-pass layers need no barrier here (the one before the next MMA issue orders the TMEM reads)
+        if (!PIPE) {
             tc_fence_before();
             __syncthreads();
-        }
-        if (EPI == EPI_FINAL && tid == 0) {
-            float s = 0.f, a = 0.f;
-#pragma unroll
-            for (int w = 0; w < TCT / 32; ++w) { s += red_s[it & 1][0][w]; a += red_s[it & 1][1][w]; }
-            // two bands per cell: two commutative float adds onto a zeroed slot -> deterministic
-            atomicAdd(mse + cell, s * (1.f / 4096.f));
-            atomicAdd(mae + cell, a * (1.f / 4096.f));
         }
     }
     tc_fence_before();
@@ -540,8 +484,7 @@ constexpr int ACC_MMA_WARPS = 4;
 constexpr int ACC_THREADS = (ACC_EPI_WARPS + ACC_MMA_WARPS) * 32;
 
 // Geometry of the accurate-accumulation kernel: ONE unit = one whole cell.  The zero-padded
-// (R+2) x (R+2) input is staged once, column-parity de-interleaved, and serves both pooled
-// X-halves (R = 32) -- half as many unit boundaries (staging, pipeline fill/drain) per MMA.
+// (R+2) x (R+2) input is staged once, column-parity de-interleaved.
 template <int CIN, int COUT, int R>
 struct AccCfg {
     static constexpr int NCH = CIN / 8;
@@ -552,8 +495,6 @@ struct AccCfg {
     static constexpr int PLANE_B = FILL_ROWS * ROW_B;
     static constexpr int CHUNK_B = 2 * PLANE_B;           // = LBO of A
     static constexpr int REGION_B = NCH * CHUNK_B;
-    static constexpr int SBO_A = 2 * ROW_B;
-    static constexpr int HALVES = R >= 32 ? 2 : 1;        // pooled 16x8 tiles per cell
     static constexpr int W_B = 9 * NCH * COUT * 16;
     static constexpr int SMEM_B = 2 * (REGION_B + W_B);
 };
@@ -615,18 +556,17 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
                    int32_t* __restrict__ status) {
     bool range_ok = true;             // every fp16 activation store of this thread was finite
     using C = AccCfg<CIN, COUT, R>;
-    // R = 16: the pooled output is only 8 x 8, so a 16-row-group tile takes BOTH row phases
-    // (row group g = conv row g, stride one staged row) and there are two tiles (px = 0, 1) instead
-    // of four half-empty ones; the 2x2 pool then pairs lanes r and r^8 with one shuffle per value.
-    constexpr bool ROWPAIR = R == 16;
-    constexpr int NT = ROWPAIR ? 2 : 4;          // accumulator tiles per stage = issuing warps
-    // STACK (N <= 32, where an MMA costs its 4 KB A-operand read whatever N is): the B operand of the
-    // hi activations is the weight image's hi and lo rows stacked along N, so hi*hi and hi*lo come out of
-    // ONE N = 2*COUT instruction in adjacent column groups and lo*hi is added to the cross group by a
+    static_assert(CIN == 64 && COUT == 32 && R == 16, "the L3 geometry: row-pair tiles, N-stacked weights");
+    // The pooled output is only 8 x 8, so a 16-row-group tile takes BOTH row phases (row group g = conv
+    // row g, stride one staged row) and there are two tiles (px = 0, 1) instead of four half-empty ones;
+    // the 2x2 pool then pairs lanes r and r^8 with one shuffle per value.
+    constexpr int NT = 2;                        // accumulator tiles per stage = issuing warps
+    // N-stacked weights (N <= 32, where an MMA costs its 4 KB A-operand read whatever N is): the B operand
+    // of the hi activations is the weight image's hi and lo rows stacked along N, so hi*hi and hi*lo come out
+    // of ONE N = 2*COUT instruction in adjacent column groups and lo*hi is added to the cross group by a
     // second one -- two A reads per k-step instead of three.  The cross group is flushed with the hi*hi
     // group (its truncations are 2^-11 of the sum's).
-    constexpr bool STACK = ROWPAIR && COUT <= 32;
-    constexpr int TILE_COLS = STACK ? 2 * COUT : COUT;
+    constexpr int TILE_COLS = 2 * COUT;
     constexpr int STAGE_COLS = NT * TILE_COLS;
     constexpr int TMEM_COLS = pow2_cols(2 * STAGE_COLS);
     constexpr int CW = COUT / 4;                 // columns per epilogue warp
@@ -643,7 +583,7 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
     int n = dev_count(n_cells, n_dev) - cell0;
     if (n > chunk_cells) n = chunk_cells;
     if (n <= 0) return;
-    const int n_units = n;                       // one unit = one cell (C::HALVES pooled tiles)
+    const int n_units = n;                       // one unit = one cell
 
     if (warp == 0) tmem_alloc(&tmem_base_s, TMEM_COLS);
     if (tid == 32) {
@@ -652,17 +592,10 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
         mbar_init(&ready_bar, ACC_EPI_WARPS);
         fence_barrier_init();
     }
-    if (STACK) {
-        // stacked image [(tap, chunk)][hi rows 0..COUT-1 | lo rows][8 halves] over both weight regions
-        for (int i = tid; i < 2 * C::W_B / 16; i += ACC_THREADS) {
-            const int tc = i / (2 * COUT), row = i - tc * (2 * COUT);
-            reinterpret_cast<uint4*>(w_part[0])[i] = row < COUT ? __ldg(w_hi + tc * COUT + row) : __ldg(w_lo + tc * COUT + row - COUT);
-        }
-    } else {
-        for (int i = tid; i < C::W_B / 16; i += ACC_THREADS) {
-            reinterpret_cast<uint4*>(w_part[0])[i] = __ldg(w_hi + i);
-            reinterpret_cast<uint4*>(w_part[1])[i] = __ldg(w_lo + i);
-        }
+    // stacked image [(tap, chunk)][hi rows 0..COUT-1 | lo rows][8 halves] over both weight regions
+    for (int i = tid; i < 2 * C::W_B / 16; i += ACC_THREADS) {
+        const int tc = i / (2 * COUT), row = i - tc * (2 * COUT);
+        reinterpret_cast<uint4*>(w_part[0])[i] = row < COUT ? __ldg(w_hi + tc * COUT + row) : __ldg(w_lo + tc * COUT + row - COUT);
     }
     fence_async_smem();
     tc_fence_before();
@@ -675,15 +608,13 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
         // ================= MMA issuers: one warp per phase tile =================
         // A single thread sustains only one tcgen05.mma per ~60 cycles (elect loop, R2UR moves,
         // dependent uniform-register adds), more than the 45-48 cycles an M128 x N<=64 MMA takes;
-        // four issuing warps, each owning the accumulator tile of one pooling phase, keep the
-        // tensor pipe fed.  Each commits to the stage's full barrier (count 4).
-        if (ISSUE_WARP(warp - ACC_EPI_WARPS < NT)) {
-            const int t = warp - ACC_EPI_WARPS, py = ROWPAIR ? 0 : t >> 1, px = t & 1;
-            constexpr uint32_t SBO = ROWPAIR ? C::ROW_B : C::SBO_A;
-            const uint64_t a_hi0 = make_smem_desc(smem_u32(a_part[0]) + py * C::ROW_B, C::CHUNK_B, SBO);
-            const uint64_t a_lo0 = make_smem_desc(smem_u32(a_part[1]) + py * C::ROW_B, C::CHUNK_B, SBO);
-            const uint64_t b_hi0 = make_smem_desc(smem_u32(w_part[0]), TILE_COLS * 16, 128);   // STACK: also the stacked operand
-            const uint64_t b_lo0 = make_smem_desc(smem_u32(w_part[1]), COUT * 16, 128);
+        // issuing warps, each owning the accumulator tile of one pooling phase, keep the tensor pipe
+        // fed.  Each commits to the stage's full barrier (count NT).
+        if (warp - ACC_EPI_WARPS < NT) {
+            const int t = warp - ACC_EPI_WARPS, px = t & 1;
+            const uint64_t a_hi0 = make_smem_desc(smem_u32(a_part[0]), C::CHUNK_B, C::ROW_B);
+            const uint64_t a_lo0 = make_smem_desc(smem_u32(a_part[1]), C::CHUNK_B, C::ROW_B);
+            const uint64_t b_hi0 = make_smem_desc(smem_u32(w_part[0]), TILE_COLS * 16, 128);   // the stacked operand
             constexpr uint32_t IDESC2 = make_idesc(128, TILE_COLS);
             uint64_t dxo[3];                   // (parity plane, half-column shift) of tap column dx, in 16-byte units
 #pragma unroll
@@ -694,59 +625,36 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
 #endif
             for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
                 DBG_T(m0);
-                MBAR_WAIT(&ready_bar, uphase);
+                mbar_wait_sleep(&ready_bar, uphase);
                 DBG_T(m1);
                 DBG_ADD(m_ready, m0, m1);
                 uphase ^= 1;
                 tc_fence_after();
 #pragma unroll
-                for (int half = 0; half < C::HALVES; ++half)
-#pragma unroll
                 for (int grp = 0; grp < NGRP; ++grp) {
                     const uint32_t st = it & 1;
                     DBG_T(m2);
-                    MBAR_WAIT(&empty_bar[st], ((it >> 1) & 1) ^ 1);
+                    mbar_wait_sleep(&empty_bar[st], ((it >> 1) & 1) ^ 1);
                     DBG_T(m3);
                     DBG_ADD(m_empty, m2, m3);
                     tc_fence_after();
                     const uint32_t d = tmem_base + st * STAGE_COLS + (uint32_t)(t * TILE_COLS);
                     ISSUE_BEGIN
-                    if (STACK) {
-                        // hi x [hi | lo] (N = 2*COUT, zero-initialising both column groups), then lo x hi into the cross group
+                    // hi x [hi | lo] (N = 2*COUT, zero-initialising both column groups), then lo x hi into the cross group
 #pragma unroll
-                        for (int pass = 0; pass < 2; ++pass) {
-#pragma unroll
-                            for (int tg = 0; tg < G; ++tg) {
-                                const int tap = grp * G + tg;
-                                if (tap < 9) {
-                                    const int dy = tap / 3, dx = tap % 3;
-                                    const uint64_t a0 = (pass == 1 ? a_lo0 : a_hi0) + dxo[dx];
-#pragma unroll
-                                    for (int s = 0; s < CIN / 16; ++s) {
-                                        const uint64_t ad = a0 + (uint64_t)(((dy * C::ROW_UNITS + 8 * half) * 16 + 2 * s * C::CHUNK_B) >> 4);
-                                        const uint64_t bd = b_hi0 + (uint64_t)(((tap * C::NCH + 2 * s) * TILE_COLS * 16) >> 4);
-                                        if (pass == 0) umma_f16(d, ad, bd, IDESC2, (tg == 0 && s == 0) ? 0u : 1u);
-                                        else umma_f16(d + COUT, ad, bd, IDESC, 1u);
-                                    }
-                                }
-                            }
-                        }
-                    } else
-                    // within a flush group: all cross terms (hi*lo, lo*hi; tiny) first, hi*hi last
-#pragma unroll
-                    for (int pass = 0; pass < 3; ++pass) {
+                    for (int pass = 0; pass < 2; ++pass) {
 #pragma unroll
                         for (int tg = 0; tg < G; ++tg) {
                             const int tap = grp * G + tg;
                             if (tap < 9) {
                                 const int dy = tap / 3, dx = tap % 3;
                                 const uint64_t a0 = (pass == 1 ? a_lo0 : a_hi0) + dxo[dx];
-                                const uint64_t b0 = pass == 0 ? b_lo0 : b_hi0;
 #pragma unroll
                                 for (int s = 0; s < CIN / 16; ++s) {
-                                    const uint64_t ad = a0 + (uint64_t)(((dy * C::ROW_UNITS + 8 * half) * 16 + 2 * s * C::CHUNK_B) >> 4);
-                                    const uint64_t bd = b0 + (uint64_t)(((tap * C::NCH + 2 * s) * COUT * 16) >> 4);
-                                    umma_f16(d, ad, bd, IDESC, (pass == 0 && tg == 0 && s == 0) ? 0u : 1u);
+                                    const uint64_t ad = a0 + (uint64_t)((dy * C::ROW_UNITS * 16 + 2 * s * C::CHUNK_B) >> 4);
+                                    const uint64_t bd = b_hi0 + (uint64_t)(((tap * C::NCH + 2 * s) * TILE_COLS * 16) >> 4);
+                                    if (pass == 0) umma_f16(d, ad, bd, IDESC2, (tg == 0 && s == 0) ? 0u : 1u);
+                                    else umma_f16(d + COUT, ad, bd, IDESC, 1u);
                                 }
                             }
                         }
@@ -779,9 +687,8 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
             const int cell = cell0 + unit;
             DBG_T(e0);
             // stage the zero-padded, column-parity de-interleaved input block (hi and lo); only the CTA's
-            // first cell is staged here, the others right after the previous cell's last flush (below;
-            // R = 16 only -- the R = 32 instance holds 64 accumulators per thread at that point)
-            if (!ROWPAIR || unit == (int)blockIdx.x) {
+            // first cell is staged here, the others right after the previous cell's last flush (below)
+            if (unit == (int)blockIdx.x) {
                 stage_pool_cell<C, R, EPT, 6>(in_hi, in_lo, a_part[0], a_part[1], cell, tid);
                 fence_async_smem();
                 __syncwarp();
@@ -793,8 +700,6 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
             ++e_units;
 #endif
 
-#pragma unroll 1
-            for (int sub = 0; sub < C::HALVES; ++sub) {
             float acc[NT][CW];
 #pragma unroll
             for (int ph = 0; ph < NT; ++ph)
@@ -804,28 +709,27 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
             for (int grp = 0; grp < NGRP; ++grp) {
                 const uint32_t st = it & 1;
                 DBG_T(e2);
-                MBAR_WAIT(&full_bar[st], (it >> 1) & 1);
+                mbar_wait_sleep(&full_bar[st], (it >> 1) & 1);
                 DBG_T(e3);
                 DBG_ADD(e_full, e2, e3);
                 tc_fence_after();
-                // two phases at a time keeps the live registers under the 120-per-thread budget
 #pragma unroll
                 for (int hp = 0; hp < NT / 2; ++hp) {
                     uint32_t v[2][CW / 8][8];
-                    uint32_t vc[2][STACK ? CW / 8 : 1][8];     // cross-term group of the stacked tiles
+                    uint32_t vc[2][CW / 8][8];     // cross-term group of the stacked tiles
 #pragma unroll
                     for (int p2 = 0; p2 < 2; ++p2)
 #pragma unroll
                         for (int k8 = 0; k8 < CW / 8; ++k8) {
                             TMEM_LD8(lane_addr + st * STAGE_COLS + (uint32_t)((2 * hp + p2) * TILE_COLS + k8 * 8), v[p2][k8]);
-                            if (STACK) TMEM_LD8(lane_addr + st * STAGE_COLS + (uint32_t)((2 * hp + p2) * TILE_COLS + COUT + k8 * 8), vc[p2][k8]);
+                            TMEM_LD8(lane_addr + st * STAGE_COLS + (uint32_t)((2 * hp + p2) * TILE_COLS + COUT + k8 * 8), vc[p2][k8]);
                         }
 #pragma unroll
                     for (int p2 = 0; p2 < 2; ++p2)
 #pragma unroll
                         for (int k8 = 0; k8 < CW / 8; ++k8) {
                             TMEM_WAIT8(v[p2][k8]);
-                            if (STACK) TMEM_WAIT8(vc[p2][k8]);
+                            TMEM_WAIT8(vc[p2][k8]);
                         }
                     if (hp == NT / 2 - 1) {
                         tc_fence_before();
@@ -840,8 +744,8 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
                         for (int k8 = 0; k8 < CW / 8; ++k8)
 #pragma unroll
                             for (int k = 0; k < 8; k += 2) {  // packed fp32x2 add (FADD2), round to nearest
-                                if (STACK) fadd2(acc[2 * hp + p2][k8 * 8 + k], acc[2 * hp + p2][k8 * 8 + k + 1],
-                                                 vc[p2][k8][k], vc[p2][k8][k + 1]);
+                                fadd2(acc[2 * hp + p2][k8 * 8 + k], acc[2 * hp + p2][k8 * 8 + k + 1],
+                                      vc[p2][k8][k], vc[p2][k8][k + 1]);
                                 fadd2(acc[2 * hp + p2][k8 * 8 + k], acc[2 * hp + p2][k8 * 8 + k + 1],
                                       v[p2][k8][k], v[p2][k8][k + 1]);
                             }
@@ -853,7 +757,7 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
             DBG_T(e6);
             // the cell's last MMAs have completed (its last full barrier): the input block is free, so the
             // next cell is staged NOW and its MMAs run under the final epilogue below
-            if (ROWPAIR && sub == C::HALVES - 1 && unit + (int)gridDim.x < n_units) {
+            if (unit + (int)gridDim.x < n_units) {
                 stage_pool_cell<C, R, EPT, 6>(in_hi, in_lo, a_part[0], a_part[1], cell + (int)gridDim.x, tid);
                 fence_async_smem();
                 __syncwarp();
@@ -861,35 +765,32 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
             }
             // final epilogue from registers: bias -> ReLU -> BN -> 2x2 max -> hi/lo fp16 (+ fp32 tap)
             constexpr int RO = R / 2;
-            const int Y = ROWPAIR ? r >> 4 : r >> 3, X = 8 * sub + (r & 7);
-            if (ROWPAIR || Y < RO) {
+            const int Y = r >> 4, X = r & 7;
 #pragma unroll
-                for (int k8 = 0; k8 < CW / 8; ++k8) {
-                    const int c0 = cq * CW + k8 * 8;
-                    float o[8];
+            for (int k8 = 0; k8 < CW / 8; ++k8) {
+                const int c0 = cq * CW + k8 * 8;
+                float o[8];
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        const float b = __ldg(bias + c0 + k), s = __ldg(bn_s + c0 + k), t = __ldg(bn_t + c0 + k);
-                        float m = acc[0][k8 * 8 + k];
+                for (int k = 0; k < 8; ++k) {
+                    const float b = __ldg(bias + c0 + k), s = __ldg(bn_s + c0 + k), t = __ldg(bn_t + c0 + k);
+                    float m = acc[0][k8 * 8 + k];
 #pragma unroll
-                        for (int ph = 1; ph < NT; ++ph) m = fmaxf(m, acc[ph][k8 * 8 + k]);
-                        if (ROWPAIR) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 8));   // conv rows 2Y, 2Y+1
-                        o[k] = pooled_act(m, inv_scale, invd, b, s, t);
-                    }
-                    if (ROWPAIR && (r & 8)) continue;      // the even conv row's lane stores the pooled pixel
-                    const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
-                    if (feat) {
-                        float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
-                                                             (size_t)(Y * RO + X) * COUT + c0);
-                        f[0] = make_float4(o[0], o[1], o[2], o[3]);
-                        f[1] = make_float4(o[4], o[5], o[6], o[7]);
-                    }
+                    for (int ph = 1; ph < NT; ++ph) m = fmaxf(m, acc[ph][k8 * 8 + k]);
+                    m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 8));   // conv rows 2Y, 2Y+1
+                    o[k] = pooled_act(m, inv_scale, invd, b, s, t);
+                }
+                if (r & 8) continue;      // the even conv row's lane stores the pooled pixel
+                const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
+                split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
+                if (feat) {
+                    float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
+                                                         (size_t)(Y * RO + X) * COUT + c0);
+                    f[0] = make_float4(o[0], o[1], o[2], o[3]);
+                    f[1] = make_float4(o[4], o[5], o[6], o[7]);
                 }
             }
             DBG_T(e7);
             DBG_ADD(e_final, e6, e7);
-            }   // sub (pooled X half)
         }
 #ifdef CIA_ACC_TIMING
         if (tid == 0) {
@@ -910,8 +811,8 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
 
 // ---------------------------------------------------------------------------------------
 // Accurate accumulation for the R = 32 pooling layer (L2): TMA-fed, double-buffered blocks.
-// In-kernel clocks on the whole-cell kernel above (profiles/r1_acc_phase_cycles.txt) show its
-// phases running back to back per cell: staging 7.7k cycles -> MMAs 22k (issue-bound at ~51
+// In-kernel clocks on a whole-cell form of the kernel above at R = 32 (since removed;
+// profiles/r1_acc_phase_cycles.txt) showed its phases running back to back per cell: staging 7.7k cycles -> MMAs 22k (issue-bound at ~51
 // cycles per M128xN64xK16 instruction) -> final epilogue 3.7k, with per-tap flushes keeping
 // the epilogue warps busier (27k) than the tensor pipe.  Here one unit = one pooled X-half
 // (16 input columns + halo, 2 x 39 KB hi/lo) and the two halves of a cell alternate between
@@ -923,18 +824,17 @@ conv_tc_acc_kernel(const __half* __restrict__ in_hi, const __half* __restrict__ 
 // ---------------------------------------------------------------------------------------
 template <int CIN, int COUT, int R_>
 struct Acc2Cfg {
-    static constexpr int R = R_;                          // 32: two half blocks per cell, two buffers; 16: one block, one buffer
+    static constexpr int R = R_;
     static constexpr int NCH = CIN / 8;
     static constexpr int FILL_ROWS = R + 2;
     static constexpr int HALVES = R / 16;                 // 16-column blocks per cell = shared-memory buffers
-    static constexpr bool ROWPAIR = R == 16;              // see conv_tc_acc_kernel: tiles take both row phases
     static constexpr int BOX_X = 16 + 2;                  // columns a box spans (every second one is read)
     static constexpr int ROW_UNITS = BOX_X / 2;           // 16-byte units per parity-plane row
     static constexpr int ROW_B = ROW_UNITS * 16;
     static constexpr int PLANE_B = FILL_ROWS * ROW_B;     // one (parity, chunk) plane = LBO of A
     static constexpr int PAR_B = NCH * PLANE_B;           // one TMA box: all chunks of one column parity
     static constexpr int REGION_B = 2 * PAR_B;            // hi or lo part of a block
-    static constexpr int SBO_A = ROWPAIR ? ROW_B : 2 * ROW_B;
+    static constexpr int SBO_A = 2 * ROW_B;
     static constexpr int BUF_B = 2 * REGION_B;            // hi + lo of one block
     static constexpr int W_B = 9 * NCH * COUT * 16;
     static constexpr int SMEM_B = HALVES * BUF_B + 2 * W_B;
@@ -971,8 +871,8 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                     int32_t* __restrict__ status) {
     bool range_ok = true;             // every fp16 activation store of this thread was finite
     using C = Acc2Cfg<CIN, COUT, R>;
-    constexpr bool ROWPAIR = C::ROWPAIR;
-    constexpr int NT = ROWPAIR ? 2 : 4;          // accumulator tiles per stage = issuing warps
+    static_assert(CIN == 32 && COUT == 64 && R == 32, "the L2 geometry: two half-cell blocks, four pooling-phase tiles");
+    constexpr int NT = 4;                        // accumulator tiles per stage = issuing warps
     constexpr int STAGE_COLS = NT * COUT;
     constexpr int TMEM_COLS = pow2_cols(2 * STAGE_COLS);
     constexpr int CW = COUT / 4;                 // columns per epilogue warp
@@ -1010,8 +910,8 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
 
     if (warp >= ACC_EPI_WARPS) {
         // ================= MMA issuers: one warp per phase tile =================
-        if (ISSUE_WARP(warp - ACC_EPI_WARPS < NT)) {
-            const int t = warp - ACC_EPI_WARPS, py = ROWPAIR ? 0 : t >> 1, px = t & 1;
+        if (warp - ACC_EPI_WARPS < NT) {
+            const int t = warp - ACC_EPI_WARPS, py = t >> 1, px = t & 1;
             const uint64_t b_hi0 = make_smem_desc(smem_u32(w_part[0]), COUT * 16, 128);
             const uint64_t b_lo0 = make_smem_desc(smem_u32(w_part[1]), COUT * 16, 128);
             uint64_t dxo[3];                   // (parity plane, half-column shift) of tap column dx, in 16-byte units
@@ -1028,7 +928,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                     const uint64_t a_hi0 = make_smem_desc(abase, C::PLANE_B, C::SBO_A);
                     const uint64_t a_lo0 = make_smem_desc(abase + C::REGION_B, C::PLANE_B, C::SBO_A);
                     DBG_T(m0);
-                    MBAR_WAIT(&ready_bar[half], cphase);
+                    mbar_wait_sleep(&ready_bar[half], cphase);
                     DBG_T(m1);
                     DBG_ADD(m_ready, m0, m1);
                     tc_fence_after();
@@ -1036,7 +936,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                     for (int grp = 0; grp < NGRP; ++grp) {
                         const uint32_t st = it & 1;
                         DBG_T(m2);
-                        MBAR_WAIT(&empty_bar[st], ((it >> 1) & 1) ^ 1);
+                        mbar_wait_sleep(&empty_bar[st], ((it >> 1) & 1) ^ 1);
                         DBG_T(m3);
                         DBG_ADD(m_empty, m2, m3);
                         tc_fence_after();
@@ -1107,7 +1007,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                 for (int grp = 0; grp < NGRP; ++grp) {
                     const uint32_t st = it & 1;
                     DBG_T(e2);
-                    MBAR_WAIT(&full_bar[st], (it >> 1) & 1);
+                    mbar_wait_sleep(&full_bar[st], (it >> 1) & 1);
                     DBG_T(e3);
                     DBG_ADD(e_full, e2, e3);
                     tc_fence_after();
@@ -1151,7 +1051,7 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                 DBG_T(e6);
                 // final epilogue from registers: bias -> ReLU -> BN -> 2x2 max -> hi/lo fp16 (+ fp32 tap)
                 constexpr int RO = R / 2;
-                const int Y = ROWPAIR ? r >> 4 : r >> 3, X = 8 * sub + (r & 7);
+                const int Y = r >> 3, X = 8 * sub + (r & 7);
 #pragma unroll
                 for (int k8 = 0; k8 < CW / 8; ++k8) {
                     const int c0 = cq * CW + k8 * 8;
@@ -1162,10 +1062,8 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
                         float m = acc[0][k8 * 8 + k];
 #pragma unroll
                         for (int ph = 1; ph < NT; ++ph) m = fmaxf(m, acc[ph][k8 * 8 + k]);
-                        if (ROWPAIR) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, 8));   // conv rows 2Y, 2Y+1
                         o[k] = pooled_act(m, inv_scale, invd, b, sc, sh);
                     }
-                    if (ROWPAIR && (r & 8)) continue;      // the even conv row's lane stores the pooled pixel
                     const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
                     split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
                     if (feat) {
@@ -1197,225 +1095,17 @@ conv_tc_acc2_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_cons
 }
 
 // ---------------------------------------------------------------------------------------
-// Layer 2 with N-STACKED weights (round 2; an A/B variant, CIA_L2_STACK=1 -- measured EQUAL to the kernel above:
-// 45.9 vs 45.1-45.9 ms per 486k cells, see the end of this comment).  conv_tc_acc2_kernel above sits on the tensor-core
-// pipe's operand-delivery limit (98.5 % busy, profiles/r2k_l2_full.txt): at N = 64 an M128 x K16 MMA costs the
-// 48 cycles of its 4 KB A + 2 KB B fetch, and the hi/lo split fetches the hi activations twice (x W_hi, x W_lo).
-// Here B is the stacked image [W_hi | W_lo] (N = 128, 64 cycles): hi x [W_hi | W_lo] puts the main product and the
-// hi*lo cross term into ADJACENT column groups [main | cross] with ONE A fetch, lo x W_hi (N = 64) adds the other
-// cross term: 112 instead of 144 pipe cycles per k-step.
-// What made the first attempt at this lose (profiles/r2_umma_microbench.txt: flushes doubled) is avoided by
-// keeping the two column groups apart in time:
-//   * the MAIN group is flushed every three taps as before (its hi*hi chain must stay short, see above); the first
-//     (tap, k-step) of a flush group is issued UN-stacked (hi x W_hi with accumulate = 0 zeroes the main group only),
-//   * the CROSS group -- 2^-11 of the sum, its truncations do not matter -- accumulates over all nine taps in TMEM
-//     and is read ONCE per tile.
-// TMEM: a tile is 128 columns, the four pooling-phase tiles of a half cell fill the 512; every tile has its own
-// full / empty barrier pair, so a tile's flush runs under the other three tiles' MMAs.
-//   warps 0..15: epilogue (quadrant = warp & 3, 16 of the 64 channels = warp >> 2), thread 0 issues the TMA refills
-//   warps 16-19: MMA issue, one warp per tile (whole warp runs the loop, elect.sync issues)
-// Measured (bench.py cae_layers, L2 ms per 486k cells; VAR = timing experiments of this kernel):
-//   stacked 45.9 | every k-step un-stacked (18 N = 64 MMAs per group) 49.5 | without the lo x W_hi MMAs 33.8 | kernel above 45.1
-// i.e. time = 13 ms + 2.0 ms per N = 64 MMA slot + 3.3 ms per N = 128 slot: in this accumulate pattern an N = 128 MMA costs
-// 1.64 N = 64 MMAs (79 cycles, not the 64 of the back-to-back microbenchmark), so stacking saves 12 % of the MMA part,
-// not 22 %, and 29 % of the kernel (flushes competing with the MMAs for TMEM, final epilogue) does not shrink with it.
-// A first version with two tiles in flight (pairs alternating) ran at 55.4 ms: an MMA waits for the previous one into
-// the same TMEM columns, the pipe needs four independent accumulate chains.
-// ---------------------------------------------------------------------------------------
-template <int G, int VAR = 0>     // VAR (timing experiments only): 1 = every k-step un-stacked, 2 = no lo x W_hi MMAs (wrong results)
-__global__ void __launch_bounds__(ACC_THREADS, 1)
-conv_tc_l2_stack_kernel(const __grid_constant__ CUtensorMap tm_hi, const __grid_constant__ CUtensorMap tm_lo,
-                        const uint4* __restrict__ w_hi, const uint4* __restrict__ w_lo, float inv_scale, float invd,
-                        const float* __restrict__ bias, const float* __restrict__ bn_s,
-                        const float* __restrict__ bn_t, __half* __restrict__ out_hi, __half* __restrict__ out_lo,
-                        float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev, int cell0,
-                        int chunk_cells,
-                        int32_t* __restrict__ status) {
-    bool range_ok = true;             // every fp16 activation store of this thread was finite
-    constexpr int CIN = 32, COUT = 64, R = 32;
-    using C = Acc2Cfg<CIN, COUT, R>;
-    constexpr int NGRP = (9 + G - 1) / G;        // main-group flushes per tile
-    constexpr int CW = COUT / 4;                 // channels per epilogue warp
-    constexpr int TILE_COLS = 2 * COUT;          // [main | cross]
-    constexpr int WS_B = 2 * C::W_B;             // stacked image: [(tap, chunk)][hi rows 0..63 | lo rows 64..127][8 halves]
-    extern __shared__ __align__(1024) unsigned char smem[];
-    __shared__ __align__(8) uint64_t full_bar[4], empty_bar[4], ready_bar[2];
-    __shared__ uint32_t tmem_base_s;
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    unsigned char* const w_s = smem + C::HALVES * C::BUF_B;
-
-    int n = dev_count(n_cells, n_dev) - cell0;
-    if (n > chunk_cells) n = chunk_cells;
-    if (n <= 0) return;
-    const int n_units = n;
-
-    if (warp == 0) tmem_alloc(&tmem_base_s, 512);
-    if (tid == 32) {
-        for (int t = 0; t < 4; ++t) { mbar_init(&full_bar[t], 1); mbar_init(&empty_bar[t], ACC_EPI_WARPS); }
-        mbar_init(&ready_bar[0], 1); mbar_init(&ready_bar[1], 1);
-        fence_barrier_init();
-    }
-    for (int i = tid; i < WS_B / 16; i += ACC_THREADS) {
-        const int tc = i / (2 * COUT), row = i - tc * (2 * COUT);
-        reinterpret_cast<uint4*>(w_s)[i] = row < COUT ? __ldg(w_hi + tc * COUT + row) : __ldg(w_lo + tc * COUT + row - COUT);
-    }
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = tmem_base_s;
-    const uint32_t sbase = smem_u32(smem);
-    constexpr uint32_t IDESC64 = make_idesc(128, COUT), IDESC128 = make_idesc(128, 2 * COUT);
-
-    if (warp >= ACC_EPI_WARPS) {
-        // ================= MMA issuers: one warp per pooling-phase tile =================
-        // The four tiles are four independent accumulate chains (an MMA into a tile waits for the previous one into
-        // the same columns: with only two tiles in flight the pipe ran at half rate) with their own full / empty
-        // barriers: a tile's flush runs under the other three tiles' MMAs, no explicit stages.
-        if (warp - ACC_EPI_WARPS < 4) {
-            const int t = warp - ACC_EPI_WARPS, py = t >> 1, px = t & 1;
-            const uint64_t b_s0 = make_smem_desc(smem_u32(w_s), 2 * COUT * 16, 128);       // stacked (and, with N = 64, W_hi)
-            const uint64_t b_l0 = b_s0 + (uint64_t)((COUT * 16) >> 4);                     // W_lo rows
-            uint64_t dxo[3];
-#pragma unroll
-            for (int dx = 0; dx < 3; ++dx) dxo[dx] = (uint64_t)((((px + dx) & 1) * C::PAR_B + ((px + dx) >> 1) * 16) >> 4);
-            const uint32_t d_main = tmem_base + (uint32_t)(t * TILE_COLS), d_cross = d_main + COUT;
-            uint32_t use = 0, cphase = 0;                    // use: running count of this tile's flush groups
-            for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
-#pragma unroll 1
-                for (int half = 0; half < 2; ++half) {
-                    MBAR_WAIT(&ready_bar[half], cphase);
-                    tc_fence_after();
-                    const uint32_t abase = sbase + half * C::BUF_B + py * C::ROW_B;
-                    const uint64_t a_hi0 = make_smem_desc(abase, C::PLANE_B, C::SBO_A);
-                    const uint64_t a_lo0 = make_smem_desc(abase + C::REGION_B, C::PLANE_B, C::SBO_A);
-#pragma unroll
-                    for (int grp = 0; grp < NGRP; ++grp, ++use) {
-                        MBAR_WAIT(&empty_bar[t], (use & 1) ^ 1);
-                        tc_fence_after();
-                        ISSUE_BEGIN
-#pragma unroll
-                        for (int tg = 0; tg < G; ++tg) {
-                            const int tap = grp * G + tg;
-                            if (tap < 9) {
-                                const int dy = tap / 3, dx = tap % 3;
-#pragma unroll
-                                for (int s = 0; s < CIN / 16; ++s) {
-                                    const uint64_t ao = dxo[dx] + (uint64_t)((dy * C::ROW_B + 2 * s * C::PLANE_B) >> 4);
-                                    const uint64_t bo = (uint64_t)(((tap * C::NCH + 2 * s) * 2 * COUT * 16) >> 4);
-                                    if ((tg == 0 && s == 0) || VAR == 1) {
-                                        // un-stacked: zero the MAIN group only; the cross group starts with the tile
-                                        umma_f16(d_main, a_hi0 + ao, b_s0 + bo, IDESC64, (tg == 0 && s == 0) ? 0u : 1u);
-                                        umma_f16(d_cross, a_hi0 + ao, b_l0 + bo, IDESC64, (grp == 0 && tg == 0 && s == 0) ? 0u : 1u);
-                                    } else {
-                                        umma_f16(d_main, a_hi0 + ao, b_s0 + bo, IDESC128, 1u);     // [main | cross] += hi x [W_hi | W_lo]
-                                    }
-                                    if (VAR != 2) umma_f16(d_cross, a_lo0 + ao, b_s0 + bo, IDESC64, 1u);         // cross += lo x W_hi
-                                }
-                            }
-                        }
-                        umma_commit(&full_bar[t]);
-                        ISSUE_END
-                    }
-                }
-                cphase ^= 1;
-            }
-        }
-    } else {
-        // ================= copy issuer / accumulating epilogue =================
-        const int q = warp & 3, cq = warp >> 2;
-        const int r = 32 * q + lane;
-        const uint32_t lane_addr = tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)(cq * CW);
-        uint32_t use = 0;
-        if (tid == 0 && (int)blockIdx.x < n_units) {
-            for (int hb = 0; hb < 2; ++hb)
-                tma_load_half_block<C>(&tm_hi, &tm_lo, sbase + hb * C::BUF_B, blockIdx.x, hb, &ready_bar[hb]);
-        }
-        for (int unit = blockIdx.x; unit < n_units; unit += gridDim.x) {
-            const int cell = cell0 + unit;
-#pragma unroll 1
-            for (int sub = 0; sub < 2; ++sub) {
-                float acc[4][CW];
-#pragma unroll
-                for (int ph = 0; ph < 4; ++ph)
-#pragma unroll
-                    for (int k = 0; k < CW; ++k) acc[ph][k] = 0.f;
-#pragma unroll 1
-                for (int grp = 0; grp < NGRP; ++grp, ++use) {
-#pragma unroll
-                    for (int t = 0; t < 4; ++t) {
-                        MBAR_WAIT(&full_bar[t], use & 1);
-                        tc_fence_after();
-                        // the last MMAs reading this half's input block are done: refill it with the same half of the next cell
-                        if (grp == NGRP - 1 && t == 3 && tid == 0 && unit + (int)gridDim.x < n_units)
-                            tma_load_half_block<C>(&tm_hi, &tm_lo, sbase + sub * C::BUF_B, unit + (int)gridDim.x, sub,
-                                                   &ready_bar[sub]);
-                        // the tile's main group; on its last flush the cross group follows (once per tile)
-#pragma unroll
-                        for (int part = 0; part < 2; ++part) {
-                            if (part == 1 && grp != NGRP - 1) break;
-                            uint32_t v[CW / 8][8];
-#pragma unroll
-                            for (int k8 = 0; k8 < CW / 8; ++k8) TMEM_LD8(lane_addr + (uint32_t)(t * TILE_COLS + part * COUT + k8 * 8), v[k8]);
-#pragma unroll
-                            for (int k8 = 0; k8 < CW / 8; ++k8) TMEM_WAIT8(v[k8]);
-                            if (part == 1 || grp != NGRP - 1) {         // all TMEM reads of this tile's step are done
-                                tc_fence_before();
-                                __syncwarp();
-                                if (lane == 0) mbar_arrive(&empty_bar[t]);
-                            }
-#pragma unroll
-                            for (int k8 = 0; k8 < CW / 8; ++k8)
-#pragma unroll
-                                for (int k = 0; k < 8; k += 2) fadd2(acc[t][k8 * 8 + k], acc[t][k8 * 8 + k + 1], v[k8][k], v[k8][k + 1]);
-                        }
-                    }
-                }
-                // final epilogue from registers: bias -> ReLU -> BN -> 2x2 max -> hi/lo fp16 (+ fp32 tap)
-                constexpr int RO = R / 2;
-                const int Y = r >> 3, X = 8 * sub + (r & 7);
-#pragma unroll
-                for (int k8 = 0; k8 < CW / 8; ++k8) {
-                    const int c0 = cq * CW + k8 * 8;
-                    float o[8];
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        const float b = __ldg(bias + c0 + k), sc = __ldg(bn_s + c0 + k), sh = __ldg(bn_t + c0 + k);
-                        const float m = fmaxf(fmaxf(acc[0][k8 * 8 + k], acc[1][k8 * 8 + k]), fmaxf(acc[2][k8 * 8 + k], acc[3][k8 * 8 + k]));
-                        o[k] = pooled_act(m, inv_scale, invd, b, sc, sh);
-                    }
-                    const size_t off = ((((size_t)cell * (COUT / 8) + c0 / 8) * RO + Y) * RO + X) * 8;
-                    split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
-                    if (feat) {
-                        float4* f = reinterpret_cast<float4*>(feat + (size_t)cell * (RO * RO * COUT) +
-                                                             (size_t)(Y * RO + X) * COUT + c0);
-                        f[0] = make_float4(o[0], o[1], o[2], o[3]);
-                        f[1] = make_float4(o[4], o[5], o[6], o[7]);
-                    }
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem_base, 512);
-    if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
-}
-
-// ---------------------------------------------------------------------------------------
 // Layer 1 (Cin = 1, K = 9)
 // ---------------------------------------------------------------------------------------
-// Layer 1 on the CUDA cores: with K = 9 the layer is epilogue-bound, not MMA-bound, and plain
-// fp32 FMAs are both faster than the im2col + tcgen05 route below and exact.  One block = one
-// quadrant of a cell (pooled 16x16 = conv 32x32); thread = (channel group of 8, pooled pixel),
-// 4 conv pixels x 8 channels in registers; output = the chunk-planar hi/lo fp16 planes.
+// Layer 1 of the single-pass path on the CUDA cores, exact fp32 FMAs (with K = 9 the layer is
+// epilogue-bound, not MMA-bound).  One block = one quadrant of a cell (pooled 16x16 = conv 32x32);
+// thread = (channel group of 8, pooled pixel), 4 conv pixels x 8 channels in registers; output =
+// the chunk-planar fp16 plane.
 __global__ void __launch_bounds__(256, 2)
 conv1_fp32_planar_kernel(const float* __restrict__ crops, const float* __restrict__ wgt /* [9][32] */,
                          const float* __restrict__ bias, const float* __restrict__ bn_s,
                          const float* __restrict__ bn_t, __half* __restrict__ out_hi,
-                         __half* __restrict__ out_lo, int n_cells, const int32_t* __restrict__ n_dev,
-                         int cell0, int chunk_cells,
+                         int n_cells, const int32_t* __restrict__ n_dev, int cell0, int chunk_cells,
                          int32_t* __restrict__ status) {
     bool range_ok = true;             // every fp16 activation store of this thread was finite
     __shared__ __align__(16) float xs[34][36];
@@ -1512,7 +1202,7 @@ conv1_fp32_planar_kernel(const float* __restrict__ crops, const float* __restric
                 }
             }
             const size_t off = ((((size_t)cell * 4 + cg) * 32 + (16 * qy + Y)) * 32 + (16 * qx + X)) * 8;
-            split_store8(o, out_hi + off, out_lo ? out_lo + off : nullptr, range_ok);
+            split_store8(o, out_hi + off, nullptr, range_ok);
         }
     }
     if (!range_ok) raise_status(status, CIA_E_UNSUPPORTED);
@@ -1608,7 +1298,7 @@ conv1_tc_split_kernel(const float* __restrict__ crops, const uint4* __restrict__
         // ================= MMA issuer: one thread, 12 MMAs per unit =================
         // (the workers never run issue code: with the issue inside four of the worker warps the
         // other four waited for them at every block barrier)
-        if (ISSUE1_WARP(true)) {
+        if (lane == 0) {
             uint64_t d_ahi[4], d_alo[4], d_whi[2], d_wlo[2];
 #pragma unroll
             for (int ph = 0; ph < 4; ++ph) {
@@ -1625,7 +1315,6 @@ conv1_tc_split_kernel(const float* __restrict__ crops, const uint4* __restrict__
                 const uint32_t buf = it & 1;
                 mbar_wait(&afull_bar[buf], (it >> 1) & 1);      // A block written AND the TMEM stage drained
                 tc_fence_after();
-                ISSUE1_BEGIN
                 const uint64_t bo = (uint64_t)(buf * (A_BUF_B >> 4));
 #pragma unroll
                 for (int ph = 0; ph < 4; ++ph) {
@@ -1635,7 +1324,6 @@ conv1_tc_split_kernel(const float* __restrict__ crops, const uint4* __restrict__
                     umma_f16(d, d_ahi[ph] + bo, d_whi[ph & 1], IDESC, 1u);
                 }
                 umma_commit(&done_bar[buf]);
-                ISSUE1_END
             }
         }
     } else {
@@ -1810,12 +1498,11 @@ final_tapsum_kernel(const __half* __restrict__ a6, const uint4* __restrict__ w_i
     const uint32_t tmem_base = tmem_base_s;
 
     if (warp == EPI_WARPS) {
-        if (ISSUE1_WARP(true)) {
+        if (lane == 0) {
             constexpr uint32_t IDESC = make_idesc(128, 32);
             const uint64_t bd0 = make_smem_desc(smem_u32(w_s), 32 * 16, 128);
             const __half* src0 = a6 + (size_t)cell0 * (A_B / 2);
             // prologue: the first two cells' activations
-            ISSUE1_BEGIN
             for (int k = 0; k < 2; ++k) {
                 const int unit = (int)blockIdx.x + k * stride;
                 if (unit < n) {
@@ -1823,14 +1510,12 @@ final_tapsum_kernel(const __half* __restrict__ a6, const uint4* __restrict__ w_i
                     bulk_load(smem_u32(smem) + k * A_B, src0 + (size_t)unit * (A_B / 2), A_B, &a_full[k]);
                 }
             }
-            ISSUE1_END
             uint32_t it = 0;
             for (int unit = blockIdx.x; unit < n; unit += stride, ++it) {
                 const uint32_t st = it & 1, ph = (it >> 1) & 1;
                 mbar_wait(&a_full[st], ph);
                 mbar_wait(&d_empty[st], ph ^ 1);            // the epilogue of two cells ago has drained this stage
                 tc_fence_after();
-                ISSUE1_BEGIN
                 const uint64_t ad0 = make_smem_desc(smem_u32(smem) + st * A_B, 1024 * 16, 128);
 #pragma unroll
                 for (int t = 0; t < 8; ++t)
@@ -1840,14 +1525,11 @@ final_tapsum_kernel(const __half* __restrict__ a6, const uint4* __restrict__ w_i
                                  ad0 + (uint64_t)((t * 128 * 16 + 2 * ks * 1024 * 16) >> 4),
                                  bd0 + (uint64_t)((2 * ks * 32 * 16) >> 4), IDESC, ks);
                 umma_commit(&d_full[st]);
-                ISSUE1_END
                 // the MMAs have read the buffer: refill it with the cell after next
                 mbar_wait(&d_full[st], ph);
                 if (unit + 2 * stride < n) {
-                    ISSUE1_BEGIN
                     mbar_expect_tx(&a_full[st], A_B);
                     bulk_load(smem_u32(smem) + st * A_B, src0 + (size_t)(unit + 2 * stride) * (A_B / 2), A_B, &a_full[st]);
-                    ISSUE1_END
                 }
             }
         }
@@ -1929,8 +1611,8 @@ final_tapsum_kernel(const __half* __restrict__ a6, const uint4* __restrict__ w_i
 // ---------------------------------------------------------------------------------------
 template <int CIN, int COUT, int R, int EPI, int NPASS, bool UPSIN = false>
 int launch_tc(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_hi, const __half* in_lo,
-              __half* out_hi, __half* out_lo, float* feat, const float* crops, float* mse, float* mae,
-              int n, const int32_t* n_dev, int cell0, int chunk, cudaStream_t s) {
+              __half* out_hi, __half* out_lo, float* feat, int n, const int32_t* n_dev, int cell0, int chunk,
+              cudaStream_t s) {
     using C = Cfg<CIN, COUT, R, EPI, NPASS>;
     auto kern = conv_tc_kernel<CIN, COUT, R, EPI, NPASS, UPSIN>;
     if (first_use(h, (const void*)kern))
@@ -1940,7 +1622,7 @@ int launch_tc(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_hi, c
     if (grid > cap) grid = cap;
     kern<<<grid, C::THREADS, C::SMEM_B, s>>>(in_hi, in_lo, (const uint4*)w.tc_w[layer][0], (const uint4*)w.tc_w[layer][1],
                                       w.tc_inv_scale[layer], w.bias[layer], w.bn_scale[layer], w.bn_shift[layer],
-                                      out_hi, out_lo, feat, crops, mse, mae, n, n_dev, cell0, chunk, h->status_dev);
+                                      out_hi, out_lo, feat, n, n_dev, cell0, chunk, h->status_dev);
     CIA_LAUNCH_CHECK();
     return CIA_OK;
 }
@@ -2040,27 +1722,6 @@ int launch_tc_acc2(cia_ctx* h, const CaeWeights& w, int layer, const __half* in_
     return CIA_OK;
 }
 
-template <int G, int VAR = 0>
-int launch_l2_stack(cia_ctx* h, const CaeWeights& w, const __half* in_hi, const __half* in_lo, int buf_cells,
-                    __half* out_hi, __half* out_lo, float* feat, int n, const int32_t* n_dev, int cell0, int chunk,
-                    cudaStream_t s) {
-    using C = Acc2Cfg<32, 64, 32>;
-    auto kern = conv_tc_l2_stack_kernel<G, VAR>;
-    if (first_use(h, (const void*)kern))
-        CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_B));
-    CUtensorMap tm_hi, tm_lo;
-    int rc;
-    if ((rc = encode_act_map(h, &tm_hi, in_hi, C::NCH, C::R, buf_cells, C::BOX_X, C::FILL_ROWS))) return rc;
-    if ((rc = encode_act_map(h, &tm_lo, in_lo, C::NCH, C::R, buf_cells, C::BOX_X, C::FILL_ROWS))) return rc;
-    int grid = chunk;
-    if (grid > h->num_sms) grid = h->num_sms;
-    kern<<<grid, ACC_THREADS, C::SMEM_B, s>>>(tm_hi, tm_lo, (const uint4*)w.tc_w[1][0], (const uint4*)w.tc_w[1][1],
-                                              w.tc_inv_scale[1], w.tc_inv_scale[1] * acc_debias(h, 1), w.bias[1],
-                                              w.bn_scale[1], w.bn_shift[1], out_hi, out_lo, feat, n, n_dev, cell0, chunk, h->status_dev);
-    CIA_LAUNCH_CHECK();
-    return CIA_OK;
-}
-
 // One B image: [(tap*NCH + chunk)*N + n][8] halves = w[tap][chunk*8 + j][n] * 2^sw, hi and lo parts.
 static void pack_image(const std::vector<float>& w /* [taps][cin][n] */, int taps, int cin, int N,
                        int n_real, int sw, std::vector<__half>& hi, std::vector<__half>& lo,
@@ -2143,8 +1804,8 @@ int k_cae_tc_prepare(cia_ctx* h, int which) {
                             for (int c = 0; c < cin; ++c)
                                 kp[((size_t)tl * cin + c) * 4 + py * 2 + px] += k[((size_t)(dy * 3 + dx) * cin + c)];
                         }
+            // the scale of the phase form's weights; final_tapsum_kernel's image (below) and tc_inv_scale[6] use it
             sw = scale_exp(kp);
-            pack_image(kp, 9, cin, 16, 4, sw, hi, lo);
             // final_tapsum_kernel's image: ONE tap, the (phase, low-resolution neighbour) pairs on 16 columns
             // + their fp16 remainders on 16 more: [chunk][32][8]
             {
@@ -2171,6 +1832,8 @@ int k_cae_tc_prepare(cia_ctx* h, int which) {
                 CIA_CUDA(cudaMalloc(&w.tc_w7, img.size() * sizeof(__half)));
                 CIA_CUDA(cudaMemcpy(w.tc_w7, img.data(), img.size() * sizeof(__half), cudaMemcpyHostToDevice));
             }
+            w.tc_inv_scale[L] = std::ldexp(1.f, -sw);
+            continue;
         } else if (L == 5) {
             // same phase form with all Cout channels: N = 4 phases x Cout, run at the low (input) resolution --
             // 2 tiles x 9 taps instead of 8 tiles x 9 taps of MMAs per cell
@@ -2274,85 +1937,57 @@ int k_cae_forward_tc(cia_ctx* h, const float* crops, int n, const int32_t* n_dev
 #define CIA_LMARK(i) do { if (h->layer_ev && pass < CIA_LAYER_PASSES) CIA_CUDA(cudaEventRecord(h->layer_ev[pass * CIA_LAYER_MARKS + (i)], s)); } while (0)
         CIA_LMARK(0);
         if (tc_feat || l3_exact) {
-            // CIA_L1_KERNEL=0 keeps layer 1 on the CUDA cores (exact fp32 FMA chains) for A/B runs;
-            // the half-ulp truncation compensation of its single accumulation: cia_set_option "cae_l1_debias"
-            static const int l1_tc = [] { const char* e = getenv("CIA_L1_KERNEL"); return e ? atoi(e) : 1; }();
+            // the half-ulp truncation compensation of layer 1's single accumulation: cia_set_option "cae_l1_debias"
             const float l1_debias = h->cae_debias[0] * 5.9604645e-8f;
-            if (l1_tc) {
-                if (first_use(h, (const void*)conv1_tc_split_kernel))
-                    CIA_CUDA(cudaFuncSetAttribute(conv1_tc_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, l1tc::SMEM_B));
-                int gridt = chunk * 8;
-                if (gridt > h->num_sms * 2) gridt = h->num_sms * 2;
-                conv1_tc_split_kernel<<<gridt, l1tc::NT, l1tc::SMEM_B, s>>>(crops, (const uint4*)ae.tc_w[0][0], ae.tc_inv_scale[0],
-                                                                            l1_debias, ae.bias[0], ae.bn_scale[0], ae.bn_shift[0],
-                                                                            a1h, a1l, n, n_dev, c0, chunk, h->status_dev);
-            } else {
-                conv1_fp32_planar_kernel<<<grid1, 256, 0, s>>>(crops, ae.kernel[0], ae.bias[0], ae.bn_scale[0],
-                                                               ae.bn_shift[0], a1h, a1l, n, n_dev, c0, chunk, h->status_dev);
-            }
+            if (first_use(h, (const void*)conv1_tc_split_kernel))
+                CIA_CUDA(cudaFuncSetAttribute(conv1_tc_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, l1tc::SMEM_B));
+            int gridt = chunk * 8;
+            if (gridt > h->num_sms * 2) gridt = h->num_sms * 2;
+            conv1_tc_split_kernel<<<gridt, l1tc::NT, l1tc::SMEM_B, s>>>(crops, (const uint4*)ae.tc_w[0][0], ae.tc_inv_scale[0],
+                                                                        l1_debias, ae.bias[0], ae.bn_scale[0], ae.bn_shift[0],
+                                                                        a1h, a1l, n, n_dev, c0, chunk, h->status_dev);
             CIA_LAUNCH_CHECK();
             CIA_LMARK(1);
             float* a2f = l3_exact ? A2f - (size_t)c0 * (16 * 16 * 64) : nullptr;
-            // taps per TMEM flush of layer 2 (CIA_L2_TAPS_PER_FLUSH=1|2|3|9; 0 = the single-buffered whole-cell
-            // kernel): 3 keeps the epilogue warps below the tensor pipe's time.  An N-stacked variant (hi x [hi|lo]
-            // as one N = 128 instruction: 112 instead of 145 pipe cycles per k-step by profiles/umma_microbench.cu)
-            // was built and measured in round 2: 53.3 vs 51.5 ms -- its flushes double (main + cross column
-            // groups) and the drain of a two-tile stage no longer hides under the other stage's MMAs (DESIGN.md 5)
-            static const int l2_g = [] { const char* e = getenv("CIA_L2_TAPS_PER_FLUSH"); return e ? atoi(e) : 3; }();
-            // CIA_L2_STACK=1: the N-stacked kernel (conv_tc_l2_stack_kernel; 2 / 3: its timing experiments) for A/B runs
-            static const int l2_stack = [] { const char* e = getenv("CIA_L2_STACK"); return e ? atoi(e) : 0; }();
-            if (l2_stack == 2 && l2_g == 3) rc = launch_l2_stack<3, 1>(h, ae, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_stack == 3 && l2_g == 3) rc = launch_l2_stack<3, 2>(h, ae, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_stack && l2_g == 3) rc = launch_l2_stack<3>(h, ae, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_g == 0) rc = launch_tc_acc<32, 64, 32, 1>(h, ae, 1, a1h, a1l, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_g == 1) rc = launch_tc_acc2<32, 64, 32, 1>(h, ae, 1, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_g == 9) rc = launch_tc_acc2<32, 64, 32, 9>(h, ae, 1, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else if (l2_g == 2) rc = launch_tc_acc2<32, 64, 32, 2>(h, ae, 1, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            else rc = launch_tc_acc2<32, 64, 32, 3>(h, ae, 1, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s);
-            if (rc) return rc;
+            // three taps per TMEM flush of layer 2 keep the epilogue warps below the tensor pipe's time.  An N-stacked
+            // variant (hi x [hi|lo] as one N = 128 instruction: 112 instead of 145 pipe cycles per k-step by
+            // profiles/umma_microbench.cu) was built and measured in round 2: 53.3 vs 51.5 ms -- its flushes double
+            // (main + cross column groups) and the drain of a two-tile stage no longer hides under the other stage's
+            // MMAs (DESIGN.md 5)
+            if ((rc = launch_tc_acc2<32, 64, 32, 3>(h, ae, 1, A1h, A1l, CH, a2h, a2l, a2f, n, n_dev, c0, chunk, s))) return rc;
             CIA_LMARK(2);
             if (l3_exact) {
-                if ((rc = launch_tc<64, 32, 16, EPI_POOL, 1>(h, ae, 2, a2h, nullptr, a3h, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+                if ((rc = launch_tc<64, 32, 16, EPI_POOL, 1>(h, ae, 2, a2h, nullptr, a3h, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
                 if (features && (rc = k_conv3_fp32(h, ae, a2f, n, n_dev, features, c0, chunk, s))) return rc;
             } else {
-                // CIA_L3_KERNEL=1 selects the TMA-fed kernel (single input buffer -- two do not fit next to the
-                // 74 KB of weights -- refilled the moment the cell's last MMAs complete).  Measured: no gain over
-                // the register-staged kernel (cae 75.6 vs 74.0 ms per 242k cells), which stays the default.
-                static const int l3_tma = [] { const char* e = getenv("CIA_L3_KERNEL"); return e ? atoi(e) : 0; }();
-                static const int l3_g = [] { const char* e = getenv("CIA_L3_TAPS_PER_FLUSH"); return e ? atoi(e) : 1; }();
-                // Measured and dropped in round 2 (DESIGN.md section 5): the input block through cp.async (27.3 vs 23.7 ms),
-                // four TMEM stages with the MMAs of two flush groups interleaved (23.8 vs 22.1 ms)
-                if (l3_tma) rc = launch_tc_acc2<64, 32, 16, 1>(h, ae, 2, A2h, A2l, CH, a3h, nullptr, feat, n, n_dev, c0, chunk, s);
-                else if (l3_g == 3) rc = launch_tc_acc<64, 32, 16, 3>(h, ae, 2, a2h, a2l, a3h, nullptr, feat, n, n_dev, c0, chunk, s);
-                else rc = launch_tc_acc<64, 32, 16, 1>(h, ae, 2, a2h, a2l, a3h, nullptr, feat, n, n_dev, c0, chunk, s);
-                if (rc) return rc;
+                // Measured and dropped (DESIGN.md section 5): a TMA-fed L3 with one input buffer refilled the moment the
+                // cell's last MMAs complete (cae 75.6 vs 74.0 ms per 242k cells), three taps per flush (no gain), the
+                // input block through cp.async (27.3 vs 23.7 ms), four TMEM stages with the MMAs of two flush groups
+                // interleaved (23.8 vs 22.1 ms)
+                if ((rc = launch_tc_acc<64, 32, 16, 1>(h, ae, 2, a2h, a2l, a3h, nullptr, feat, n, n_dev, c0, chunk, s))) return rc;
             }
         } else {
             conv1_fp32_planar_kernel<<<grid1, 256, 0, s>>>(crops, ae.kernel[0], ae.bias[0], ae.bn_scale[0],
-                                                           ae.bn_shift[0], a1h, nullptr, n, n_dev, c0, chunk, h->status_dev);
+                                                           ae.bn_shift[0], a1h, n, n_dev, c0, chunk, h->status_dev);
             CIA_LAUNCH_CHECK();
             CIA_LMARK(1);
-            if ((rc = launch_tc<32, 64, 32, EPI_POOL, 1>(h, ae, 1, a1h, nullptr, a2h, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+            if ((rc = launch_tc<32, 64, 32, EPI_POOL, 1>(h, ae, 1, a1h, nullptr, a2h, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
             CIA_LMARK(2);
-            if ((rc = launch_tc<64, 32, 16, EPI_POOL, 1>(h, ae, 2, a2h, nullptr, a3h, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+            if ((rc = launch_tc<64, 32, 16, EPI_POOL, 1>(h, ae, 2, a2h, nullptr, a3h, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
         }
         CIA_LMARK(3);
-        if ((rc = launch_tc<32, 32, 8, EPI_PLAIN, 1>(h, ae, 3, a3h, nullptr, a4, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+        if ((rc = launch_tc<32, 32, 8, EPI_PLAIN, 1>(h, ae, 3, a3h, nullptr, a4, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
         CIA_LMARK(4);
-        if ((rc = launch_tc<32, 64, 16, EPI_PLAIN, 1, true>(h, ae, 4, a4, nullptr, a5, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+        if ((rc = launch_tc<32, 64, 16, EPI_PLAIN, 1, true>(h, ae, 4, a4, nullptr, a5, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
         CIA_LMARK(5);
-        if ((rc = launch_tc<64, 128, 16, EPI_PHASE, 1>(h, ae, 5, a5, nullptr, a6p, nullptr, nullptr, nullptr, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
+        if ((rc = launch_tc<64, 128, 16, EPI_PHASE, 1>(h, ae, 5, a5, nullptr, a6p, nullptr, nullptr, n, n_dev, c0, chunk, s))) return rc;
         CIA_LMARK(6);
-        // CIA_L7_KERNEL=0: the nine-tap implicit GEMM (conv_tc_kernel<EPI_FINAL>, 144 MMAs per cell) for A/B runs
-        static const int l7_tapsum = [] { const char* e = getenv("CIA_L7_KERNEL"); return e ? atoi(e) : 1; }();
-        if (l7_tapsum) {
-            if (first_use(h, (const void*)final_tapsum_kernel))
-                CIA_CUDA(cudaFuncSetAttribute(final_tapsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, l7::SMEM_B));
-            int g7 = chunk < h->num_sms ? chunk : h->num_sms;
-            final_tapsum_kernel<<<g7, l7::NT, l7::SMEM_B, s>>>(a6p, (const uint4*)ae.tc_w7, ae.tc_inv_scale[6], ae.bias[6],
-                                                              crops, mse, mae, n, n_dev, c0, chunk);
-            CIA_LAUNCH_CHECK();
-        } else if ((rc = launch_tc<32, 16, 32, EPI_FINAL, 1>(h, ae, 6, a6p, nullptr, nullptr, nullptr, nullptr, crops, mse, mae, n, n_dev, c0, chunk, s))) return rc;
+        if (first_use(h, (const void*)final_tapsum_kernel))
+            CIA_CUDA(cudaFuncSetAttribute(final_tapsum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, l7::SMEM_B));
+        int g7 = chunk < h->num_sms ? chunk : h->num_sms;
+        final_tapsum_kernel<<<g7, l7::NT, l7::SMEM_B, s>>>(a6p, (const uint4*)ae.tc_w7, ae.tc_inv_scale[6], ae.bias[6],
+                                                          crops, mse, mae, n, n_dev, c0, chunk);
+        CIA_LAUNCH_CHECK();
         CIA_LMARK(7);
 #undef CIA_LMARK
     }

@@ -58,7 +58,6 @@ struct ScalerPca {
     double* scale = nullptr;    // [F]
     double* rscale = nullptr;   // [F] 1 / scale, correctly rounded on the host (division by FMA correction)
     bool rscale_ok = false;     // every scale and reciprocal is a normal number
-    double* comp_t = nullptr;   // [F, C] transposed components
     double* comp_pad = nullptr; // [F rounded up to 32, CP] zero-padded copy for the cp.async-fed DMMA kernel
     int CP = 0;                 // C rounded up to a multiple of 104
     double* offset = nullptr;   // [C]
@@ -112,11 +111,6 @@ struct cia_ctx {
     // cia_set_option "svm_kernel": 1 = tcgen05 GEMM form (score_tc.cu), 0 = fp64 DMMA anchor (score.cu)
     int svm_kernel = 1;
     int pca_kernel = 1;        // "pca_kernel": 1 = tcgen05 projection (score_tc.cu), 0 = fp64 DMMA anchor
-    int seg_fuse_first = 0;    // "seg_fuse_first": the Cin = 1 layer evaluated inside the second layer's producer warps
-                               // (bit-identical; measured SLOWER: 336 us against 110 + 128 us for the two launches, the eight
-                               // producer warps become the bottleneck; the same evaluation inside the staged kernel, by all
-                               // threads of three CTAs per SM, measured 295 us and was removed again: the layer's 288 FMAs per
-                               // pixel cost what they cost wherever they run -- kept as an option, off by default)
     int seg_pool_out = 1;      // "seg_pool_out": TMA-fed layers also write the max-pooled copy the next layer reads (0: it pools itself)
     int seg_conv_ws = 1;       // "seg_conv_ws": warp-specialised software-producer kernel for the other layers (0: staged kernel)
     int seg_conv_tma = 1;      // "seg_conv_tma": segment.cu's TMA-fed convolution kernel for Cin = 32 direct layers (0: staged kernel)

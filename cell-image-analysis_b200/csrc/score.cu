@@ -1,7 +1,7 @@
 // score.cu -- K4 RobustScaler -> PCA projection, K5 RBF one-class SVM decision for
 // both detectors (GEMM form on the fp64 tensor pipe with the RBF/dual-coef reduction fused into
-// the tile epilogue; the direct-difference fp64 kernel stays as the wide-D fallback and A/B
-// anchor), K6 per-strain accumulators.
+// the tile epilogue; the direct-difference fp64 kernel stays as the wide-D fallback), K6
+// per-strain accumulators.
 //
 // Replaces improved_detection.py:134-135 (scaler.transform, pca.transform), :138-142
 // (predict + decision_function of the two OneClassSVMs; libsvm k_function RBF,
@@ -13,94 +13,10 @@
 
 namespace {
 
-constexpr int PT = 256;        // threads
-constexpr int PB = 64;         // cells per block
-constexpr int PFT = 32;        // features per shared-memory tile
-constexpr int PCT = 128;       // components per block tile
-constexpr int XPAD = PB + 2;   // padded row of the transposed x tile
-
-// z[c] = sum_f x2[f] * Wt[f][c] - offset[c]: a register-blocked fp64 GEMM tile (64 cells x 128
-// components per block, 8 x 4 accumulators per thread) over fp32-rounded inputs.
-// x2 mirrors sklearn's in-place float32 flow: x1 = f32(x - center), x2 = f32(f64(x1)/scale).
-__global__ void __launch_bounds__(PT)
-scaler_pca_kernel(const float* __restrict__ feat, int n_cells, const int32_t* __restrict__ n_dev,
-                  int F, int C, const double* __restrict__ center, const double* __restrict__ scale,
-                  int center_is_f32, const double* __restrict__ comp_t,
-                  const double* __restrict__ offset, int f32_flow, double* __restrict__ z_out) {
-    extern __shared__ __align__(16) unsigned char pca_smem[];
-    double (*ws)[PCT] = reinterpret_cast<double (*)[PCT]>(pca_smem);
-    double (*xs)[XPAD] = reinterpret_cast<double (*)[XPAD]>(pca_smem + sizeof(double) * PFT * PCT);
-    const int n = dev_count(n_cells, n_dev);
-    const int cell0 = blockIdx.x * PB;
-    if (cell0 >= n) return;
-    const int c_tile0 = blockIdx.y * PCT;
-    const int tid = threadIdx.x, cx = tid & 31, cy = tid >> 5;
-    double acc[8][4];
-#pragma unroll
-    for (int i = 0; i < 8; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.0;
-
-    for (int f0 = 0; f0 < F; f0 += PFT) {
-        __syncthreads();
-        for (int idx = tid; idx < PB * PFT; idx += PT) {
-            const int i = idx / PFT, ff = idx - i * PFT;
-            const int f = f0 + ff, cell = cell0 + i;
-            float v = 0.f;
-            if (cell < n && f < F) {
-                v = __ldg(feat + (size_t)cell * F + f);
-                if (center) {
-                    if (center_is_f32) v = __fsub_rn(v, (float)center[f]);
-                    else v = (float)__dsub_rn((double)v, center[f]);
-                }
-                if (scale) v = (float)__ddiv_rn((double)v, scale[f]);
-            }
-            xs[ff][i] = (double)v;
-        }
-        for (int idx = tid; idx < PFT * PCT; idx += PT) {
-            const int ff = idx / PCT, c = idx - ff * PCT;
-            const int f = f0 + ff, cc = c_tile0 + c;
-            ws[ff][c] = (f < F && cc < C) ? __ldg(comp_t + (size_t)f * C + cc) : 0.0;
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (int ff = 0; ff < PFT; ++ff) {
-            double w[4], x[8];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) w[j] = ws[ff][cx + 32 * j];
-#pragma unroll
-            for (int i = 0; i < 8; i += 2) {
-                const double2 t = *reinterpret_cast<const double2*>(&xs[ff][cy * 8 + i]);
-                x[i] = t.x; x[i + 1] = t.y;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = fma(x[i], w[j], acc[i][j]);
-        }
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int c = c_tile0 + cx + 32 * j;
-        if (c >= C) continue;
-        const double off = offset[c];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const int cell = cell0 + cy * 8 + i;
-            if (cell < n) {
-                double z;
-                if (f32_flow) z = (double)__fsub_rn((float)acc[i][j], (float)off);
-                else z = __dsub_rn(acc[i][j], off);
-                z_out[(size_t)cell * C + c] = z;
-            }
-        }
-    }
-}
-
 // ---- fp64 tensor-core form of the projection (mma.sync m8n8k4 f64), software pipelined ----
-// Measured on this B200 (profiles/fp64_peak_test.cu): DFMA 36 TFLOP/s, DMMA 37 TFLOP/s; the
-// register-tiled kernel above reaches ~9 because every 32-feature stage first waits for its
-// global loads.  Here the components come through cp.async into a second buffer and the raw
+// Measured on this B200 (profiles/fp64_peak_test.cu): DFMA 36 TFLOP/s, DMMA 37 TFLOP/s; a
+// register-tiled CUDA-core fp64 kernel (removed) reached ~9 because every 32-feature stage first
+// waited for its global loads.  Here the components come through cp.async into a second buffer and the raw
 // features of the next stage are prefetched into registers while the current stage computes.
 // Block = 16 warps = 64 cells x 104 components (13 n8 tiles; blockIdx.y tiles wider PCAs);
 // warp = 16 cells x 3-4 n8 tiles (4 cell groups x 4 component groups).  A call scores ~15k cells =
@@ -259,6 +175,7 @@ scaler_pca_dmma_kernel(const float* __restrict__ feat, int n_cells, const int32_
     }
 }
 
+constexpr int PT = 256;     // threads of the direct-difference SVM kernel
 constexpr int SCELLS = 8;   // cells per block in the SVM kernel
 
 // dec = sum_i coef_i * exp(-gamma * ||z - sv_i||^2) - rho  (fp64, direct difference).
@@ -531,34 +448,25 @@ int k_svm_decision(cia_ctx* h, const float* features, int n, const int32_t* n_de
     }
     if (first_use(h, (const void*)svm_rbf_kernel)) {
         CIA_CUDA(cudaFuncSetAttribute(svm_rbf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        CIA_CUDA(cudaFuncSetAttribute(scaler_pca_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
         CIA_CUDA(cudaFuncSetAttribute(scaler_pca_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     }
-    static const bool vector_pca = getenv("CIA_PCA_VECTOR") != nullptr;   // A/B switch: CUDA-core fp64 tile
     bool pca_done = false;
-    if (h->pca_kernel == 1 && !vector_pca) {          // tensor-core projection (score_tc.cu)
+    if (h->pca_kernel == 1) {                         // tensor-core projection (score_tc.cu)
         int rc = k_pca_tc(h, features, n, n_dev, z, &pca_done, s);
         if (rc) return rc;
     }
-    if (pca_done) {
-    } else if (vector_pca) {
-        const size_t sm1 = sizeof(double) * PFT * (PCT + XPAD);
-        scaler_pca_kernel<<<dim3((n + PB - 1) / PB, (sp.C + PCT - 1) / PCT), PT, sm1, s>>>(
-            features, n, n_dev, sp.F, sp.C, sp.has_center ? sp.center : nullptr,
-            sp.has_scale ? sp.scale : nullptr, sp.center_is_f32, sp.comp_t, sp.offset, sp.f32_flow, z);
-    } else {
+    if (!pca_done) {
         const size_t sm1 = sizeof(double) * 2 * (DM * DXP + DK * DWP);
         scaler_pca_dmma_kernel<<<dim3((n + DM - 1) / DM, sp.CP / DN), DT, sm1, s>>>(
             features, n, n_dev, sp.F, sp.C, sp.CP, sp.has_center ? sp.center : nullptr,
             sp.has_scale ? sp.scale : nullptr, sp.has_scale && sp.rscale_ok ? sp.rscale : nullptr, sp.center_is_f32, sp.comp_pad,
             sp.offset, sp.f32_flow, z);
+        CIA_LAUNCH_CHECK();
     }
-    if (!pca_done) CIA_LAUNCH_CHECK();
-    static const bool direct_svm = getenv("CIA_SVM_DIRECT") != nullptr;   // A/B switch: CUDA-core direct-difference form
     for (int which = 0; which < 2; ++which) {
         const SvmModel& m = h->svm[which];
         if (m.dim != sp.C) { h->err = "svm dimension != pca components"; return CIA_E_STATE; }
-        if (h->svm_kernel == 1 && !direct_svm) {
+        if (h->svm_kernel == 1) {
             // tensor-core GEMM form (score_tc.cu); falls through when the model is not served by it
             bool done = false;
             int rc = k_svm_tc(h, m, z, n, n_dev, which == 0 ? dec_cons : dec_mod, which == 0 ? pred_cons : pred_mod, &done, s);
@@ -566,7 +474,7 @@ int k_svm_decision(cia_ctx* h, const float* features, int n, const int32_t* n_de
             if (done) continue;
         }
         const size_t sm3 = sizeof(double) * ((size_t)GM * (m.dim_pad + 4) + 2 * GN * GSP + GM + 4 * GM);
-        if (!direct_svm && sm3 <= (size_t)h->max_smem_optin) {
+        if (sm3 <= (size_t)h->max_smem_optin) {
             if (first_use(h, (const void*)svm_rbf_dmma_kernel))
                 CIA_CUDA(cudaFuncSetAttribute(svm_rbf_dmma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem_optin));
             // fill the SMs: when the call has few cell blocks, split the SV tiles over blockIdx.y
@@ -589,7 +497,7 @@ int k_svm_decision(cia_ctx* h, const float* features, int n, const int32_t* n_de
                 CIA_LAUNCH_CHECK();
                 svm_finalize_kernel<<<(n + 255) / 256, 256, 0, s>>>(partial, n, splits, n, n_dev, m.rho, dec, pred);
             }
-        } else {   // very wide feature spaces (z tile does not fit) and the A/B switch
+        } else {   // very wide feature spaces: the z tile does not fit in shared memory
             const size_t sm2 = (size_t)SCELLS * m.dim * sizeof(double);
             svm_rbf_kernel<<<(n + SCELLS - 1) / SCELLS, PT, sm2, s>>>(
                 z, n, n_dev, m.dim, m.sv_t, m.coef, m.n_sv, m.n_sv_pad, m.gamma, m.rho,

@@ -26,7 +26,7 @@
 //   * the per-cell term log2(e) * gamma||z||^2 is split into an integer (added to the exponent field as an
 //     integer) and a fraction that multiplies the finished row sum in fp64;
 //   * 2^t is a Cody-Waite reduction + degree-6 minimax polynomial in packed FFMA2 (max rel. error 1e-7,
-//     mean 4e-10; ex2.approx measured 1.3e-4 in the decision at 5 000 SVs: CIA_SVM_MUFU=1 keeps the A/B);
+//     mean 4e-10; ex2.approx measured 1.3e-4 in the decision at 5 000 SVs);
 //   * row sums: fp32 over 32 terms, then 64-bit fixed point -- integer addition is associative, so a cell's
 //     decision does not depend on how its SV tiles were cut over CTAs, i.e. on its position in the call;
 //   * decisions within the kernel's error of zero are recomputed in fp64 (svm_refine_kernel).
@@ -97,16 +97,10 @@ __device__ __forceinline__ unsigned long long add2(unsigned long long a, unsigne
 // exponent field, nsh = nrow << 23) are added to the exponent as integers.  t is clamped to
 // tmin = -126 - nrow (the result underflows to ~1e-38 instead of wrapping).  Relative error <= 1.0e-7
 // (fp32 Horner), mean 4e-10 (fit and figures: DESIGN.md section 4).
-template <bool MUFU, bool SLOW>
-__device__ __forceinline__ void exp2x2(unsigned long long t, float tmin, float tmax, uint32_t nsh, float nrow, float& r0f, float& r1f) {
+template <bool SLOW>
+__device__ __forceinline__ void exp2x2(unsigned long long t, float tmin, float tmax, uint32_t nsh, float& r0f, float& r1f) {
     float t0, t1;
     unpack2(t, t0, t1);
-    if (MUFU) {       // A/B variant: ex2.approx (max rel. error 2^-22, unknown mean)
-        t0 += nrow; t1 += nrow;
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r0f) : "f"(t0));
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r1f) : "f"(t1));
-        return;
-    }
     t0 = fmaxf(t0, tmin);                     // fmaxf also drops a NaN (0 * inf of a degenerate row)
     t1 = fmaxf(t1, tmin);
     if (SLOW) { t0 = fminf(t0, tmax); t1 = fminf(t1, tmax); }
@@ -134,7 +128,6 @@ __device__ unsigned long long g_svm_dbg[16];
 #define SDBG_ADD(acc, a, b)
 #endif
 
-template <bool MUFU>
 __global__ void __launch_bounds__(svmtc::NT, 1)
 svm_rbf_tc_kernel(const double* __restrict__ z, int n_cells, const int32_t* __restrict__ n_dev, int D, int Dpad,
                   const __half* __restrict__ sv_hi, const __half* __restrict__ sv_lo,
@@ -392,8 +385,8 @@ svm_rbf_tc_kernel(const double* __restrict__ z, int n_cells, const int32_t* __re
                         const unsigned long long ta = fma2(a01, rf2, fma2(a01, rfl2, pack2(g.x, g.y)));
                         const unsigned long long tb = fma2(a23, rf2, fma2(a23, rfl2, pack2(g.z, g.w)));
                         float e0, e1, e2, e3;
-                        exp2x2<MUFU, false>(ta, tmin, tmax, nsh, nrc, e0, e1);
-                        exp2x2<MUFU, false>(tb, tmin, tmax, nsh, nrc, e2, e3);
+                        exp2x2<false>(ta, tmin, tmax, nsh, e0, e1);
+                        exp2x2<false>(tb, tmin, tmax, nsh, e2, e3);
                         s0 += e0; s1 += e1; s2 += e2; s3 += e3;
                     }
                 } else {
@@ -404,8 +397,8 @@ svm_rbf_tc_kernel(const double* __restrict__ z, int n_cells, const int32_t* __re
                         const unsigned long long ta = add2(fma2(a01, rf2, fma2(a01, rfl2, pack2(g.x, g.y))), rem2);
                         const unsigned long long tb = add2(fma2(a23, rf2, fma2(a23, rfl2, pack2(g.z, g.w))), rem2);
                         float e0, e1, e2, e3;
-                        exp2x2<MUFU, true>(ta, tmin, tmax, nsh, nrc, e0, e1);
-                        exp2x2<MUFU, true>(tb, tmin, tmax, nsh, nrc, e2, e3);
+                        exp2x2<true>(ta, tmin, tmax, nsh, e0, e1);
+                        exp2x2<true>(tb, tmin, tmax, nsh, e2, e3);
                         s0 += e0; s1 += e1; s2 += e2; s3 += e3;
                     }
                 }
@@ -821,8 +814,7 @@ int k_svm_tc(cia_ctx* h, const SvmModel& m, const double* z, int n, const int32_
     if (stages < 3) return CIA_OK;
     stages = std::min(stages, MAX_STAGES);
     const int smem_b = a_bytes + stages * STAGE_B;
-    static const bool mufu = getenv("CIA_SVM_MUFU") != nullptr;       // A/B switch: ex2.approx instead of the polynomial
-    auto kern = mufu ? svm_rbf_tc_kernel<true> : svm_rbf_tc_kernel<false>;
+    auto kern = svm_rbf_tc_kernel;
     if (first_use(h, (const void*)kern))
         CIA_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem_optin - STATIC_SMEM_EST));
     const int n_ct = (n + TM - 1) / TM;
@@ -840,7 +832,7 @@ int k_svm_tc(cia_ctx* h, const SvmModel& m, const double* z, int n, const int32_
     // mean deficit of the full-magnitude round-toward-zero accumulations of a flush group, in units of 2^-25
     // (a flush group is FL = 2 stages = four hi*hi k-steps whose running sum is truncated four times:
     // (1/4 + 2/4 + 3/4 + 1) = 2.5 mean truncations of the group sum)
-    static const double debias = [] { const char* e = getenv("CIA_SVM_DEBIAS"); return e ? atof(e) : 2.5; }();
+    constexpr double debias = 2.5;
     const double fac_base = std::ldexp(2.0 * m.gamma * LOG2E, -m.tc_es) * (1.0 + debias * 2.9802322387695312e-8);
     kern<<<grid, NT, smem_b, s>>>(z, n, n_dev, m.dim, m.dim_pad, (const __half*)m.tc_hi, (const __half*)m.tc_lo, m.tc_gcol, m.tc_svt, fac_base,
                                   m.gamma, per_cta, stages, std::ldexp(1.0, m.tc_fx), partial, n, rowmul);

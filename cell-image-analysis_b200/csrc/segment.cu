@@ -278,11 +278,6 @@ struct SegConvArgs {
     int H, W;            // output resolution
     int F;               // fields: every map is [F][...] with the field outermost, units are decomposed per field
     int c0, c1, mode, ntaps, groups, chunks;
-    // mode 3 (seg_conv_ws_kernel only): the input IS the first layer, evaluated by the producer warps on the fly from
-    // the normalized fp32 image: ReLU(conv3x3(img, w1) + b1) with c0 output channels (seg_first_kernel's arithmetic)
-    const float* img;
-    const float* w1;
-    const float* b1;
     // seg_conv_tma_kernel: POOL 1 / 2 also writes (only writes) MaxPooling2D((2, 2)) of the output for the next layer
     __half* out_pool;
 };
@@ -797,7 +792,6 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
     extern __shared__ __align__(1024) unsigned char smem[];
     __shared__ __align__(8) uint64_t full[T::STAGES], empty[T::STAGES], tfull[2], tempty[2];
     __shared__ uint32_t tmem_base_s;
-    __shared__ __align__(16) float s_first[10 * 128];      // mode 3: first-layer weights [9][c0] and bias [c0]
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int tiles_x = (a.W + 8 * TILES - 1) / (8 * TILES), tiles_y = (a.H + 15) / 16;
     const int per_field = tiles_x * tiles_y, per_group = per_field * a.F;    // unit = (group, field, tile)
@@ -811,8 +805,6 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
         mbar_init(&tempty[0], 8); mbar_init(&tempty[1], 8);
         fence_barrier_init();
     }
-    if (a.mode == 3)
-        for (int i = tid; i < 10 * a.c0; i += T::THREADS) s_first[i] = i < 9 * a.c0 ? a.w1[i] : a.b1[i - 9 * a.c0];
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -831,7 +823,6 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
             const int y0 = 16 * ty, x0 = 8 * TILES * tx;
             const uint4 *s0, *s1;
             seg_src(a, f, s0, s1);
-            const float* fimg = a.img + (size_t)f * a.H * a.W;
             for (int kc = 0; kc < a.chunks; ++kc, ++step) {
                 const int s = step % T::STAGES;
                 mbar_wait(&empty[s], (uint32_t)(((step / T::STAGES) & 1) ^ 1));
@@ -839,50 +830,6 @@ __global__ void __launch_bounds__(SegWsCfg<N, TILES>::THREADS, 1) seg_conv_ws_ke
                 unsigned char* sw = sa + C::A_B;
                 const uint4* wsrc = a.w + (size_t)(g * a.chunks + kc) * w_units;
                 for (int i = pt; i < w_units; i += T::PROD) reinterpret_cast<uint4*>(sw)[i] = __ldg(wsrc + i);
-                if (a.mode == 3) {
-                    // one thread per pixel of the block: 9 image taps, the chunk's 32 first-layer channels as packed
-                    // fp32x2 FMAs (bias first, taps in order: bit-identical to seg_first_kernel), four 16-byte stores
-                    const ulonglong2* w2 = reinterpret_cast<const ulonglong2*>(s_first);
-                    for (int px = pt; px < 18 * C::COLS; px += T::PROD) {
-                        const int ry = px / C::COLS, rc = px - ry * C::COLS;
-                        const int y = y0 + ry - 1, x = x0 + rc - 1;
-                        const bool inside = y >= 0 && y < a.H && x >= 0 && x < a.W;
-                        unsigned long long v2[9];
-#pragma unroll
-                        for (int t = 0; t < 9; ++t) {
-                            const int yy = y + t / 3 - 1, xx = x + t % 3 - 1;
-                            const float v = (inside && yy >= 0 && yy < a.H && xx >= 0 && xx < a.W) ? __ldg(fimg + (size_t)yy * a.W + xx) : 0.f;
-                            v2[t] = pack2(v, v);
-                        }
-#pragma unroll 1
-                        for (int c = 0; c < SEG_KC / 8; ++c) {
-                            const int ch = kc * SEG_KC + c * 8;
-                            unsigned long long acc[4];
-                            {
-                                const ulonglong2 b0 = w2[(9 * a.c0 + ch) / 4], b1 = w2[(9 * a.c0 + ch) / 4 + 1];
-                                acc[0] = b0.x; acc[1] = b0.y; acc[2] = b1.x; acc[3] = b1.y;
-                            }
-#pragma unroll
-                            for (int t = 0; t < 9; ++t) {
-                                const ulonglong2 w0 = w2[(t * a.c0 + ch) / 4], w1v = w2[(t * a.c0 + ch) / 4 + 1];
-                                acc[0] = fma2(v2[t], w0.x, acc[0]); acc[1] = fma2(v2[t], w0.y, acc[1]);
-                                acc[2] = fma2(v2[t], w1v.x, acc[2]); acc[3] = fma2(v2[t], w1v.y, acc[3]);
-                            }
-                            __align__(16) __half o[8];
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) {
-                                float lo, hi;
-                                unpack2(acc[k], lo, hi);
-                                o[2 * k] = __float2half_rn(inside ? fmaxf(lo, 0.f) : 0.f);
-                                o[2 * k + 1] = __float2half_rn(inside ? fmaxf(hi, 0.f) : 0.f);
-                            }
-                            *reinterpret_cast<uint4*>(sa + (size_t)((c * 18 + ry) * C::COLS + rc) * 16) = *reinterpret_cast<const uint4*>(o);
-                        }
-                    }
-                    fence_async_smem();
-                    mbar_arrive(&full[s]);
-                    continue;
-                }
                 constexpr int SB = ((C::NU + T::PROD - 1) / T::PROD + 1) / 2;
 #pragma unroll 1
                 for (int i0 = pt; i0 < C::NU; i0 += SB * T::PROD) {
@@ -1887,28 +1834,12 @@ int k_seg_predict(cia_ctx* h, const float* img, int F, int H, int W, float* prob
     m->prob_map = (float*)(base + prob_off); m->dist_map = (float*)(base + dist_off);
     m->last_hg = Hg; m->last_wg = Wg;
 
-    // the first layer (Cin = 1) is evaluated inside the second layer's producer warps when that layer reads it
-    // directly: no 2 x 268 MB round trip of the full-resolution 32-channel map through HBM, one launch less
-    const bool fuse_first = h->seg_fuse_first && m->ops.size() >= 2 && m->ops[0].mode == -1 && m->ops[1].mode == 0 &&
-                            m->ops[1].src0 == m->ops[0].dst && m->conv[0].cout % SEG_KC == 0 && m->conv[0].cout <= 128;
     std::vector<char> pooled_by_producer(m->ops.size(), 0);
     for (size_t l = 0; l < m->ops.size(); ++l) {
         const SegOp& op = m->ops[l];
         const SegConv& c = m->conv[l];
         const int Ho = H >> op.shift, Wo = W >> op.shift;
         __half* out = (__half*)(base + off[op.dst]);
-        if (fuse_first && l == 0) continue;
-        if (fuse_first && l == 1) {
-            SegConvArgs a{};
-            a.w = (const uint4*)c.w_img; a.bias = c.bias; a.out = out;
-            a.H = Ho; a.W = Wo; a.F = F; a.c0 = op.c0; a.c1 = 0; a.mode = 3; a.ntaps = 9; a.groups = c.groups; a.chunks = c.chunks;
-            a.img = img; a.w1 = m->conv[0].w32; a.b1 = m->conv[0].bias;
-            if (c.n_tile == 128) rc = launch_seg_conv_ws<128, 2>(h, a, s);
-            else if (c.n_tile == 64) rc = launch_seg_conv_ws<64, 4>(h, a, s);
-            else rc = launch_seg_conv_ws<32, 4>(h, a, s);
-            if (rc) return rc;
-            continue;
-        }
         if (op.mode == -1) {
             const size_t n = (size_t)F * Ho * ((Wo + 1) / 2);
             seg_first_kernel<<<(unsigned)((n + 255) / 256), 256, 10 * c.cout * sizeof(float), s>>>(img, c.w32, c.bias, out, Ho, Wo, c.cout, F);

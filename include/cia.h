@@ -123,8 +123,6 @@ int  cia_check_status(cia_handle h, void* stream);
  *                     faster; 2: for every layer the TMA kernel does not take; 0: off
  *   "seg_pool_out"    1 (default): a TMA-fed layer whose output the next layer max-pools writes the pooled copy itself
  *                     (and only that, where nothing else reads the full-resolution map); 0: the consumer pools (bit-identical)
- *   "seg_fuse_first"  1: the Cin = 1 layer evaluated inside the second layer's producer warps (bit-identical,
- *                     measured slower); 0 (default): two launches
  * A `precision` 0 call (cia_screen_fields*, cia_cae_forward) is the exact anchor end to end and uses the
  * fp64 scoring kernels whatever these options say. */
 int  cia_set_option(cia_handle h, const char* name, double value);

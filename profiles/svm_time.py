@@ -1,5 +1,5 @@
 """Times cia_svm_decision (scaler/PCA + both detectors) at the default artifact sizes and at
-config 4 (20k SVs x 256-d). CIA_SVM_DIRECT=1 selects the direct-difference kernel (A/B)."""
+config 4 (20k SVs x 256-d)."""
 import os, sys, time
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -21,7 +21,7 @@ def run(tag, arts, n, reps=5):
     ms = e0.elapsed_time(e1) / reps
     sv = sum(arts[k]["sv"].shape[0] for k in ("svm_conservative", "svm_moderate"))
     D = arts["scaler_pca"]["C"]
-    print(f"{tag}: n={n} D={D} nSV(total)={sv} direct={'CIA_SVM_DIRECT' in os.environ} "
+    print(f"{tag}: n={n} D={D} nSV(total)={sv} "
           f"{ms:.3f} ms per call (PCA + 2 SVM), SVM GEMM-form {2*D*sv*n/ms/1e9:.2f} TFLOP/s if SVM-only, "
           f"checksum {float(out[0][:n].sum()):.12e}")
     eng.close()

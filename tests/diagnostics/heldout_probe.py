@@ -35,7 +35,7 @@ for seed, scale, nneg in SETS:
     for mode in modes:
         for deb in ((0.5, 2.4, 1.2), (0, 0, 0)) if mode in (1, 3) else ((0, 0, 0),):
             for name, v in zip(("cae_l1_debias", "cae_l2_debias", "cae_l3_debias"), deb):
-                eng.set_option(name, v) if not (os.environ.get("CIA_L2_DEBIAS") and name == "cae_l2_debias" and v) else None
+                eng.set_option(name, v)
             mse, mae, feat = eng.cae_forward(x, n, precision=mode)
             dc, dm, pc, pm, _ = eng.svm_decision(feat, n)
             f = feat[:n].cpu().numpy()

@@ -17,7 +17,7 @@ from cell_image_analysis_b200 import synth             # noqa: E402
 H = W = int(os.environ.get("SEG_SIDE", "2048"))
 w = sd.random_model(T.CFG, seed=11)
 m = StarDist2D.from_arrays(T.CFG, w, {"prob": 0.479071, "nms": 0.3})
-for opt in ("seg_fuse_first", "seg_conv_tma", "seg_conv_ws"):      # A/B runs: SEG_FUSE_FIRST=1 etc.
+for opt in ("seg_conv_tma", "seg_conv_ws"):      # A/B runs: SEG_CONV_TMA=0 etc.
     if os.environ.get(opt.upper()):
         m.engine.set_option(opt, float(os.environ[opt.upper()]))
 green, _ = synth.make_field(0, 2048, 2048, *synth.FIELD_CONFIGS["config1"][2:])

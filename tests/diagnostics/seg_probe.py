@@ -46,7 +46,7 @@ def main():
     m = StarDist2D.from_arrays(T.CFG, w, {"prob": 0.479071, "nms": 0.3})
     m.oracle_weights = w
     eng = m.engine
-    for opt in ("seg_fuse_first", "seg_conv_tma", "seg_conv_ws"):      # A/B runs: SEG_FUSE_FIRST=1 etc.
+    for opt in ("seg_conv_tma", "seg_conv_ws"):      # A/B runs: SEG_CONV_TMA=0 etc.
         if os.environ.get(opt.upper()):
             eng.set_option(opt, float(os.environ[opt.upper()]))
 

@@ -29,19 +29,15 @@ under a 1e-3 gate.  Here every layer is judged on its own:
   error / bound ratio of every layer is printed even when the test passes.
 
 The CPU tests at the bottom check the reference itself (no GPU needed): chained without fp16
-rounding or packing it must reproduce ``oracle.cae.forward``, and the weight-image mirror must
-reconstruct the weights and the up-sampled convolution.
-
-    python tests/test_gpu_cae_layers.py --child CROPS.npy   # one per-layer check in a fresh process
-                                                           # (the CIA_* kernel-variant variables are read once)
+rounding or packing it must reproduce ``oracle.cae.forward``, the weight-image mirror must
+reconstruct the weights and the up-sampled convolution, and the layer-2 gate must reject a layer 2
+that leaves out one of the split-precision cross products.
 """
 from __future__ import annotations
 
 import ctypes as C
-import json
 import math
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -69,15 +65,6 @@ COUT = [32, 64, 32, 32, 64, 32, 1]
 # ws_misc buffers in k_cae_forward_tc order: (name, channel chunks of 8, resolution)
 WS_BUFFERS = (("A1h", 4, 32), ("A1l", 4, 32), ("A2h", 8, 16), ("A2l", 8, 16), ("A3h", 4, 8),
               ("A4u", 4, 8), ("A5u", 8, 16), ("A6", 4, 32))
-# the kernel variants that run the same arithmetic (environment, read once per process)
-VARIANTS = [{"CIA_L1_KERNEL": "0"}, {"CIA_L2_TAPS_PER_FLUSH": "0"}, {"CIA_L2_TAPS_PER_FLUSH": "1"},
-            {"CIA_L2_TAPS_PER_FLUSH": "2"}, {"CIA_L2_TAPS_PER_FLUSH": "9"}, {"CIA_L2_STACK": "1"},
-            {"CIA_L3_KERNEL": "1"}, {"CIA_L3_TAPS_PER_FLUSH": "3"}, {"CIA_L7_KERNEL": "0"}]
-# negative control: this timing experiment drops the lo x W_hi MMAs of layer 2
-BROKEN_L2 = {"CIA_L2_STACK": "3", "CIA_L2_TAPS_PER_FLUSH": "3"}
-VARIANT_ENV = ("CIA_L1_KERNEL", "CIA_L2_TAPS_PER_FLUSH", "CIA_L2_STACK", "CIA_L3_KERNEL",
-               "CIA_L3_TAPS_PER_FLUSH", "CIA_L7_KERNEL", "CIA_CAE_CHUNK", "CIA_L1_DEBIAS", "CIA_L2_DEBIAS",
-               "CIA_L3_DEBIAS")
 
 
 # ---------------------------------------------------------------------------------------------
@@ -157,8 +144,8 @@ def tapsum_form(k, dtype=np.float32):
 
 def pack_weights(w: dict):
     """The tensor-core weight images of k_cae_tc_prepare, per layer: scale exponent, inverse scale and
-    the fp16 hi / lo images (standard HWIO; layer 6 in phase form; layer 7 in phase form for the
-    nine-tap kernel and in tap-sum form for final_tapsum_kernel, with kp's scale).  The sign of the BN
+    the fp16 hi / lo images (standard HWIO; layers 6 and 7 in phase form, whose scale layer 7 uses;
+    layer 7 also in tap-sum form for final_tapsum_kernel, with the phase form's scale).  The sign of the BN
     scale that the pooling layers fold into their columns is left out: fp16 rounding is symmetric, so
     the folded products are the unfolded ones negated, and max(sign * c) undone equals the pooled f(c)."""
     packs = []
@@ -247,6 +234,13 @@ def store_bound(y, dy, split):
     return dy + (2.0 ** -22 * mag + 2.0 ** -25 if split else half_ulp16(mag))
 
 
+def split_store(y):
+    """fp16 hi and lo of the fp32 value, as split_store8 stores an activation."""
+    o = y.float()
+    hi = o.half()
+    return hi.double(), (o - hi.float()).half().double()
+
+
 def split_conv(ahi, alo, whi, wlo, op=conv):
     """hi*hi + hi*lo + lo*hi (lo*lo dropped) and the same over absolute values."""
     acc = op(ahi, whi) + op(ahi, wlo) + op(alo, whi)
@@ -265,21 +259,17 @@ def hi_conv(a, w, op=conv):
 # rec (1 - rec) r; the add 1 + e (2^-24) and the division (2 x 2^-23) move it relatively.
 SIG_EXP_ULP = (2.0, 1.173)
 SIG_DIV_ULP = 2.0
-# sequential fp32 additions a per-pixel term passes through on its way into MSE / MAE:
-#   final_tapsum_kernel: 8 per thread + 5 warp_sum levels + 16 per-warp sums  = 29
-#   conv_tc_kernel<EPI_FINAL>: 8 per thread + 5 + 8 per-warp sums + 1 atomicAdd of two bands = 22
-REDUCE_DEPTH = {True: 29, False: 22}
+# sequential fp32 additions a per-pixel term passes through on its way into MSE / MAE in
+# final_tapsum_kernel: 8 per thread + 5 warp_sum levels + 16 per-warp sums
+REDUCE_DEPTH = 29
 
 
-def l7_reference(a6, X, pk, bias, tapsum: bool):
+def l7_reference(a6, X, pk, bias):
     """Per-cell (mse, mae, mse bound, mae bound) of layer 7 on the device's A6 (hi only)."""
     dev = a6.device
-    if tapsum:   # hi and lo weight columns: 2 RZ steps each, their sum and 3 tap-sum adds (2^-24 each)
-        acc, S = split_conv(a6, torch.zeros_like(a6), _t(pk["t_hi"], dev), _t(pk["t_lo"], dev), tapsum_conv)
-        steps = 2 + 4 * U / EPS
-    else:        # nine-tap phase form, hi weights: 9 taps x 2 K16 steps
-        acc, S = hi_conv(a6, _t(pk["hi"], dev), phase_conv)
-        steps = 18
+    # hi and lo weight columns: 2 RZ steps each, their sum and 3 tap-sum adds (2^-24 each)
+    acc, S = split_conv(a6, torch.zeros_like(a6), _t(pk["t_hi"], dev), _t(pk["t_lo"], dev), tapsum_conv)
+    steps = 2 + 4 * U / EPS
     b = float(bias[0])
     a = acc[:, 0] * pk["inv"] + b
     amag = S[:, 0] * pk["inv"] + abs(b)
@@ -290,7 +280,7 @@ def l7_reference(a6, X, pk, bias, tapsum: bool):
     x = _t(X, dev)
     d = x - rec
     dd = drec + U * (d.abs() + drec)                                        # the fp32 subtraction
-    g = REDUCE_DEPTH[tapsum] * U * 1.001
+    g = REDUCE_DEPTH * U * 1.001
     sq_b = 2 * d.abs() * dd + dd * dd
     mse = (d * d).sum((1, 2)) / 4096
     mae = d.abs().sum((1, 2)) / 4096
@@ -343,7 +333,38 @@ def read_taps(eng, n, pass_cells):
     return out, c0, chunk
 
 
-def check_layers(tag, w, packs, X, taps, mse, mae, feat, cells, path, l1_tc=True, l7_tapsum=True, dev="cuda"):
+def l1_reference(x, w, packs, bn, split):
+    """Layer 1's pooled output and bound from the crops x [cell][1][64][64]: conv1_tc_split_kernel
+    (split) or conv1_fp32_planar_kernel."""
+    dev = x.device
+    if split:    # the input scaled by 2^XSCALE_EXP and split into fp16 hi / lo, 3 MMAs of one K16 step
+        v = (x * 2.0 ** XSCALE_EXP).float()
+        xh = v.half().double()
+        xl = (v - v.half().float()).half().double()
+        acc, S = split_conv(xh, xl, _t(packs[0]["hi"], dev), _t(packs[0]["lo"], dev))
+        y, dy = act(acc, S, packs[0]["inv"], w["biases"][0], *bn[0], 3, DEBIAS[0], 2)
+    else:        # fp32 weights and crops, a 9-FMA chain started at the bias
+        acc, S = hi_conv(x.double(), _t(w["kernels"][0], dev))
+        y, dy = act(acc, S, 1.0, w["biases"][0], *bn[0], 0, 0.0, 9)
+    return pool2(y), pool2(dy)
+
+
+def check_l2(rep, w, packs, bn, a1h, a1l, a2, split, cells):
+    """The layer-2 gate: the reference of layer 2 on the device's layer-1 output (a1h, and a1l on the
+    split path) against the device's layer-2 output a2 (hi + lo on the split path).  The accumulating
+    kernel of the split path: 3 x 9 x Cin/16 MMAs + at most 18 fp32 flush adds."""
+    whi, wlo = _t(packs[1]["hi"], a1h.device), _t(packs[1]["lo"], a1h.device)
+    if split:
+        acc, S = split_conv(a1h, a1l, whi, wlo)
+        y, dy = act(acc, S, packs[1]["inv"], w["biases"][1], *bn[1], 3 * 9 * 2 + 18, DEBIAS[1], 2)
+    else:
+        acc, S = hi_conv(a1h, whi)
+        y, dy = act(acc, S, packs[1]["inv"], w["biases"][1], *bn[1], 9 * 2, 0.0, 2)
+    y, dy = pool2(y), pool2(dy)
+    rep.check("L2", a2, y, store_bound(y, dy, split), cells)
+
+
+def check_layers(tag, w, packs, X, taps, mse, mae, feat, cells, path, dev="cuda"):
     """Judge L1..L7 of one tensor-core call.  path 1: split L1-L3 (features tapped from L3); path 2: the
     fp32 layer 1 and single-pass L2 / L3 (precision 2, and precision 1 with a separate encoder).
     X: the crops of ``cells``; taps: their activations (read_taps); mse / mae / feat: the call's outputs
@@ -356,29 +377,12 @@ def check_layers(tag, w, packs, X, taps, mse, mae, feat, cells, path, l1_tc=True
     hw = [(_t(p["hi"], dev), _t(p["lo"], dev)) for p in packs]
 
     # L1
-    if split and l1_tc:
-        v = (x * 2.0 ** XSCALE_EXP).float()
-        xh = v.half().double()
-        xl = (v - v.half().float()).half().double()
-        acc, S = split_conv(xh, xl, *hw[0])
-        y, dy = act(acc, S, packs[0]["inv"], w["biases"][0], *bn[0], 3, DEBIAS[0], 2)
-    else:        # conv1_fp32_planar_kernel: fp32 weights and crops, a 9-FMA chain started at the bias
-        acc, S = hi_conv(x.double(), _t(w["kernels"][0], dev))
-        y, dy = act(acc, S, 1.0, w["biases"][0], *bn[0], 0, 0.0, 9)
-    y, dy = pool2(y), pool2(dy)
+    y, dy = l1_reference(x, w, packs, bn, split)
     a1 = T["A1h"] + T["A1l"] if split else T["A1h"]
     rep.check("L1", a1, y, store_bound(y, dy, split), cells)
 
-    # L2 (pool layers' accumulating kernels: 3 x 9 x Cin/16 MMAs + at most 18 fp32 flush adds)
-    if split:
-        acc, S = split_conv(T["A1h"], T["A1l"], *hw[1])
-        y, dy = act(acc, S, packs[1]["inv"], w["biases"][1], *bn[1], 3 * 9 * 2 + 18, DEBIAS[1], 2)
-    else:
-        acc, S = hi_conv(T["A1h"], hw[1][0])
-        y, dy = act(acc, S, packs[1]["inv"], w["biases"][1], *bn[1], 9 * 2, 0.0, 2)
-    y, dy = pool2(y), pool2(dy)
-    a2 = T["A2h"] + T["A2l"] if split else T["A2h"]
-    rep.check("L2", a2, y, store_bound(y, dy, split), cells)
+    # L2
+    check_l2(rep, w, packs, bn, T["A1h"], T["A1l"], T["A2h"] + T["A2l"] if split else T["A2h"], split, cells)
 
     # L3
     if split:
@@ -414,7 +418,7 @@ def check_layers(tag, w, packs, X, taps, mse, mae, feat, cells, path, l1_tc=True
     rep.check("L6", T["A6"], y, store_bound(y, dy, False), cells)
 
     # L7: MSE / MAE
-    rm, ra, bm, ba = l7_reference(T["A6"], X, packs[6], w["biases"][6], l7_tapsum)
+    rm, ra, bm, ba = l7_reference(T["A6"], X, packs[6], w["biases"][6])
     col = lambda v: torch.from_numpy(np.asarray(v, np.float64)).to(dev)  # noqa: E731
     rep.check("L7 mse", col(mse), rm, bm, cells, kind="cell")
     rep.check("L7 mae", col(mae), ra, ba, cells, kind="cell")
@@ -478,7 +482,7 @@ def make_engine(w, encoder=None):
 
 
 def run_and_check(eng, tag, w, packs, X, n, precision, path, n_dev=None, pass_cells=PASS_CELLS,
-                  l1_tc=True, l7_tapsum=True, feat_from_tc=None):
+                  feat_from_tc=None):
     """One cae_forward call on the first n crops, then the per-layer check of its last pass."""
     x = torch.from_numpy(np.ascontiguousarray(X[:n])).to(eng.tdev)
     mse, mae, feat = eng.cae_forward(x, n, n_dev=n_dev, precision=precision)
@@ -488,7 +492,7 @@ def run_and_check(eng, tag, w, packs, X, n, precision, path, n_dev=None, pass_ce
     cells = np.arange(c0, n)
     tc_feat = path == 1 if feat_from_tc is None else feat_from_tc
     rep = check_layers(tag, w, packs, X[c0:n], taps, mse[c0:], mae[c0:], feat[c0:] if tc_feat else None,
-                       cells, path, l1_tc, l7_tapsum, dev=str(eng.tdev))
+                       cells, path, dev=str(eng.tdev))
     return rep, (mse, mae, feat)
 
 
@@ -625,67 +629,6 @@ def test_n_cells_dev_contract(engines, layer_crops):
             for a, b, name in zip(got, sub, ("mse", "mae", "features")):
                 assert np.array_equal(a[:173].view(np.int32), b.view(np.int32)), f"precision 2 {name} of cells < 173"
         assert not got[0][173:].any() and not got[1][173:].any(), f"precision {prec}: mse / mae beyond the device count"
-
-
-def _child_env(extra):
-    env = {k: v for k, v in os.environ.items() if k not in VARIANT_ENV}
-    env.update(extra)
-    return env
-
-
-@pytest.mark.gpu
-def test_kernel_variants(tmp_path, layer_crops):
-    """Every same-arithmetic A/B variant selected by environment (each read once per process, so each
-    runs in a child process) meets the per-layer gate on one small case; the variant that drops layer
-    2's lo x W_hi products must fail it at L2 by a large factor (the gate has teeth)."""
-    crops = tmp_path / "crops.npy"
-    np.save(crops, layer_crops[:149])
-    runs = VARIANTS + [BROKEN_L2]
-    procs = []
-    try:
-        for v in runs:
-            out = tmp_path / ("variant_%d.json" % len(procs))
-            procs.append((v, out, subprocess.Popen([sys.executable, os.path.abspath(__file__), "--child", str(crops),
-                                                    str(out)], env=_child_env(v), cwd=ROOT,
-                                                   stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
-        logs = [p.communicate(timeout=900)[0] for _, _, p in procs]
-    finally:
-        for _, _, p in procs:
-            if p.poll() is None:
-                p.kill()
-                p.wait()
-    problems = []
-    for (v, out, p), log in zip(procs, logs):
-        if not out.exists():
-            problems.append(f"{v}: child exited {p.returncode} without a result:\n{log[-3000:]}")
-            continue
-        res = json.loads(out.read_text())
-        print(f"{v}: " + "  ".join(f"{k} {r:.3g}" for k, r in res["ratio"].items()))
-        if v is BROKEN_L2:
-            if not res["ratio"].get("L2", 0.0) > 10.0:
-                problems.append(f"{v}: the L2 gate did not catch the dropped lo x W_hi MMAs: {res['ratio']}")
-        elif res["failures"] or p.returncode != 0:
-            problems.append(f"{v}: exit {p.returncode}\n" + "\n".join(res["failures"]))
-    assert not problems, "\n".join(problems)
-
-
-def _child_main(crops_path, out_path):
-    X = np.load(crops_path)
-    from cell_image_analysis_b200.artifacts import load_model_dir
-    ae = load_model_dir(os.path.join(HERE, "golden", "model_dir"))["autoencoder"]
-    w = {"kernels": ae["kernels"], "biases": ae["biases"], "bns": ae["bns"]}
-    eng = make_engine(w)
-    try:
-        tag = " ".join(f"{k}={os.environ[k]}" for k in VARIANT_ENV if k in os.environ) or "default"
-        rep, _ = run_and_check(eng, tag, w, pack_weights(w), X, len(X), 1, 1,
-                               l1_tc=os.environ.get("CIA_L1_KERNEL", "1") != "0",
-                               l7_tapsum=os.environ.get("CIA_L7_KERNEL", "1") != "0")
-    finally:
-        eng.close()
-    print(rep.line())
-    with open(out_path, "w") as f:
-        json.dump({"ratio": rep.ratio, "failures": rep.failures}, f)
-    return 1 if rep.failures else 0
 
 
 @pytest.mark.gpu
@@ -854,8 +797,30 @@ def test_ws_layout_rule():
     assert total == 2 * 32768 + 2 * 16384 + 2048 + 2048 + 16384 + 32768     # per_cell halves
 
 
-if __name__ == "__main__":
-    if len(sys.argv) == 4 and sys.argv[1] == "--child":
-        sys.exit(_child_main(sys.argv[2], sys.argv[3]))
-    print(__doc__)
-    sys.exit(2)
+
+def test_l2_gate_catches_dropped_cross_term(oracle_weights, golden_tiny):
+    """The layer-2 gate has teeth: a layer 2 that leaves out the A1l x W_hi products (one of the three
+    split-precision MMAs per k-step) fails it by more than a factor 10, while the correct layer, stored
+    as the device stores it, passes.  Layer 1's output is the reference of layer 1 on the golden tiny
+    crops, stored as fp16 hi / lo."""
+    w = model_sets(oracle_weights)["golden"]
+    packs, bn = pack_weights(w), bn_params(w)
+    X = golden_tiny["crops"].astype(np.float32)
+    cells = np.arange(len(X))
+    y1, _ = l1_reference(torch.from_numpy(X)[:, None], w, packs, bn, True)
+    a1h, a1l = split_store(y1)
+
+    def layer2(cross_lo_hi):
+        whi, wlo = _t(packs[1]["hi"], "cpu"), _t(packs[1]["lo"], "cpu")
+        acc = conv(a1h, whi) + conv(a1h, wlo) + (conv(a1l, whi) if cross_lo_hi else 0)
+        y = pool2(act(acc, acc.abs(), packs[1]["inv"], w["biases"][1], *bn[1], 0, 0.0, 0)[0])
+        return sum(split_store(y))
+
+    good = Report("correct L2")
+    check_l2(good, w, packs, bn, a1h, a1l, layer2(True), True, cells)
+    print(good.line())
+    assert not good.failures, "\n".join(good.failures)
+    bad = Report("L2 without A1l x W_hi")
+    check_l2(bad, w, packs, bn, a1h, a1l, layer2(False), True, cells)
+    print(bad.line())
+    assert bad.ratio["L2"] > 10.0, bad.line()

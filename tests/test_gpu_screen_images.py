@@ -102,15 +102,14 @@ def _predict_one(model, x, Hp, Wp):
 
 
 # option settings that route every layer through each kernel form: TMA-fed (+ pooled output), software-producer,
-# staged, the fused first layer, consumer-side pooling
+# staged, consumer-side pooling
 SETTINGS = {
     "default": {},
     "ws_everywhere": dict(seg_conv_tma=0, seg_conv_ws=2),
     "staged": dict(seg_conv_tma=0, seg_conv_ws=0),
     "no_pool_out": dict(seg_pool_out=0),
-    "fuse_first": dict(seg_fuse_first=1),
 }
-DEFAULTS = dict(seg_conv_tma=1, seg_conv_ws=1, seg_pool_out=1, seg_fuse_first=0)
+DEFAULTS = dict(seg_conv_tma=1, seg_conv_ws=1, seg_pool_out=1)
 
 
 @pytest.mark.parametrize("setting", list(SETTINGS))

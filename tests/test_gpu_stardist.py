@@ -255,21 +255,6 @@ def test_training_twin_with_the_gpu_model(tmp_path):
     assert all(s["file"] == "field_7.tif" and "solidity" in s for s in stats)
 
 
-def test_fused_first_layer_is_bit_identical(model):
-    """seg_fuse_first (an option, off by default: measured slower): the Cin = 1 layer evaluated inside the second
-    layer's producer warps gives the maps of the two-launch route bit for bit (same FMA order, same MMA order)."""
-    rng = np.random.default_rng(12)
-    x = rng.uniform(-0.2, 1.6, (144, 208)).astype(np.float32)
-    eng = model.engine
-    p0, d0 = model.predict(x)
-    eng.set_option("seg_fuse_first", 1)
-    try:
-        p1, d1 = model.predict(x)
-    finally:
-        eng.set_option("seg_fuse_first", 0)
-    assert np.array_equal(p0.cpu().numpy(), p1.cpu().numpy()) and np.array_equal(d0.cpu().numpy(), d1.cpu().numpy())
-
-
 def test_round_trip_through_the_screen(model):
     """true labels -> star maps -> GPU instances -> region scan, gates, crops, scores: the objects come back (labels
     bit-equal to the oracle's instances, IoU > 0.9 with the truth) and the screen keeps the same cells as it does on
