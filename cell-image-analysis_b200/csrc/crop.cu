@@ -613,9 +613,9 @@ crop_fast_kernel(const uint16_t* __restrict__ images, int H, int W, const cia_ce
         int mn = 65535, mx = 0;
         {
             const int chunks = L.pitch >> 3;
-            const unsigned c_magic = k_magic.v[chunks];                  // chunks in 2..13
+            const unsigned c_magic = k_magic.v[chunks];                  // chunks in 1..13 (1: w == 1, no magic)
             for (int i = tid; i < h * chunks; i += KF_THREADS) {
-                const int y = (int)__umulhi((unsigned)i, c_magic), c = i - y * chunks;
+                const int y = (chunks == 1) ? i : (int)__umulhi((unsigned)i, c_magic), c = i - y * chunks;
                 const int e0 = (e00 + y * wlow) & 7;
                 const int first = 8 * c - e0;                            // bbox column of the chunk's first pixel
                 if (first >= w) continue;

@@ -119,24 +119,11 @@ def interpolate(bins: np.ndarray, maps: np.ndarray, k) -> np.ndarray:
     return res.astype(np.uint16)
 
 
-def equalize_adapthist(cell: np.ndarray, clip_limit: float = 0.02) -> np.ndarray:
-    """det:98.  uint16 [h, w] -> float64 [h, w] in [0, 1]."""
-    q = quantise(cell)
-    k = kernel_size(cell.shape)
-    before, after = padding(cell.shape, k)
-    qp = np.pad(q, [(before[0], after[0]), (before[1], after[1])], mode="reflect")
-    bins = (qp // BIN_SIZE).astype(np.uint16)
+def clip_count(clip_limit: float, k) -> int:
+    """A.2 step 5: the per-bin count limit of a tile of ``k[0] x k[1]`` pixels; clip_limit 0 is plain
+    AHE (no clipping)."""
     npx = k[0] * k[1]
-    clim = int(np.clip(clip_limit * npx, 1, None)) if clip_limit > 0 else NR_OF_GRAY
-    maps = tile_maps(bins, k, clim)
-    res = interpolate(bins, maps, k)
-    res = res[before[0]: res.shape[0] - after[0], before[1]: res.shape[1] - after[1]]
-    r = res.astype(np.float64)
-    rmin, rmax = float(r.min()), float(r.max())
-    if rmin != rmax:
-        r = (r - rmin) / (rmax - rmin)
-        return r * 1.0 + 0.0
-    return np.clip(r, 0.0, 1.0)
+    return int(np.clip(clip_limit * npx, 1, None)) if clip_limit > 0 else NR_OF_GRAY
 
 
 def clahe_levels(cell: np.ndarray, clip_limit: float = 0.02) -> np.ndarray:
@@ -146,6 +133,15 @@ def clahe_levels(cell: np.ndarray, clip_limit: float = 0.02) -> np.ndarray:
     before, after = padding(cell.shape, k)
     qp = np.pad(q, [(before[0], after[0]), (before[1], after[1])], mode="reflect")
     bins = (qp // BIN_SIZE).astype(np.uint16)
-    clim = int(np.clip(clip_limit * k[0] * k[1], 1, None))
-    res = interpolate(bins, tile_maps(bins, k, clim), k)
+    res = interpolate(bins, tile_maps(bins, k, clip_count(clip_limit, k)), k)
     return res[before[0]: res.shape[0] - after[0], before[1]: res.shape[1] - after[1]]
+
+
+def equalize_adapthist(cell: np.ndarray, clip_limit: float = 0.02) -> np.ndarray:
+    """det:98.  uint16 [h, w] -> float64 [h, w] in [0, 1]."""
+    r = clahe_levels(cell, clip_limit).astype(np.float64)
+    rmin, rmax = float(r.min()), float(r.max())
+    if rmin != rmax:
+        r = (r - rmin) / (rmax - rmin)
+        return r * 1.0 + 0.0
+    return np.clip(r, 0.0, 1.0)

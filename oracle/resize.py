@@ -49,10 +49,11 @@ def resize_formula(img: np.ndarray, out: int = OUT) -> np.ndarray:
         if sigma > 1e-15:
             w, r = gaussian_weights(sigma)
             idx = _mirror(np.arange(n)[:, None] + np.arange(-r, r + 1)[None, :], n)
-            if ax == 0:
-                a = np.einsum("ikc,k->ic", a[idx], w)
-            else:
-                a = np.einsum("rik,k->ri", a[:, idx], w)
+            # tap by tap: a 1024-px side has 61 taps, too many to gather all at once
+            acc = np.zeros_like(a)
+            for j in range(2 * r + 1):
+                acc += w[j] * (a[idx[:, j]] if ax == 0 else a[:, idx[:, j]])
+            a = acc
     h, w_ = a.shape
 
     def taps(n):
