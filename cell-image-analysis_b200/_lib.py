@@ -52,6 +52,12 @@ REGION_DTYPE = np.dtype([("area", "<u4"), ("minr", "<i4"), ("minc", "<i4"), ("ma
 CELL_DTYPE = np.dtype([("field", "<i4"), ("label", "<i4"), ("minr", "<i4"), ("minc", "<i4"),
                        ("maxr", "<i4"), ("maxc", "<i4"), ("area", "<i4"), ("pad_", "<i4"),
                        ("eccentricity", "<f8"), ("mean_intensity", "<f8"), ("std_intensity", "<f8")])
+# cia_tiff_segment: one compressed strip / tile of a field (cia_tiff_decode_fields)
+TIFF_SEGMENT_DTYPE = np.dtype([("src_off", "<u8"), ("src_len", "<u8"), ("dst_off", "<u8"), ("field", "<i4"),
+                               ("compression", "<i4"), ("predictor", "<i4"), ("bytes_per_sample", "<i4"),
+                               ("big_endian", "<i4"), ("samples", "<i4"), ("y0", "<i4"), ("x0", "<i4"),
+                               ("rows", "<i4"), ("cols", "<i4"), ("seg_sample", "<i4"), ("img_sample", "<i4")])
+assert TIFF_SEGMENT_DTYPE.itemsize == 72
 assert REGION_DTYPE.itemsize == C.sizeof(Region) == 64
 assert CELL_DTYPE.itemsize == C.sizeof(Cell) == 56
 
@@ -95,6 +101,7 @@ SIGNATURES = {
                                            _P, _I, _P, _P, C.POINTER(Scores), _P, _P, _P, _P, _I, _P]),
     "cia_tiff_lzw_decode": (C.c_longlong, [_P, C.c_size_t, _P, C.c_size_t]),
     "cia_tiff_packbits_decode": (C.c_longlong, [_P, C.c_size_t, _P, C.c_size_t]),
+    "cia_tiff_decode_fields": (_I, [_P, _P, C.c_size_t, _P, _I, _I, _I, _I, _P, C.c_size_t, _P, _P, _P, _P]),
     "cia_profile_begin": (_I, [_P, _I]),
     "cia_profile_end": (_I, [_P, C.POINTER(C.c_double), C.POINTER(_I)]),
     "cia_profile_layers": (_I, [_P, C.POINTER(C.c_double)]),

@@ -238,11 +238,14 @@ class BatchScreen:
         self._last_fields = n_fields
         self.last_rle_share = n_rle / max(n_chunks, 1)        # share of the chunks that crossed PCIe as runs
 
-    def _read_back(self, i, b, o):
-        """D2H of chunk i's results (device buffer set b) on the read-back stream"""
+    def _read_back(self, i, b, o, status=None):
+        """D2H of chunk i's results (device buffer set b) on the read-back stream; ``status`` (host, device): chunk
+        i's TIFF decode flags, copied before ``out_free[b]`` lets chunk i + NB decode into the same buffer set"""
         S = self._stage
         with torch.cuda.stream(self.d2h):
             self.d2h.wait_event(S["out_ready"][b])
+            if status is not None:
+                status[0].copy_(status[1], non_blocking=True)
             self.h_counts[i].copy_(o["counts"], non_blocking=True)
             self.h_cells[i].copy_(o["cells"], non_blocking=True)
             self.h_mse[i].copy_(o["mse"], non_blocking=True)
@@ -254,10 +257,14 @@ class BatchScreen:
             S["out_free"][b].record(self.d2h)
 
     def run_images_host(self, seg_pinned: torch.Tensor, images_pinned: torch.Tensor, n_fields: int, prob_thresh: float,
-                        nms_thresh: float, strain_of_visit: torch.Tensor | None = None):
+                        nms_thresh: float, strain_of_visit: torch.Tensor | None = None, tiff=None):
         """``run_host`` with the labels made on the device: only images cross PCIe -- one buffer per chunk when
         ``seg_pinned`` is ``images_pinned`` (single-channel fields), two when the segmentation channel differs.
-        Same chunking, double buffering, read-back and ``collect_host`` as ``run_host``."""
+        Same chunking, double buffering, read-back and ``collect_host`` as ``run_host``.
+        ``tiff``: per chunk None or a ``tiff_device.TiffChunk``; the fields at its slots are not copied from the
+        pinned pools but decoded on the device from their compressed TIFF segments (one copy of the packed chunk on
+        the copy stream, ``cia_tiff_decode_fields`` on the compute stream).  A field the decoder flags takes no part
+        in the per-strain accumulators; ``tiff_status`` [chunk, field] holds the flags after ``collect_host``."""
         P = images_pinned.shape[0]
         assert P % self.Fc == 0 and seg_pinned.shape == images_pinned.shape
         n_chunks = -(-n_fields // self.Fc)          # the last chunk may be short
@@ -266,17 +273,27 @@ class BatchScreen:
         same = seg_pinned is images_pinned
         if not same and "seg" not in S:
             S["seg"] = [torch.empty((self.Fc, self.H, self.W), dtype=torch.int16, device=eng.tdev) for _ in range(self.NB)]
+        tiff = tiff or [None] * n_chunks
+        if any(t is not None for t in tiff):
+            self._ensure_tiff_stage(n_chunks, tiff)
         self.h2d_bytes = 0
         for i in range(n_chunks):
             b = i % self.NB
             p0 = (i * self.Fc) % P
             nf = min(self.Fc, n_fields - i * self.Fc)
+            t = tiff[i]
             with torch.cuda.stream(self.copy):
                 self.copy.wait_event(S["done"][b])
-                S["img"][b][:nf].copy_(images_pinned[p0:p0 + nf], non_blocking=True)
-                if not same:
-                    S["seg"][b][:nf].copy_(seg_pinned[p0:p0 + nf], non_blocking=True)
-                self.h2d_bytes += (1 if same else 2) * 2 * nf * self.H * self.W
+                host = range(nf) if t is None else [k for k in range(nf) if k not in t.slots]
+                runs = [(k, k + 1) for k in host] if t is not None else [(0, nf)]
+                for k0, k1 in runs:
+                    S["img"][b][k0:k1].copy_(images_pinned[p0 + k0:p0 + k1], non_blocking=True)
+                    if not same:
+                        S["seg"][b][k0:k1].copy_(seg_pinned[p0 + k0:p0 + k1], non_blocking=True)
+                self.h2d_bytes += (1 if same else 2) * 2 * len(host) * self.H * self.W
+                if t is not None:
+                    t.upload(S["tiff_src"][b])
+                    self.h2d_bytes += t.total
                 S["ready"][b].record(self.copy)
             with torch.cuda.stream(self.compute):
                 self.compute.wait_event(S["ready"][b])
@@ -284,13 +301,35 @@ class BatchScreen:
                 o = self.out[b]
                 o["counts"][1 + nf:].zero_()            # per-field counts of the fields a short chunk does not have
                 st = None if strain_of_visit is None else strain_of_visit[i * self.Fc:i * self.Fc + nf]
+                if t is not None:
+                    status = S["tiff_status"][b]
+                    t.decode(eng, S["tiff_src"][b], S["tiff_scratch"][b], None if same else S["seg"][b],
+                             S["img"][b], status)
+                    if st is None:                      # every field is strain 0 ...
+                        st = torch.zeros(nf, dtype=torch.int32, device=eng.tdev)
+                    st = torch.where(status[:nf] != 0, -1, st)     # ... except a damaged file's: out of the totals
                 eng.screen_images((S["img"][b] if same else S["seg"][b])[:nf], S["img"][b][:nf], self.max_label, o,
                                   prob_thresh, nms_thresh, field_strain=st, acc=self.acc)
                 S["done"][b].record(self.compute)
                 S["out_ready"][b].record(self.compute)
-            self._read_back(i, b, o)
+            self._read_back(i, b, o, status=(self.tiff_status[i], S["tiff_status"][b]) if t is not None else None)
         self._last_chunks = n_chunks
         self._last_fields = n_fields
+
+    def _ensure_tiff_stage(self, n_chunks, chunks):
+        """grow-only device staging of the compressed chunks (packed bytes, decode scratch, per-field status)"""
+        S, d = self._stage, self.eng.tdev
+        need = max(t.total for t in chunks if t is not None)
+        scratch = max(t.scratch_bytes for t in chunks if t is not None)
+        if "tiff_src" not in S or S["tiff_src"][0].numel() < need:
+            S["tiff_src"] = [torch.empty(need, dtype=torch.uint8, device=d) for _ in range(self.NB)]
+        if "tiff_scratch" not in S or S["tiff_scratch"][0].numel() < max(scratch, 1):
+            S["tiff_scratch"] = [torch.empty(max(scratch, 1), dtype=torch.uint8, device=d) for _ in range(self.NB)]
+        if "tiff_status" not in S:
+            S["tiff_status"] = [torch.zeros(self.Fc, dtype=torch.int32, device=d) for _ in range(self.NB)]
+        if getattr(self, "tiff_status", None) is None or self.tiff_status.shape[0] < n_chunks:
+            self.tiff_status = torch.zeros((n_chunks, self.Fc), dtype=torch.int32, pin_memory=True)
+        self.tiff_status[:n_chunks].zero_()
 
     def collect_host(self):
         """Compact the per-chunk host buffers of the last ``run_host`` into flat arrays.  Raises if

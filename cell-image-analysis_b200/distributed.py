@@ -159,13 +159,16 @@ class GpuFieldScorer:
 
 
     def score_images(self, fields, strains, n_strains, prob_thresh: float, nms_thresh: float, max_label: int = 4096):
-        """``score`` for fields given as (seg channel, green channel) uint16 [H,W] pairs (or zero-argument callables
-        returning one; None = the loader gave up on the file): each chunk is segmented AND screened on the device
+        """``score`` for fields given as (seg channel, green channel) uint16 [H,W] pairs or ``tiff_device.TiffField``
+        compressed files decoded on the device (or zero-argument callables returning one; None = the loader gave up on
+        the file): each chunk is segmented AND screened on the device
         through ``BatchScreen.run_images_host`` (StarDist model loaded on the engine), so only the images cross PCIe
         and the loader threads make no GPU calls.  ``max_label`` bounds the instances of one field (CIA_E_LABEL
         beyond).  Returns what ``score`` returns."""
         from concurrent.futures import ThreadPoolExecutor
         from .batch import BatchScreen
+        from .tiff_device import TiffChunk, TiffField
+        _shape = lambda f: f.shape if isinstance(f, TiffField) else f[1].shape
         dev = self.eng.tdev
         total = torch.zeros((n_strains, ACC_COLS), dtype=torch.float64, device=dev)
         if not fields:
@@ -183,7 +186,7 @@ class GpuFieldScorer:
                 if not ok:
                     out.extend(empty() for _ in chunk)
                     continue
-                H, W = chunk[ok[0]][1].shape
+                H, W = _shape(chunk[ok[0]])
                 bs = self._bs
                 if bs is None or (bs.H, bs.W, bs.n_strains, bs.max_label) != (H, W, n_strains, max_label):
                     if bs is not None:
@@ -193,23 +196,35 @@ class GpuFieldScorer:
                     self._s = torch.zeros((self.Fc, H, W), dtype=torch.int16).pin_memory()
                     self._bs = bs
                 bs.acc.zero_()
-                same = all(chunk[j][0] is chunk[j][1] for j in ok)     # single-channel fields: one upload
+                dev_fields = {k: chunk[j] for k, j in enumerate(ok) if isinstance(chunk[j], TiffField)}
+                same = all(chunk[j].channels == 1 if k in dev_fields else chunk[j][0] is chunk[j][1]
+                           for k, j in enumerate(ok))                  # single-channel fields: one upload
                 for k, j in enumerate(ok):
-                    seg, g = chunk[j]
-                    if seg.shape != (H, W) or g.shape != (H, W):
+                    if _shape(chunk[j]) != (H, W):
                         raise ValueError("a chunk needs equally sized fields (pad or group by size)")
+                    if k in dev_fields:
+                        continue
+                    seg, g = chunk[j]
                     if g.dtype != np.uint16 or seg.dtype not in (np.uint16, np.uint8):
                         raise TypeError("fields must be uint16 (widen 8-bit fields before screening)")
                     self._g[k].copy_(torch.from_numpy(np.ascontiguousarray(g).view(np.int16)))
                     if not same:
                         self._s[k].copy_(torch.from_numpy(np.ascontiguousarray(seg, np.uint16).view(np.int16)))
+                tiff = None
+                if dev_fields:
+                    tiff = [TiffChunk(list(dev_fields.values()), list(dev_fields), getattr(self, "_tiff_pin", None))]
+                    self._tiff_pin = tiff[0].pinned
                 st = torch.tensor([strains[idx[j]] for j in ok], dtype=torch.int32)
-                bs.run_images_host(self._g if same else self._s, self._g, len(ok), prob_thresh, nms_thresh, st.to(dev))
+                bs.run_images_host(self._g if same else self._s, self._g, len(ok), prob_thresh, nms_thresh, st.to(dev),
+                                   tiff=tiff)
                 r = bs.collect_host()                          # synchronises, raises on a device-side status
                 total += bs.acc
                 starts = np.concatenate([[0], np.cumsum(r["field_counts"])])
                 rows = {}
                 for k, j in enumerate(ok):
+                    if k in dev_fields and int(bs.tiff_status[0, k]):     # det:113-115: the file contributes no cells
+                        print(f"Error processing {dev_fields[k].path}: corrupt or truncated compressed TIFF data")
+                        continue
                     s0, s1 = int(starts[k]), int(starts[k + 1])
                     rows[j] = {kk: r[kk][s0:s1].copy() for kk in ROW_KEYS}
                     rows[j]["label"] = r["cells"]["label"][s0:s1].copy()
@@ -259,6 +274,11 @@ class ShardedScreen:
         return acc_np, {k: (np.concatenate(v) if v else np.zeros(0)) for k, v in cols.items()}
 
 
+def _read_file(path):
+    with open(path, "rb") as f:
+        return f.read()
+
+
 def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, chunk_fields: int = 16):
     """Sharded twin of ``ProductionMutantScreening.screen_mutant_samples`` (det:155-244): call it
     from every rank of an initialised process group (one process per GPU; ``screener`` built on that
@@ -266,7 +286,9 @@ def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, 
     sharded round robin, read and segmented on their rank, scored through the fused path; the
     per-strain numbers come from the all-reduced accumulator.  With a GPU StarDist model (``stardist_dir=``)
     the loader threads only read files and split channels; segmentation and screening run per chunk in
-    ``cia_screen_images`` on the rank's stream (no labels through the host).  A caller's own ``segmenter``
+    ``cia_screen_images`` on the rank's stream (no labels through the host).  With the default reader, a compressed
+    uint16 TIFF the device decodes (``tiff_device.device_route``) is only read and its directory parsed by the loader;
+    its compressed strips / tiles cross PCIe and are decoded in ``cia_tiff_decode_fields`` ahead of the screen.  A caller's own ``segmenter``
     keeps the (green, labels) route.  Returns ``(results, detailed_results)``
     on rank 0 -- same keys as det:202-212 / 225-234 -- and ``({}, [])`` elsewhere."""
     rank, world = _world()
@@ -284,10 +306,20 @@ def screen_mutant_samples_sharded(screener, test_folders_dict, output_dir=None, 
         return {}, []
 
     sd_model = screener.stardist_model
+    from .screening import _default_imread
+    from .tiff_device import device_route
+    on_device = screener.imread is _default_imread
 
     def load_images(i):
         try:
-            image = screener.imread(files[i])
+            if on_device:                     # the file is read once: parsed for the route, else decoded here
+                buf = _read_file(files[i])
+                f = device_route(files[i], buf)
+                if f is not None:             # a compressed file: decoded on the device with its chunk
+                    return f
+                image = screener.imread(files[i], buf)
+            else:
+                image = screener.imread(files[i])
             if image.ndim == 3 and image.shape[-1] >= 3:                  # det:54-59
                 return np.ascontiguousarray(image[..., 2]), np.ascontiguousarray(image[..., 1])
             return image, image

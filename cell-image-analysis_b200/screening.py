@@ -9,6 +9,7 @@ the built library raises.
 from __future__ import annotations
 
 import ctypes as C
+import io
 import os
 from glob import glob
 
@@ -357,21 +358,23 @@ class Engine:
         return res
 
 
-def _default_imread(path):
+def _default_imread(path, buf=None):
     """tiff.imread (det:51): tifffile when installed, else the in-tree baseline-TIFF reader
     (uncompressed strips), else OpenCV's decoder with the file's channel order restored.
-    Upstream of the hot path (SURVEY N1)."""
+    Upstream of the hot path (SURVEY N1).  ``buf``: the file's bytes when the caller has already
+    read them (the file is then not read again)."""
     try:
         import tifffile
-        return tifffile.imread(path)
+        return tifffile.imread(path if buf is None else io.BytesIO(buf))
     except ImportError:
         pass
     from .tiff_min import TiffError, read_tiff
     try:
-        return read_tiff(path)
+        return read_tiff(path if buf is None else buf)
     except TiffError:
         import cv2
-        img = cv2.imread(path, cv2.IMREAD_UNCHANGED)
+        img = cv2.imread(path, cv2.IMREAD_UNCHANGED) if buf is None else \
+            cv2.imdecode(np.frombuffer(buf, np.uint8), cv2.IMREAD_UNCHANGED)
         if img is None:
             raise IOError(f"cannot read {path}")
         if img.ndim == 3 and img.shape[-1] >= 3:

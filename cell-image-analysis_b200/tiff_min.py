@@ -122,8 +122,37 @@ def _decompress(data: bytes, compression: int, cap: int) -> bytes:
     raise TiffError(f"TIFF compression {compression} is not supported")
 
 
-def _read_page(buf, bo, big, ifd):
-    """One IFD -> (array, offset of the next IFD)."""
+class PageLayout:
+    """One IFD, parsed: what decoding the page needs, on the host or on the device (``cia_tiff_decode_fields``).
+    ``segments`` lists (file offset, byte count) of each strip / tile in decode order (plane, row, column), the
+    count clipped to the file's end as the reader slices it; ``rows`` is the decoded rows of each (tiles are always
+    full size, the last strip is not)."""
+    __slots__ = ("H", "W", "dtype", "spp", "planar", "compression", "predictor", "tiled", "tw", "th", "segments",
+                 "next_ifd")
+
+    def __init__(self, **kw):
+        for k, v in kw.items():
+            setattr(self, k, v)
+
+    def segment_rects(self):
+        """(plane, y0, x0, rows, cols) of each segment, in the order of ``segments``."""
+        planes = self.spp if self.planar == 2 else 1
+        across, down = -(-self.W // self.tw), -(-self.H // self.th)
+        return [(p, ty * self.th, tx * self.tw, self.th if self.tiled else min(self.th, self.H - ty * self.th),
+                 self.tw) for p in range(planes) for ty in range(down) for tx in range(across)]
+
+    def device_decodable(self) -> bool:
+        """Single-page file of 8- or 16-bit unsigned samples, compression none / LZW / Deflate / PackBits, predictor
+        1 or 2: what ``cia_tiff_decode_fields`` decodes bit for bit like ``read_tiff``."""
+        return (self.next_ifd == 0 and self.dtype.kind == "u" and self.dtype.itemsize in (1, 2)
+                and self.compression in DEVICE_COMPRESSIONS and self.predictor in (1, 2))
+
+
+DEVICE_COMPRESSIONS = (1, 5, 8, 32946, 32773)
+
+
+def _parse_page(buf, bo, big, ifd) -> PageLayout:
+    """One IFD -> its layout (no pixel data is read)."""
     if big:
         (n_entries,) = struct.unpack(bo + "Q", buf[ifd:ifd + 8])
         base, esz, vsz, ofmt = ifd + 8, 20, 8, "Q"
@@ -163,7 +192,6 @@ def _read_page(buf, bo, big, ifd):
     if predictor not in (1, 2) or (predictor == 2 and fmt == 3):
         raise TiffError(f"unsupported Predictor {predictor}")
     planes = spp if planar == 2 else 1              # separately stored sample planes
-    cs = 1 if planar == 2 else spp                  # samples per pixel inside one segment
     tiled = 322 in tags or 324 in tags
     if tiled:
         tw, th = tag1(322), tag1(323)
@@ -182,33 +210,43 @@ def _read_page(buf, bo, big, ifd):
         counts = [H * W * spp * dt.itemsize]
     if len(counts) != len(offsets) or len(offsets) < across * down * planes:
         raise TiffError("inconsistent strip / tile tables")
+    n = len(buf)
+    segments = [(o, max(0, min(c, n - o))) for o, c in zip(offsets[:across * down * planes], counts)]
+    return PageLayout(H=H, W=W, dtype=dt, spp=spp, planar=planar, compression=compression, predictor=predictor,
+                      tiled=tiled, tw=tw, th=th, segments=segments, next_ifd=next_ifd)
+
+
+def _decode_page(buf, lay: PageLayout) -> np.ndarray:
+    """The pixels of a parsed page, decoded on the host."""
+    dt, H, W, spp = lay.dtype, lay.H, lay.W, lay.spp
+    planes = spp if lay.planar == 2 else 1
+    cs = 1 if lay.planar == 2 else spp              # samples per pixel inside one segment
     out = np.zeros((planes, H, W, cs), dt.newbyteorder("="))
-    k = 0
-    for p in range(planes):
-        for ty in range(down):
-            for tx in range(across):
-                rows = th if tiled else min(th, H - ty * th)        # tiles are always full size, the last strip is not
-                need = rows * tw * cs * dt.itemsize
-                raw = _decompress(bytes(buf[offsets[k]:offsets[k] + counts[k]]), compression, need)
-                k += 1
-                if len(raw) < need:
-                    raise TiffError("truncated strip / tile data")
-                seg = np.frombuffer(raw, dt, rows * tw * cs).reshape(rows, tw, cs).astype(dt.newbyteorder("="))
-                if predictor == 2:
-                    seg = np.cumsum(seg, axis=1, dtype=seg.dtype)   # horizontal differencing, wraps like the writer
-                y0, x0 = ty * th, tx * tw
-                hh, ww = min(rows, H - y0), min(tw, W - x0)
-                out[p, y0:y0 + hh, x0:x0 + ww] = seg[:hh, :ww]
-    if planar == 2:
+    for (off, cnt), (p, y0, x0, rows, tw) in zip(lay.segments, lay.segment_rects()):
+        need = rows * tw * cs * dt.itemsize
+        raw = _decompress(bytes(buf[off:off + cnt]), lay.compression, need)
+        if len(raw) < need:
+            raise TiffError("truncated strip / tile data")
+        seg = np.frombuffer(raw, dt, rows * tw * cs).reshape(rows, tw, cs).astype(dt.newbyteorder("="))
+        if lay.predictor == 2:
+            seg = np.cumsum(seg, axis=1, dtype=seg.dtype)   # horizontal differencing, wraps like the writer
+        hh, ww = min(rows, H - y0), min(tw, W - x0)
+        out[p, y0:y0 + hh, x0:x0 + ww] = seg[:hh, :ww]
+    if lay.planar == 2:
         img = out[..., 0].transpose(1, 2, 0) if spp > 1 else out[0, ..., 0]
     else:
         img = out[0] if spp > 1 else out[0, ..., 0]
-    return np.ascontiguousarray(img), next_ifd
+    return np.ascontiguousarray(img)
 
 
-def read_tiff(path: str) -> np.ndarray:
-    with open(path, "rb") as f:
-        buf = f.read()
+def _read_page(buf, bo, big, ifd):
+    """One IFD -> (array, offset of the next IFD)."""
+    lay = _parse_page(buf, bo, big, ifd)
+    return _decode_page(buf, lay), lay.next_ifd
+
+
+def _header(buf):
+    """(byte order, BigTIFF?, offset of the first IFD)"""
     if len(buf) < 8:
         raise TiffError("not a TIFF file")
     if buf[:2] == b"II":
@@ -228,6 +266,31 @@ def read_tiff(path: str) -> np.ndarray:
         (ifd,) = struct.unpack(bo + "Q", buf[8:16])
     else:
         raise TiffError("not a TIFF file")
+    return bo, big, ifd
+
+
+def page_layout(buf) -> PageLayout:
+    """Layout of the first page of the TIFF file held in ``buf`` (bytes), parsed exactly as ``read_tiff`` parses it;
+    raises ``TiffError`` where ``read_tiff`` would on the directory."""
+    bo, big, ifd = _header(buf)
+    if not ifd or ifd >= len(buf):
+        raise TiffError("no image in file")
+    try:
+        return _parse_page(buf, bo, big, ifd)
+    except TiffError:
+        raise
+    except (struct.error, TypeError, IndexError, ValueError, OverflowError, MemoryError) as e:
+        raise TiffError(f"malformed TIFF directory: {type(e).__name__}: {e}") from e
+
+
+def read_tiff(path) -> np.ndarray:
+    """The image of a TIFF file; ``path`` may also be the file's bytes, already read."""
+    if isinstance(path, (bytes, bytearray, memoryview)):
+        buf = bytes(path)
+    else:
+        with open(path, "rb") as f:
+            buf = f.read()
+    bo, big, ifd = _header(buf)
     pages, seen = [], set()
     while ifd and ifd not in seen and ifd < len(buf):
         seen.add(ifd)

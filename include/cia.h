@@ -318,6 +318,33 @@ int cia_screen_fields_rle(cia_handle h, const uint16_t* images, const uint32_t* 
 long long cia_tiff_lzw_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap);
 long long cia_tiff_packbits_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap);
 
+/* One compressed strip or tile of a field (tiff_min.page_layout parses it from the file's directory). */
+typedef struct cia_tiff_segment {
+    uint64_t src_off, src_len;      /* its compressed bytes: src[src_off, src_off + src_len)             */
+    uint64_t dst_off;               /* decoded into scratch[dst_off, dst_off + rows * cols * samples * bytes) */
+    int32_t  field;                 /* [0, n_fields)                                                     */
+    int32_t  compression;           /* 1, 5 (LZW), 8 or 32946 (Deflate), 32773 (PackBits)                */
+    int32_t  predictor;             /* 1, or 2 (horizontal differencing, per sample, wrapping)           */
+    int32_t  bytes_per_sample;      /* 1 (widened to uint16) or 2                                        */
+    int32_t  big_endian;            /* 16-bit samples are stored big endian                              */
+    int32_t  samples;               /* interleaved samples per pixel in the segment (planar files: 1)    */
+    int32_t  y0, x0, rows, cols;    /* its rectangle in the field; pixels past H / W (tile edges) are dropped */
+    int32_t  seg_sample, img_sample;/* sample written to seg_out / img_out, -1: none                     */
+} cia_tiff_segment;                  /* 72 bytes                                                          */
+
+/* Decodes the strips / tiles of n_fields TIFF fields in one launch (one warp per segment, csrc/tiff_dev.cu) into
+ * uint16 [n_fields][H][W] planes: seg_out (may be NULL) takes the segmentation channel, img_out the analysis
+ * channel of cia_screen_images (det:54-59).  src, segs, scratch, the planes and field_status are DEVICE pointers.
+ * field_status int32 [n_fields] is zeroed, then bit 0 marks a corrupt stream, bit 1 a segment that decoded short
+ * and bit 2 a descriptor outside src / scratch, with rows or cols outside [1, 2^20], samples outside [1, 16] or
+ * another field outside its range; a field with a nonzero status is unusable and the other fields are unaffected.
+ * A descriptor whose `field` is outside [0, n_fields) is skipped: there is no field to flag, so the caller must
+ * give every field its segments (tiff_device.pack_fields does).  Reads stay inside each segment's bytes, writes inside its rectangle of its own
+ * field.  Deflate streams are accepted and refused exactly as Python's zlib.decompress does. */
+int cia_tiff_decode_fields(cia_handle h, const uint8_t* src, size_t src_bytes, const cia_tiff_segment* segs,
+                           int n_segs, int n_fields, int H, int W, uint8_t* scratch, size_t scratch_bytes,
+                           uint16_t* seg_out, uint16_t* img_out, int32_t* field_status, void* stream);
+
 /* Stage timing of the fused path with CUDA events recorded in-stream (no host sync is
  * added to the timed region): after cia_profile_begin(h, R) the next R calls of
  * cia_screen_fields bracket scan / gates / crop / CAE / SVM / accumulate with events;
