@@ -101,6 +101,7 @@ SIGNATURES = {
                                            _P, _I, _P, _P, C.POINTER(Scores), _P, _P, _P, _P, _I, _P]),
     "cia_tiff_lzw_decode": (C.c_longlong, [_P, C.c_size_t, _P, C.c_size_t]),
     "cia_tiff_packbits_decode": (C.c_longlong, [_P, C.c_size_t, _P, C.c_size_t]),
+    "cia_tiff_zstd_decode": (C.c_longlong, [_P, C.c_size_t, _P, C.c_size_t]),
     "cia_tiff_decode_fields": (_I, [_P, _P, C.c_size_t, _P, _I, _I, _I, _I, _P, C.c_size_t, _P, _P, _P, _P]),
     "cia_profile_begin": (_I, [_P, _I]),
     "cia_profile_end": (_I, [_P, C.POINTER(C.c_double), C.POINTER(_I)]),

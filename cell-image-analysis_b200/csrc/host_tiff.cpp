@@ -1,10 +1,14 @@
 // host_tiff.cpp -- host-side TIFF strip / tile decompressors behind tiff_min.read_tiff (the reader
 // standing in for tiff.imread, improved_detection.py:51): LZW (TIFF 6.0 section 13, MSB-first codes,
 // "early change") and PackBits.  Plain C++, no CUDA; exported through the C-ABI so that the Python
-// reader does not decode 8 MB fields byte by byte in the interpreter.  Deflate is zlib's (Python).
+// reader does not decode 8 MB fields byte by byte in the interpreter.  Deflate is zlib's (Python).  Zstandard is
+// td_zstd of tiff_decode.h, the decoder the device runs, compiled for the host.
 #include <stddef.h>
 #include <stdint.h>
+#include <memory>
 #include <vector>
+
+#include "tiff_decode.h"
 
 extern "C" {
 
@@ -78,6 +82,13 @@ long long cia_tiff_packbits_decode(const uint8_t* src, size_t n, uint8_t* dst, s
         }
     }
     return (long long)op;
+}
+
+// Zstandard frames (RFC 8878) with the contract of cia_tiff_lzw_decode: output clipped at cap, -1 on a corrupt stream.
+long long cia_tiff_zstd_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap) {
+    if (!src || !dst) return -1;
+    std::unique_ptr<TdZstdWork> w(new TdZstdWork);
+    return td_zstd(src, n, dst, cap, w.get());
 }
 
 }  // extern "C"

@@ -1,9 +1,9 @@
 // tiff_dev.cu -- device decode of compressed TIFF fields (SURVEY 8f row N1): the strips / tiles of a chunk of
 // fields are independent streams, so one launch decodes all of them, one warp per segment.  Lane 0 runs the serial
-// decoder of tiff_decode.h into the caller's scratch with its tables and Deflate window in shared memory; then the
-// warp undoes horizontal differencing along each row with a shuffle scan, swaps big-endian samples, widens 8-bit
-// samples and writes the segment's rectangle (cropped at the field's edges) into the uint16 planes that
-// cia_screen_images reads.
+// decoder of tiff_decode.h (Deflate, LZW, PackBits or Zstandard) into the caller's scratch with its tables and the
+// Deflate window in shared memory; then the warp undoes horizontal differencing along each row with a shuffle scan,
+// swaps big-endian samples, widens 8-bit samples and writes the segment's rectangle (cropped at the field's edges)
+// into the uint16 planes that cia_screen_images reads.
 #include "common.cuh"
 #include "tiff_decode.h"
 
@@ -26,6 +26,7 @@ __global__ void __launch_bounds__(32) tiff_decode_kernel(const uint8_t* __restri
     __shared__ union {
         TdInflateWork inflate;
         TdLzwWork lzw;
+        TdZstdWork zstd;
     } work;
     __shared__ long long produced;
     const int lane = threadIdx.x;
@@ -53,6 +54,7 @@ __global__ void __launch_bounds__(32) tiff_decode_kernel(const uint8_t* __restri
             case 5: n = td_lzw(s, g.src_len, d, need, &work.lzw); break;
             case 8: case 32946: n = td_inflate(s, g.src_len, d, need, &work.inflate); break;
             case 32773: n = td_packbits(s, g.src_len, d, need); break;
+            case 50000: case 34926: n = td_zstd(s, g.src_len, d, need, &work.zstd); break;
             default: n = -1;
         }
         produced = n;

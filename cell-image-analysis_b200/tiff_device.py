@@ -12,11 +12,21 @@ import numpy as np
 import torch
 
 from . import _lib
-from .tiff_min import PageLayout, TiffError, page_layout
+from .tiff_min import ZSTD_COMPRESSIONS, PageLayout, TiffError, page_layout
 
 # A field whose largest strip / tile decodes to more bytes than this goes through the host reader: one segment is
 # one serial stream on the device (tools/tiff_decode_probe.py, DESIGN §6 "TIFF decode on the device").
 MAX_DEVICE_SEGMENT_BYTES = 1 << 20
+# The same limit for Zstandard, set end to end: one warp decodes a zstd segment at about 5 MB/s, and the host route
+# decodes on all loader threads while the device screens, so the sharded screen is faster with the device route up
+# to 512 KB segments (128 rows of a 2048-wide uint16 field) and slower from 1 MB on (tools/tiff_zstd_probe.py,
+# DESIGN §6).
+MAX_DEVICE_ZSTD_SEGMENT_BYTES = 1 << 19
+
+
+def max_device_segment_bytes(compression: int) -> int:
+    """The largest decoded strip / tile of a field ``device_route`` sends to the device, by codec"""
+    return MAX_DEVICE_ZSTD_SEGMENT_BYTES if compression in ZSTD_COMPRESSIONS else MAX_DEVICE_SEGMENT_BYTES
 
 
 class TiffField:
@@ -60,7 +70,8 @@ def device_route(path: str, buf: bytes, dtype=np.uint16):
     lay = f.layout
     cs = 1 if lay.planar == 2 else lay.spp
     seg_bytes = lay.th * lay.tw * cs * lay.dtype.itemsize
-    if lay.compression == 1 or lay.dtype.newbyteorder("=") != np.dtype(dtype) or seg_bytes > MAX_DEVICE_SEGMENT_BYTES:
+    if (lay.compression == 1 or lay.dtype.newbyteorder("=") != np.dtype(dtype)
+            or seg_bytes > max_device_segment_bytes(lay.compression)):
         return None
     return f
 

@@ -3,10 +3,11 @@
 
 Reads what acquisition software and ImageJ write for 8/16/32-bit fields: classic TIFF and BigTIFF,
 little or big endian, strips or tiles, chunky or planar samples, integer and IEEE float samples,
-compression none / LZW / Deflate (zlib, both tag values) / PackBits, horizontal differencing
-(Predictor 2), and multi-page files (pages of one shape come back stacked ``[pages, H, W(, S)]`` like
-``tifffile.imread``).  LZW and PackBits are decoded natively (libcia: csrc/host_tiff.cpp) with a
-pure-Python fallback when the library has not been built.  JPEG / JPEG-XR / LERC etc. raise
+compression none / LZW / Deflate (zlib, both tag values) / PackBits / Zstandard (50000 and the older 34926),
+horizontal differencing (Predictor 2), and multi-page files (pages of one shape come back stacked
+``[pages, H, W(, S)]`` like ``tifffile.imread``).  LZW and PackBits are decoded natively (libcia:
+csrc/host_tiff.cpp) with a pure-Python fallback when the library has not been built; Zstandard is decoded
+only by libcia, with the decoder the device runs.  JPEG / JPEG-XR / LERC etc. raise
 ``TiffError`` -- ``_default_imread`` then tries tifffile / OpenCV when they are present.
 """
 from __future__ import annotations
@@ -119,6 +120,16 @@ def _decompress(data: bytes, compression: int, cap: int) -> bytes:
                 raise TiffError("corrupt LZW / PackBits stream")
             return dst.raw[:n]
         return _lzw_python(data, cap) if compression == 5 else _packbits_python(data, cap)
+    if compression in ZSTD_COMPRESSIONS:
+        lib = _native()
+        if lib is None:
+            raise TiffError("Zstandard TIFF data needs libcia.so: build it with `python __graft_entry__.py build`")
+        import ctypes as C
+        dst = C.create_string_buffer(cap)
+        n = lib.cia_tiff_zstd_decode(data, len(data), dst, cap)
+        if n < 0:
+            raise TiffError("corrupt Zstandard stream")
+        return dst.raw[:n]
     raise TiffError(f"TIFF compression {compression} is not supported")
 
 
@@ -142,13 +153,14 @@ class PageLayout:
                  self.tw) for p in range(planes) for ty in range(down) for tx in range(across)]
 
     def device_decodable(self) -> bool:
-        """Single-page file of 8- or 16-bit unsigned samples, compression none / LZW / Deflate / PackBits, predictor
-        1 or 2: what ``cia_tiff_decode_fields`` decodes bit for bit like ``read_tiff``."""
+        """Single-page file of 8- or 16-bit unsigned samples, compression none / LZW / Deflate / PackBits / Zstandard,
+        predictor 1 or 2: what ``cia_tiff_decode_fields`` decodes bit for bit like ``read_tiff``."""
         return (self.next_ifd == 0 and self.dtype.kind == "u" and self.dtype.itemsize in (1, 2)
                 and self.compression in DEVICE_COMPRESSIONS and self.predictor in (1, 2))
 
 
-DEVICE_COMPRESSIONS = (1, 5, 8, 32946, 32773)
+ZSTD_COMPRESSIONS = (50000, 34926)      # libtiff's COMPRESSION_ZSTD, and the code older tifffile versions wrote
+DEVICE_COMPRESSIONS = (1, 5, 8, 32946, 32773) + ZSTD_COMPRESSIONS
 
 
 def _parse_page(buf, bo, big, ifd) -> PageLayout:

@@ -313,17 +313,20 @@ int cia_screen_fields_rle(cia_handle h, const uint16_t* images, const uint32_t* 
                           void* stream);
 
 /* Host-only strip / tile decompressors of the TIFF reader that stands in for tiff.imread
- * (improved_detection.py:51; SURVEY 8f row N1): TIFF-LZW and PackBits.  Return the bytes written
- * to dst (at most cap) or -1 on a corrupt stream. */
+ * (improved_detection.py:51; SURVEY 8f row N1): TIFF-LZW, PackBits and Zstandard (RFC 8878 frames, the
+ * decoder cia_tiff_decode_fields runs; dictionaries are refused, content sizes and checksums are verified; a few
+ * non-conforming streams libzstd accepts are refused, see csrc/tiff_decode.h).  Return the bytes written to dst
+ * (at most cap) or -1 on a corrupt stream. */
 long long cia_tiff_lzw_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap);
 long long cia_tiff_packbits_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap);
+long long cia_tiff_zstd_decode(const uint8_t* src, size_t n, uint8_t* dst, size_t cap);
 
 /* One compressed strip or tile of a field (tiff_min.page_layout parses it from the file's directory). */
 typedef struct cia_tiff_segment {
     uint64_t src_off, src_len;      /* its compressed bytes: src[src_off, src_off + src_len)             */
     uint64_t dst_off;               /* decoded into scratch[dst_off, dst_off + rows * cols * samples * bytes) */
     int32_t  field;                 /* [0, n_fields)                                                     */
-    int32_t  compression;           /* 1, 5 (LZW), 8 or 32946 (Deflate), 32773 (PackBits)                */
+    int32_t  compression;           /* 1, 5 (LZW), 8 or 32946 (Deflate), 32773 (PackBits), 50000 or 34926 (Zstandard) */
     int32_t  predictor;             /* 1, or 2 (horizontal differencing, per sample, wrapping)           */
     int32_t  bytes_per_sample;      /* 1 (widened to uint16) or 2                                        */
     int32_t  big_endian;            /* 16-bit samples are stored big endian                              */
@@ -340,7 +343,8 @@ typedef struct cia_tiff_segment {
  * another field outside its range; a field with a nonzero status is unusable and the other fields are unaffected.
  * A descriptor whose `field` is outside [0, n_fields) is skipped: there is no field to flag, so the caller must
  * give every field its segments (tiff_device.pack_fields does).  Reads stay inside each segment's bytes, writes inside its rectangle of its own
- * field.  Deflate streams are accepted and refused exactly as Python's zlib.decompress does. */
+ * field.  Deflate streams are accepted and refused exactly as Python's zlib.decompress does; Zstandard streams
+ * exactly as cia_tiff_zstd_decode does. */
 int cia_tiff_decode_fields(cia_handle h, const uint8_t* src, size_t src_bytes, const cia_tiff_segment* segs,
                            int n_segs, int n_fields, int H, int W, uint8_t* scratch, size_t scratch_bytes,
                            uint16_t* seg_out, uint16_t* img_out, int32_t* field_status, void* stream);
